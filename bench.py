@@ -3,7 +3,7 @@
 collision-resolved particle-steps/s at 1/2/4/8 B200 + fraction of the HBM roofline).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--workload temp_pore|cube] [--particles-per-gpu M]
+                  [--workload temp_pore|cube] [--particles-per-gpu M] [--dump-outputs DIR]
 
 One "step" = one whole timestep (drift, walls, recapture, cell sort, pair detection, the ordered
 8-colour-group resolution, recapture, MFP / momentum bookkeeping) over all particles of the job.
@@ -40,9 +40,28 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 B_STEP = 162.0      # algorithmic bytes per particle-step, fp64 state read + written once (SURVEY 8d)
 B_PAIR = 32.0       # algorithmic bytes per particle for the pair kernel: 3 x f64 position + cell header
+DUMP_SAMPLE = 1 << 19   # particles in the --dump-outputs sample: 11 state arrays + the indices, x 8 B x 2^19 = 50 MB
+
+
+def dump_outputs(path, sim, last):
+    """--dump-outputs: what the timed path hands its caller after its last step, as float64 .npy files in `path`:
+    the particle state (get_state, particle-index order) of a fixed, seeded sample of the particles, the sample's
+    particle indices, and the counters of that step.  The inputs are seeded too, so the files of two builds run with
+    the same arguments can be compared one by one."""
+    os.makedirs(path, exist_ok=True)
+    state = sim.get_state()
+    n = len(state["x"])
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    np.save(os.path.join(path, "particle_index.npy"), idx.astype(np.float64))
+    for k, v in state.items():
+        np.save(os.path.join(path, k + ".npy"), v[idx].astype(np.float64))
+    for k, v in last.items():
+        if k != "pair_checks_exec":     # the pair tests the kernels executed: a measure of their work, not a result
+            np.save(os.path.join(path, "step_" + k + ".npy"), np.atleast_1d(np.asarray(v, dtype=np.float64)))
 
 
 def ncu_traffic(kernel, particles):
@@ -293,6 +312,8 @@ def run_ours(args):
     barrier()
     clk = clocks.stop()
     digest = sim.state_digest()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sim, stats[-1])
     dev_ms = max_over_ranks(ms[4])
     total_particles = sum_over_ranks(float(n))
     value = total_particles * args.steps / (dev_ms * 1e-3)
@@ -729,7 +750,14 @@ def main():
     ap.add_argument("--no-ref", action="store_true", help="skip the 1.5-minute run of the unmodified upstream script (cpu_baseline_reference)")
     ap.add_argument("--no-verify", action="store_true", help="skip the out-of-band check against the oracle / the 1-GPU replay")
     ap.add_argument("--port-only", action="store_true", help="--impl reference: time only the C port of the reference algorithm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single-GPU temp_pore: after the timed steps, write the state of a seeded particle sample and the "
+                         "last step's counters to DIR/<name>.npy (float64, about 50 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "temp_pore" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is available for the single-GPU temp_pore workload of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

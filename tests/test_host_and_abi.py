@@ -6,7 +6,6 @@ import os
 import re
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
@@ -81,13 +80,16 @@ def test_ctypes_structs_match_the_header_layout():
     assert ctypes.sizeof(amc.AmcStepStats) == 8 * (10 + 10 + 3)
 
 
-def test_no_cpu_fallback_without_a_device(pore_cfg):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from argon_monte_carlo_b200 import amc
-    with pytest.raises(amc.AmcError):
-        amc.Simulation(pore_cfg)
+def test_no_cpu_fallback_without_a_device():
+    """In a process that sees no device (CUDA_VISIBLE_DEVICES empty, so this runs on GPU machines too) creating a
+    simulation raises AmcError instead of computing anywhere else."""
+    import subprocess
+    import sys
+    code = ("from argon_monte_carlo_b200 import amc, config\n"
+            "try:\n    amc.Simulation(config.pore_config(False))\nexcept amc.AmcError as e:\n    print('AmcError', e)\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.startswith("AmcError"), r.stdout + r.stderr
 
 
 def test_product_never_imports_the_oracle():

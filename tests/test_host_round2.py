@@ -53,7 +53,7 @@ def test_state_digest_restatement_is_order_independent_and_additive():
     assert amc.digest_of_arrays(ids2, st) != d
 
 
-def test_reference_runner_parses_the_scripts_own_timing_prints(monkeypatch):
+def test_reference_runner_parses_the_scripts_own_timing_prints(monkeypatch, tmp_path):
     """baseline/stage.py takes the per-step times from the lines the upstream scripts print (Pore:517, 554 / Temp:810, 849);
     fed a canned transcript, it returns particle-steps/s from the steps after the initial-overlap transient."""
     sys.path.insert(0, os.path.join(ROOT, "baseline"))
@@ -68,10 +68,16 @@ def test_reference_runner_parses_the_scripts_own_timing_prints(monkeypatch):
     assert r["kind"] == "reference" and r["cores"] == os.cpu_count()
     assert abs(r["ms_per_step"] - 40000.0) < 1e-6 and abs(r["value"] - 557649 / 40.0) < 1e-6      # step 0 dropped
     assert r["detail"]["collisions_per_step"] == [1402, 563]
-    # the staged copy in this container is byte-identical to the upstream tree, if that is present
-    if os.path.isdir("/root/reference") and os.path.isdir(stage.REF_DIR):
-        for f in stage.FILES:
-            assert open(os.path.join("/root/reference", f), "rb").read() == open(os.path.join(stage.REF_DIR, f), "rb").read()
+    # staging copies the upstream files byte for byte (a stand-in upstream tree with distinct contents per file)
+    src, dst = tmp_path / "upstream", tmp_path / "_ref"
+    src.mkdir()
+    for k, f in enumerate(stage.FILES):
+        (src / f).write_bytes(bytes(range(k, 256)) + b"\r\n" + f.encode())
+    monkeypatch.setattr(stage, "REF_DIR", str(dst))
+    assert stage.stage(str(src))
+    for f in stage.FILES:
+        assert (dst / f).read_bytes() == (src / f).read_bytes()
+    assert not stage.stage(str(tmp_path / "missing"))
 
 
 def test_clock_sampler_selects_rows_by_timestamp():
