@@ -90,7 +90,14 @@ EXPORTS = ("amc_create", "amc_destroy", "amc_last_error", "amc_abi_version", "am
            "amc_get_outputs_raw", "amc_set_outputs_raw", "amc_get_step_index",
            "amc_slab_enable", "amc_set_stream", "amc_set_ids", "amc_slab_advect", "amc_slab_sort", "amc_slab_pairs_begin",
            "amc_slab_group", "amc_slab_apply", "amc_slab_finish", "amc_slab_get_owned", "amc_state_digest",
-           "amc_slab_p2p_setup", "amc_slab_p2p_connect", "amc_slab_step", "amc_wall_operator", "amc_seed_relax", "amc_last_scatter_ms")
+           "amc_slab_p2p_setup", "amc_slab_p2p_connect", "amc_slab_step", "amc_wall_operator", "amc_seed_relax", "amc_last_scatter_ms",
+           "amc_sample_enable", "amc_sample_disable", "amc_sample_now", "amc_sample_get_raw", "amc_sample_set_raw",
+           "amc_last_sample_ms")
+
+# field sampling (include/amc.h): words per cell and the binary scales of the fixed-point limbs
+SAMPLE_WORDS = 13
+SAMPLE_V1, SAMPLE_V2 = 19, 49     # velocity sums: high / low limb
+SAMPLE_Q1, SAMPLE_Q2 = 6, 36      # sums of squares: high / low limb
 
 
 def load_library():
@@ -162,6 +169,76 @@ def digest_of_arrays(ids, state):
     return int(s0), int(s1), int(len(ids))
 
 
+def sample_grid_shape(grid):
+    """(nx, ny, nz) cells of the sampling grid of a handle on `grid` (a slab run: the global grid)."""
+    return tuple(int(v) for v in grid.nc)
+
+
+def sample_cells_of(x, y, z, grid):
+    """Sampling cell of every particle (x-major, z-minor) and a mask of the particles inside the grid: the owner-cell
+    rule edge[a][k] <= v < edge[a][k+1] of the sort; NaN and anything outside the grid on any axis is outside."""
+    idx, inside = [], None
+    for a, v in enumerate((x, y, z)):
+        e = np.asarray(grid.edge[a], dtype=np.float64)
+        k = np.searchsorted(e, np.asarray(v, dtype=np.float64), side="right") - 1
+        ok = (k >= 0) & (k < len(e) - 1)
+        inside = ok if inside is None else inside & ok
+        idx.append(k)
+    nx, ny, nz = sample_grid_shape(grid)
+    cell = (idx[0] * ny + idx[1]) * nz + idx[2]
+    return np.where(inside, cell, -1), inside
+
+
+def sample_limbs(v, s1, s2):
+    """The two fixed-point limbs one value adds (acc_add's scheme, include/amc.h), as int64 arrays."""
+    v = np.asarray(v, dtype=np.float64)
+    with np.errstate(invalid="ignore"):
+        i1 = np.rint(v * 2.0 ** s1).astype(np.int64)
+        rem = v - i1.astype(np.float64) * 2.0 ** -s1
+        i2 = np.rint(rem * 2.0 ** s2).astype(np.int64)
+    return i1, i2
+
+
+def sample_moments_of_arrays(state, grid, ids=None):
+    """NumPy restatement of one amc_sample_now on `state` (mapping with 'x', 'y', 'z', 'vx', 'vy', 'vz'):
+    (acc [cells][SAMPLE_WORDS] uint64, 1, n_outside), the layout of Simulation.sample_raw.  ids: optional indices
+    into the arrays selecting the particles (default: all).  Integer sums: the result does not depend on the order of
+    the particles, and the raw arrays of disjoint parts add up (mod 2^64) to the raw array of the whole."""
+    sel = (lambda a: np.asarray(a)) if ids is None else (lambda a: np.asarray(a)[np.asarray(ids)])
+    cell, inside = sample_cells_of(sel(state["x"]), sel(state["y"]), sel(state["z"]), grid)
+    ncell = int(np.prod(sample_grid_shape(grid)))
+    acc = np.zeros((ncell, SAMPLE_WORDS), dtype=np.uint64)
+    c = cell[inside]
+    order = np.argsort(c, kind="stable")
+    cs = c[order]
+    starts = np.flatnonzero(np.concatenate([[True], cs[1:] != cs[:-1]])) if len(cs) else np.zeros(0, dtype=np.int64)
+    acc[:, 0] = np.bincount(c, minlength=ncell).astype(np.uint64)
+    words = []
+    for k in ("vx", "vy", "vz"):
+        words += list(sample_limbs(sel(state[k])[inside], SAMPLE_V1, SAMPLE_V2))
+    for k in ("vx", "vy", "vz"):
+        v = np.asarray(sel(state[k]), dtype=np.float64)[inside]
+        words += list(sample_limbs(v * v, SAMPLE_Q1, SAMPLE_Q2))
+    if len(cs):
+        for j, w in enumerate(words):       # per-cell sums of the sorted words (uint64 adds wrap mod 2^64)
+            acc[cs[starts], 1 + j] = np.add.reduceat(w.view(np.uint64)[order], starts)
+    return acc, 1, int(np.count_nonzero(~inside))
+
+
+def merge_sample_ranks(parts):
+    """Raw samples of the ranks of one run (each (acc, n_samples, n_outside)): element-wise sums mod 2^64; every rank
+    took the same samples."""
+    parts = list(parts)
+    ns = {int(p[1]) for p in parts}
+    if len(ns) != 1:
+        raise AmcError("ranks disagree on the number of samples taken: %s" % sorted(ns))
+    acc = parts[0][0].copy()
+    with np.errstate(over="ignore"):
+        for p in parts[1:]:
+            acc += p[0]
+    return acc, ns.pop(), sum(int(p[2]) for p in parts) & ((1 << 64) - 1)
+
+
 def combine_digests(parts):
     """Sum of per-rank digests (mod 2^64 per component)."""
     m = (1 << 64) - 1
@@ -225,6 +302,9 @@ class Simulation:
             self.h = None
             raise AmcError("amc_create failed (%d): %s" % (rc, msg.decode() if msg else "?"))
         self.n = 0
+        self.sample_grid = grid     # a slab rank's handle samples the global grid (slab.SlabRank sets it)
+        self.sampling = None    # (every, first_step) while field sampling is enabled
+        self.host_steps = 0     # timesteps taken by step_host_rng (the index the sampling schedule of that path uses)
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -393,7 +473,55 @@ class Simulation:
                   oob_after_walls_recapture=oob_walls_after, oob_after_pp_recapture=oob_pp_after,
                   dpz=dpz, e_cold=e_cold, e_hot=e_hot, collisions=wall_hits + st["pp_collisions"],
                   errors=st["errors"] + errors)
+        self.host_steps += 1
+        if self.sample_due(self.host_steps - 1):
+            self.sample_now()
         return st
+
+    # ------------------------------------------------------------------ field sampling
+    def sample_enable(self, every=0, first_step=0):
+        """Accumulate per-cell moments of the state (amc_sample_enable): after every timestep s with s >= first_step
+        and (s - first_step) % every == 0 (every = 0: only on sample_now()).  Zeroes the accumulators."""
+        self._check(self.lib.amc_sample_enable(self.h, C.c_int32(int(every)), C.c_int64(int(first_step))), "amc_sample_enable")
+        self.sampling = (int(every), int(first_step))
+
+    def sample_disable(self):
+        self._check(self.lib.amc_sample_disable(self.h), "amc_sample_disable")
+        self.sampling = None
+
+    def sample_due(self, step):
+        if self.sampling is None or self.sampling[0] <= 0:
+            return False
+        every, first = self.sampling
+        return step >= first and (step - first) % every == 0
+
+    def sample_now(self):
+        """One sample of the current state."""
+        self._check(self.lib.amc_sample_now(self.h), "amc_sample_now")
+
+    def sample_cells(self):
+        return int(np.prod(sample_grid_shape(self.sample_grid)))
+
+    def sample_raw(self):
+        """(acc [cells][SAMPLE_WORDS] uint64, samples taken, particles found outside the grid)."""
+        acc = np.zeros((self.sample_cells(), SAMPLE_WORDS), dtype=np.uint64)
+        ns, no = C.c_uint64(0), C.c_uint64(0)
+        self._check(self.lib.amc_sample_get_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(ns), C.byref(no)),
+                    "amc_sample_get_raw")
+        return acc, int(ns.value), int(no.value)
+
+    def sample_set_raw(self, acc, n_samples, n_outside):
+        acc = np.ascontiguousarray(acc, dtype=np.uint64)
+        if acc.size != self.sample_cells() * SAMPLE_WORDS:
+            raise AmcError("sample accumulators of %d words for a grid of %d cells" % (acc.size, self.sample_cells()))
+        self._check(self.lib.amc_sample_set_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64)), C.c_uint64(int(n_samples)),
+                                                C.c_uint64(int(n_outside))), "amc_sample_set_raw")
+
+    def last_sample_ms(self):
+        """Device time (ms) of the sampling kernel, summed over the samples of the last step() / sample_now() call."""
+        v = C.c_double(0.0)
+        self._check(self.lib.amc_last_sample_ms(self.h, C.byref(v)), "amc_last_sample_ms")
+        return float(v.value)
 
     # ------------------------------------------------------------------ outputs
     def histograms(self):
@@ -448,6 +576,10 @@ class Simulation:
             import pickle
             import random
             st["host_rng"] = np.frombuffer(pickle.dumps((np.random.get_state(), random.getstate())), dtype=np.uint8)
+        if self.sampling is not None:
+            acc, ns, no = self.sample_raw()
+            st.update(sample_acc=acc, sample_n=np.uint64(ns), sample_outside=np.uint64(no),
+                      sample_schedule=np.array(self.sampling, dtype=np.int64), host_steps=np.int64(self.host_steps))
         if path is not None:
             np.savez(path, **st)
         return st
@@ -471,6 +603,11 @@ class Simulation:
             np_state, py_state = pickle.loads(np.asarray(ck["host_rng"], dtype=np.uint8).tobytes())
             np.random.set_state(np_state)
             random.setstate(py_state)
+        if "sample_acc" in ck:          # checkpoints written without sampling have none of these keys
+            every, first = (int(v) for v in ck["sample_schedule"])
+            self.sample_enable(every, first)
+            self.sample_set_raw(ck["sample_acc"], int(ck["sample_n"]), int(ck["sample_outside"]))
+            self.host_steps = int(ck["host_steps"])
 
     def state_digest(self):
         """(sum0, sum1, count): order-independent checksum of the owned particle state, computed on the device

@@ -69,6 +69,15 @@ struct amc_handle {
     std::vector<cudaEvent_t> sc_events;  // two per step of the last amc_step chunk: around k_scatter_advect
     double last_scatter_ms = 0;
     int64_t last_launches = 0;
+    // field sampling (amc_sample_*): accumulators [cells][AMC_SAMPLE_WORDS] + the outside counter; null: disabled
+    unsigned long long *d_sample = nullptr;
+    int64_t sample_cells = 0;
+    int32_t sample_every = 0;
+    int64_t sample_first = 0;
+    uint64_t n_samples = 0;
+    std::vector<cudaEvent_t> sample_events; // two per sample of the last call: around k_sample
+    int sample_slot = 0;                    // samples recorded into sample_events by the current call
+    double last_sample_ms = 0;
     std::string error;
 
     int fail(int code, const std::string &msg)
@@ -175,6 +184,8 @@ extern "C" int amc_destroy(amc_handle *h)
     for (cudaEvent_t e : h->events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->det_events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->sc_events) cudaEventDestroy(e);
+    for (cudaEvent_t e : h->sample_events) cudaEventDestroy(e);
+    if (h->d_sample) cudaFree(h->d_sample);
     if (h->h_stats) cudaFreeHost(h->h_stats);
     if (h->aux) { cudaStreamSynchronize(h->aux); cudaStreamDestroy(h->aux); }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -596,6 +607,133 @@ static int ensure_events(amc_handle *h, size_t count)
     return AMC_OK;
 }
 
+// ---- field sampling --------------------------------------------------------------------------------
+static bool sample_due(const amc_handle *h, int64_t step)
+{
+    return h->d_sample && h->sample_every > 0 && step >= h->sample_first && (step - h->sample_first) % h->sample_every == 0;
+}
+
+static void sample_reset_timing(amc_handle *h)
+{
+    h->sample_slot = 0;
+    h->last_sample_ms = 0;
+}
+
+// one sample of the state in h->p.a on h->stream (count: p.n, or the device-resident count inside amc_slab_step);
+// grid_n: slots the launch covers; launches (nullable) counts the kernel launch
+static int launch_sample(amc_handle *h, int64_t grid_n, int64_t *launches)
+{
+    while (h->sample_events.size() < (size_t)(2 * h->sample_slot + 2)) {
+        cudaEvent_t e;
+        CK(cudaEventCreate(&e));
+        h->sample_events.push_back(e);
+    }
+    const P &p = h->p;
+    SampleArgs sa;
+    sa.acc = h->d_sample;
+    sa.outside = h->d_sample + h->sample_cells * AMC_SAMPLE_WORDS;
+    if (p.slab) { sa.zedge = p.gz_edge; sa.ncz = p.gncz; sa.ze0 = p.g_e0z; sa.zinv = p.g_inv_dz; }
+    else { sa.zedge = p.edge[2]; sa.ncz = p.nc[2]; sa.ze0 = p.e0[2]; sa.zinv = p.inv_d[2]; }
+    CK(cudaEventRecord(h->sample_events[2 * h->sample_slot], h->stream));
+    if (grid_n > 0) {
+        k_sample<<<grid_for(grid_n, SAMPLE_THREADS), SAMPLE_THREADS, 0, h->stream>>>(p, sa);
+        if (launches) *launches += 1;
+    }
+    CK(cudaEventRecord(h->sample_events[2 * h->sample_slot + 1], h->stream));
+    CK(cudaGetLastError());
+    h->sample_slot++;
+    h->n_samples++;
+    return AMC_OK;
+}
+
+// after a synchronisation: add the kernel times of the samples recorded since the last call
+static int sample_collect_timing(amc_handle *h)
+{
+    for (int k = 0; k < h->sample_slot; k++) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, h->sample_events[2 * k], h->sample_events[2 * k + 1]));
+        h->last_sample_ms += ms;
+    }
+    h->sample_slot = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_sample_enable(amc_handle *h, int32_t every, int64_t first_step)
+{
+    if (!h) return AMC_E_INVALID;
+    if (every < 0) return h->fail(AMC_E_INVALID, "every < 0");
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    const int64_t ncz = h->slab ? h->p.gncz : h->cfg.nc[2];
+    const int64_t cells = (int64_t)h->cfg.nc[0] * h->cfg.nc[1] * ncz;
+    if (h->d_sample && cells != h->sample_cells) { cudaFree(h->d_sample); h->d_sample = nullptr; }
+    const size_t bytes = ((size_t)cells * AMC_SAMPLE_WORDS + 1) * sizeof(unsigned long long);
+    if (!h->d_sample) {
+        cudaError_t e = cudaMalloc(&h->d_sample, bytes);
+        if (e != cudaSuccess) { h->d_sample = nullptr; return h->fail(AMC_E_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e)); }
+    }
+    CK(cudaMemset(h->d_sample, 0, bytes));
+    h->sample_cells = cells;
+    h->sample_every = every;
+    h->sample_first = first_step;
+    h->n_samples = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_sample_disable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    if (h->d_sample) CK(cudaFree(h->d_sample));
+    h->d_sample = nullptr;
+    h->sample_cells = 0; h->sample_every = 0; h->sample_first = 0; h->n_samples = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_sample_now(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_sample) return h->fail(AMC_E_STATE, "sampling is not enabled (amc_sample_enable)");
+    CK(cudaSetDevice(h->device));
+    sample_reset_timing(h);
+    int rc = launch_sample(h, h->n, nullptr);
+    if (rc != AMC_OK) return rc;
+    CK(cudaStreamSynchronize(h->stream));
+    return sample_collect_timing(h);
+}
+
+extern "C" int amc_sample_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_samples, uint64_t *n_outside)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_sample) return h->fail(AMC_E_STATE, "sampling is not enabled (amc_sample_enable)");
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    if (acc) CK(cudaMemcpy(acc, h->d_sample, (size_t)h->sample_cells * AMC_SAMPLE_WORDS * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    if (n_outside) CK(cudaMemcpy(n_outside, h->d_sample + h->sample_cells * AMC_SAMPLE_WORDS, sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    if (n_samples) *n_samples = h->n_samples;
+    return AMC_OK;
+}
+
+extern "C" int amc_sample_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_samples, uint64_t n_outside)
+{
+    if (!h || !acc) return AMC_E_INVALID;
+    if (!h->d_sample) return h->fail(AMC_E_STATE, "sampling is not enabled (amc_sample_enable)");
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpy(h->d_sample, acc, (size_t)h->sample_cells * AMC_SAMPLE_WORDS * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(h->d_sample + h->sample_cells * AMC_SAMPLE_WORDS, &n_outside, sizeof(uint64_t), cudaMemcpyHostToDevice));
+    h->n_samples = n_samples;
+    return AMC_OK;
+}
+
+extern "C" int amc_last_sample_ms(amc_handle *h, double *ms)
+{
+    if (!h || !ms) return AMC_E_INVALID;
+    *ms = h->last_sample_ms;
+    return AMC_OK;
+}
+
 extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
 {
     if (!h) return AMC_E_INVALID;
@@ -611,6 +749,7 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
     h->last_detect_ms = 0;
     h->last_scatter_ms = 0;
     h->last_launches = 0;
+    sample_reset_timing(h);
     int done = 0;
     if (sweep && h->n) { // the sweep kernel addresses particles by id: keep slot == id
         int rc = unsort(h);
@@ -632,12 +771,15 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
         }
         CK(cudaMemsetAsync(h->d_stats, 0, chunk * sizeof(StatsDev), h->stream));
         CK(cudaEventRecord(h->events[0], h->stream));
+        bool closed_prev = true; // the step before this one ended with its own recapture launch
         for (int s = 0; s < chunk; s++) {
             p.stats = h->d_stats + s;
             p.step = h->step_index++;
+            // a sampled step is closed like the last step of a chunk, so the sample sees the state at its end
+            const bool sample = sample_due(h, p.step);
             if (h->n > 0) {
                 // the recapture that closes step s-1's pair pass rides along in step s's advect kernel
-                const bool fuse_prev = has_recap && s > 0;
+                const bool fuse_prev = has_recap && !closed_prev;
                 p.stats_prev = fuse_prev ? h->d_stats + (s - 1) : h->d_stats + s;
                 int phase = PH_DRIFT | PH_WALLS | (has_recap ? PH_RECAP : 0) | (fuse_prev ? PH_RECAP_POST : 0);
                 if (sweep) {
@@ -677,17 +819,20 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
                 h->det_slot = -1;
                 if (rc != AMC_OK) return rc;
                 CK(cudaEventRecord(h->events[4 * s + 3], h->stream));
-                if (has_recap && s == chunk - 1) { // last step of the call: close it now
+                closed_prev = s == chunk - 1 || sample;
+                if (has_recap && closed_prev) { // last step of the call (or a sampled step): close it now
                     if (sweep) k_recapture_post<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p);
                     else k_recapture_list<<<148, ADVECT_THREADS, 0, h->stream>>>(p);
                     h->last_launches += 1;
                 }
+                if (sample && (rc = launch_sample(h, h->n, &h->last_launches)) != AMC_OK) return rc;
                 CK(cudaEventRecord(h->events[4 * s + 4], h->stream));
-            }
+            } else if (sample && (rc = launch_sample(h, 0, nullptr)) != AMC_OK) return rc;
         }
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(h->h_stats, h->d_stats, chunk * sizeof(StatsDev), cudaMemcpyDeviceToHost, h->stream));
         CK(cudaStreamSynchronize(h->stream));
+        if ((rc = sample_collect_timing(h)) != AMC_OK) return rc;
         if (h->n > 0)
             for (int s = 0; s < chunk; s++) {
                 float ms;
@@ -1103,6 +1248,7 @@ extern "C" int amc_slab_enable(amc_handle *h, const amc_slab_config *c)
     if (c->nranks < 1 || c->rank < 0 || c->rank >= c->nranks || !c->cuts || !c->gz_edge || !c->gz_lo) return h->fail(AMC_E_INVALID, "bad slab config");
     if (c->cuts[c->rank + 1] - c->cuts[c->rank] != h->cfg.nc[2]) return h->fail(AMC_E_INVALID, "handle z grid does not match its slab");
     if (h->p.wall_bits) return h->fail(AMC_E_INVALID, "AMC_TAP_WALL_BITS is indexed by particle id (global on a slab handle): not available with slabs");
+    if (h->d_sample) return h->fail(AMC_E_STATE, "enable sampling after amc_slab_enable (a slab handle samples the global grid)");
     CK(cudaSetDevice(h->device));
     P &p = h->p;
     p.slab = 1; p.srank = c->rank; p.nranks = c->nranks; p.zoff = c->cuts[c->rank]; p.gncz = c->gncz;
@@ -1446,6 +1592,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
     const unsigned pgrid = (unsigned)std::min<int64_t>((int64_t)std::min(h->pair_grid, h->pair_grid_fused), std::max<int64_t>(ncell / 8, 1));
     const int phase = PH_DRIFT | PH_WALLS | (p.kind != AMC_KIND_CUBE ? PH_RECAP : 0);
     memset(h->last_ms, 0, sizeof(h->last_ms));
+    sample_reset_timing(h);
     int32_t n32 = (int32_t)h->n;
     CK(cudaMemcpyAsync(h->d_n, &n32, sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
     p.n_dev = h->d_n;
@@ -1530,6 +1677,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
             }
             CK(cudaEventRecord(h->events[4 * s + 3], h->stream));
             if (p.kind != AMC_KIND_CUBE) { k_recapture_list<<<148, ADVECT_THREADS, 0, h->stream>>>(p); h->last_launches += 1; }
+            if (sample_due(h, p.step) && (rc = launch_sample(h, p.n_hint, &h->last_launches)) != AMC_OK) { p.n_dev = nullptr; return rc; } /* count: cur_n */
             k_slab_set_n<<<1, 32, 0, h->stream>>>(p, 0);
             CK(cudaEventRecord(h->events[4 * s + 4], h->stream));
             CK(cudaGetLastError());
@@ -1541,6 +1689,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
         cudaError_t e = cudaStreamSynchronize(h->stream);
         p.n_dev = nullptr;
         if (e != cudaSuccess) return h->fail(AMC_E_CUDA, std::string("amc_slab_step: ") + cudaGetErrorString(e));
+        if ((rc = sample_collect_timing(h)) != AMC_OK) return rc;
         {
             unsigned int timeouts = 0;
             CK(cudaMemcpyFromSymbol(&timeouts, g_flag_timeouts, sizeof(timeouts)));

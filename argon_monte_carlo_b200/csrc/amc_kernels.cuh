@@ -2681,3 +2681,91 @@ __global__ void __launch_bounds__(ADVECT_THREADS) k_state_digest(const __grid_co
     __syncthreads();
     if (threadIdx.x < 3 && sh[threadIdx.x]) atomicAdd(&out[threadIdx.x], sh[threadIdx.x]);
 }
+
+// ---------------------------------------------------------------- field sampling (amc_sample_*)
+// Per-cell moments of the state at the end of a timestep (include/amc.h): count, and sum v, sum v^2 per axis as
+// two fixed-point limbs each.  The particles sit sorted by owner cell, so the lanes of a warp hold two or three
+// runs of one cell: the lanes of each cell (__match_any_sync) add their words with __reduce_add_sync and one lane
+// issues one set of 13 atomics per cell and warp.  __reduce_add_sync adds 32-bit values: a word is split into its
+// low 21 bits (unsigned) and the rest (signed), whose sums over 32 lanes cannot overflow while every word of the
+// warp is below 2^40 in magnitude (|v| < 2^17 m/s); a warp with a larger word falls back to per-particle atomics.
+// Plain 32-byte record + 3 velocities per particle: 56 bytes read, nothing written but the atomics.
+#define SAMPLE_THREADS 256
+struct SampleArgs {
+    unsigned long long *acc;     /* [cells][AMC_SAMPLE_WORDS] */
+    unsigned long long *outside; /* [1] */
+    const double *zedge;         /* z edges of the sampling grid (a slab handle: the global ones) */
+    int32_t ncz;
+    double ze0, zinv;
+};
+__device__ __forceinline__ void sample_limbs(const double v, const double s1, const double s1inv, const double s2, long long &i1, long long &i2)
+{
+    i1 = __double2ll_rn(v * s1);
+    const double rem = v - (double)i1 * s1inv;
+    i2 = __double2ll_rn(rem * s2);
+}
+__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample(const __grid_constant__ P p, const SampleArgs sa)
+{
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned lane = threadIdx.x & 31u;
+    int cell = -1; /* -1: no particle of this rank in the slot, -2: outside the grid */
+    long long w[12];
+#pragma unroll
+    for (int k = 0; k < 12; k++) w[k] = 0;
+    if (s < cur_n(p)) {
+        const PosRec r = p.a.pos[s];
+        if (!(r.flag & AMC_FLAG_GHOST)) { /* the owning rank samples it (same predicate as k_state_digest) */
+            const int ox = owner_axis(p.edge[0], p.nc[0], p.e0[0], p.inv_d[0], r.x);
+            const int oy = owner_axis(p.edge[1], p.nc[1], p.e0[1], p.inv_d[1], r.y);
+            const int oz = owner_axis(sa.zedge, sa.ncz, sa.ze0, sa.zinv, r.z);
+            if (ox < 0 || ox >= p.nc[0] || oy < 0 || oy >= p.nc[1] || oz < 0 || oz >= sa.ncz) cell = -2;
+            else {
+                cell = (ox * p.nc[1] + oy) * sa.ncz + oz;
+                const double v[3] = {p.a.vx[s], p.a.vy[s], p.a.vz[s]};
+#pragma unroll
+                for (int a = 0; a < 3; a++) {
+                    sample_limbs(v[a], 0x1p19, 0x1p-19, 0x1p49, w[2 * a], w[2 * a + 1]);
+                    sample_limbs(v[a] * v[a], 0x1p6, 0x1p-6, 0x1p36, w[6 + 2 * a], w[6 + 2 * a + 1]);
+                }
+            }
+        }
+    }
+    static_assert(AMC_SAMPLE_V1 == 19 && AMC_SAMPLE_V2 == 49 && AMC_SAMPLE_Q1 == 6 && AMC_SAMPLE_Q2 == 36, "scales of k_sample");
+    const unsigned outside = __ballot_sync(0xffffffffu, cell == -2);
+    if (lane == 0 && outside) atomicAdd(sa.outside, (unsigned long long)__popc(outside));
+    bool narrow = true;
+#pragma unroll
+    for (int k = 0; k < 12; k++) narrow &= (unsigned long long)(w[k] + (1ll << 40)) < (1ull << 41);
+    if (__any_sync(0xffffffffu, !narrow)) { /* a word beyond 2^40: one set of atomics per particle */
+        if (cell >= 0) {
+            unsigned long long *a = sa.acc + (size_t)cell * AMC_SAMPLE_WORDS;
+            atomicAdd(a, 1ull);
+#pragma unroll
+            for (int k = 0; k < 12; k++) if (w[k]) atomicAdd(a + 1 + k, (unsigned long long)w[k]);
+        }
+        return;
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, cell);
+    unsigned todo = __ballot_sync(0xffffffffu, cell >= 0);
+    while (todo) { /* one cell of the warp at a time: every lane of `grp` executes the reductions with the same mask */
+        const int first = __ffs(todo) - 1;
+        const unsigned grp = __shfl_sync(0xffffffffu, peers, first);
+        todo &= ~grp;
+        if (grp & (1u << lane)) {
+            long long tot[12];
+#pragma unroll
+            for (int k = 0; k < 12; k++) {
+                const unsigned lo = __reduce_add_sync(grp, (unsigned)(w[k] & 0x1FFFFF));
+                const int hi = __reduce_add_sync(grp, (int)(w[k] >> 21));
+                tot[k] = (long long)hi * (1ll << 21) + (long long)lo;
+            }
+            if ((int)lane == first) {
+                unsigned long long *a = sa.acc + (size_t)cell * AMC_SAMPLE_WORDS;
+                atomicAdd(a, (unsigned long long)__popc(grp));
+#pragma unroll
+                for (int k = 0; k < 12; k++) if (tot[k]) atomicAdd(a + 1 + k, (unsigned long long)tot[k]);
+            }
+        }
+        __syncwarp();
+    }
+}

@@ -11,7 +11,7 @@ import numpy as np
 from . import outputs
 
 
-def parse_args(default_steps, description, temp=False):
+def parse_args(default_steps, description, temp=False, argv=None):
     ap = argparse.ArgumentParser(description=description)
     ap.add_argument("--steps", type=int, default=int(os.environ.get("AMC_STEPS", default_steps)),
                     help="number of timesteps (default: the script's own num_timesteps = %d)" % default_steps)
@@ -23,7 +23,26 @@ def parse_args(default_steps, description, temp=False):
                         help="host: the reference's Mersenne-Twister draws in its order (reproduces "
                              "momentum_energy.csv); device: Philox on the GPU, no host round trips")
     ap.add_argument("--show", action="store_true", help="plt.show() at the end if matplotlib is installed")
-    return ap.parse_args()
+    ap.add_argument("--sample-every", type=int, default=0, metavar="K",
+                    help="sample density, flow velocity and temperature per collision cell after every K-th timestep "
+                         "and write profile_z.csv (default 0: off)")
+    ap.add_argument("--sample-start", type=int, default=0, metavar="S", help="first timestep sampled (default 0)")
+    args = ap.parse_args(argv)
+    if args.sample_every < 0 or args.sample_start < 0:
+        ap.error("--sample-every and --sample-start must be >= 0")
+    return args
+
+
+def sampling_begin(sim, args):
+    """Enable field sampling on `sim` if --sample-every asks for it."""
+    if args.sample_every > 0:
+        sim.sample_enable(args.sample_every, args.sample_start)
+
+
+def sampling_finish(sim, cfg, args):
+    """Write profile_z.csv (one row per z layer) into --outdir if sampling was on."""
+    if args.sample_every > 0:
+        outputs.write_axial_profile(os.path.join(args.outdir, "profile_z.csv"), outputs.axial_profile(sim.sample_raw(), cfg))
 
 
 def final_report(sim, total_errs, total_cols, start, outdir, show=False, labels=("Simulation mean free path: ",

@@ -139,6 +139,7 @@ class SlabRank:
         self.sim = amc.Simulation(cfg, kind=kind, pp_mode=amc.PP_GROUPS, device=device, seed=seed,
                                   grid=local_grid(g, cuts[rank], cuts[rank + 1]), max_particles=max_particles, taps=taps,
                                   cheb=cheb)
+        self.sim.sample_grid = g    # sampling covers the global grid: a particle is binned where it is, whoever owns it
         self.p2p = p2p
         if p2p:
             # device-resident stepping (amc_slab_step): the handle owns the exchange buffers and runs on its own stream
@@ -217,7 +218,7 @@ class LocalTransport:
         return value
 
     def allreduce_u64(self, values):
-        return tuple(values)
+        return values if isinstance(values, np.ndarray) else tuple(values)
 
 
 class DistTransport:
@@ -285,13 +286,16 @@ class DistTransport:
         return out
 
     def allreduce_u64(self, values):
-        """Component-wise sum mod 2^64 over all ranks (int64 adds wrap like uint64 ones)."""
+        """Component-wise sum mod 2^64 over all ranks (int64 adds wrap like uint64 ones).  A uint64 ndarray comes back
+        as an ndarray of the same shape, anything else as a tuple of ints."""
         import torch
-        t = torch.as_tensor(np.array(values, dtype=np.uint64).view(np.int64).copy())
+        arr = np.array(values, dtype=np.uint64)
+        t = torch.as_tensor(arr.view(np.int64).copy())
         if self.dist.get_backend(self.group) == "nccl":
             t = t.cuda()
         self.dist.all_reduce(t, group=self.group)
-        return tuple(int(v) for v in t.cpu().numpy().view(np.uint64))
+        out = t.cpu().numpy().view(np.uint64).reshape(arr.shape)
+        return out if isinstance(values, np.ndarray) else tuple(int(v) for v in out)
 
 
 SUM_KEYS = ("wall_collisions", "pp_collisions", "pair_checks_ref", "pair_checks_exec", "oob_after_walls", "oob_after_pp",
@@ -461,6 +465,8 @@ class SlabSimulation:
             for r in R:
                 st = amc.AmcStepStats()
                 r.call("amc_slab_finish", C.byref(st))
+                if r.sim.sample_due(amc.load_library().amc_get_step_index(r.sim.h) - 1):
+                    r.sim.sample_now()
                 d = st.as_dict()
                 if tot is None:
                     tot = d
@@ -528,6 +534,33 @@ class SlabSimulation:
         the single-domain run of the same job iff the id-ordered states agree bit for bit."""
         d = amc.combine_digests([r.sim.state_digest() for r in self.ranks])
         return self.transport.allreduce_u64(d) if reduce else d
+
+    # ------------------------------------------------------------------ field sampling
+    def sample_enable(self, every=0, first_step=0):
+        """Field sampling on every local rank (Simulation.sample_enable); each rank bins its own particles on the
+        global grid, so the merged accumulators equal those of the single-domain run bit for bit."""
+        for r in self.ranks:
+            r.sim.sample_enable(every, first_step)
+
+    def sample_disable(self):
+        for r in self.ranks:
+            r.sim.sample_disable()
+
+    def sample_now(self):
+        for r in self.ranks:
+            r.sim.sample_now()
+
+    def sample_raw(self, reduce=True):
+        """(acc, samples taken, particles outside the grid) summed over the local ranks and, with a distributed
+        transport and reduce=True, over all processes (element-wise uint64 sums)."""
+        acc, ns, no = amc.merge_sample_ranks([r.sim.sample_raw() for r in self.ranks])
+        if reduce and not isinstance(self.transport, LocalTransport):
+            acc = self.transport.allreduce_u64(acc)
+            (no,) = self.transport.allreduce_u64((no,))
+        return acc, ns, no
+
+    def last_sample_ms(self):
+        return [r.sim.last_sample_ms() for r in self.ranks]
 
     def histograms(self):
         counts, n, sums = None, 0, None

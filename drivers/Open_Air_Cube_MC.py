@@ -20,6 +20,7 @@ if __name__ == "__main__":
     state = init_state.cube_initial_state(cfg)
     sim = amc.Simulation(cfg, device=args.device)
     sim.set_state(*state)
+    driver_common.sampling_begin(sim, args)
     done = 0
     while done < args.steps:
         chunk = min(args.chunk, args.steps - done)
@@ -33,5 +34,6 @@ if __name__ == "__main__":
         print('Simulation 1 ' + lab + str(m))
     print('Num of collisions total: ' + str(n_paths))
     outputs.write_histograms(counts, args.outdir)
+    driver_common.sampling_finish(sim, cfg, args)
     sim.close()
     driver_common.maybe_show(args.show)

@@ -24,6 +24,7 @@ if __name__ == "__main__":
     state = init_state.pore_initial_state(cfg)          # seeds 17 / 17, reference draw order
     sim = amc.Simulation(cfg, device=args.device)
     sim.set_state(*state)
+    driver_common.sampling_begin(sim, args)
     print('Initialization Runtime: ' + str(time() - start) + ' seconds')
     print('  There are {} particles out of bounds after initialization.'.format(sim.recapture()))
     total_cols = total_errs = 0
@@ -44,6 +45,7 @@ if __name__ == "__main__":
             print('   ', s["collisions"], ' collisions from this timestep')
         done += chunk
     driver_common.final_report(sim, total_errs, total_cols, start, args.outdir)
+    driver_common.sampling_finish(sim, cfg, args)
     print('Runtime: ' + str((time() - start) / 60.0) + ' minutes')
     sim.close()
     driver_common.maybe_show(args.show)

@@ -39,6 +39,7 @@ if __name__ == "__main__":
     host = args.rng == "host"
     sim = amc.Simulation(cfg, device=args.device, rng_mode=amc.RNG_HOST if host else amc.RNG_DEVICE)
     sim.set_state(*state)
+    driver_common.sampling_begin(sim, args)
     print('Initialization Runtime: ' + str(time() - start) + ' seconds')
     print('  There are {} particles out of bounds after initialization.'.format(census_after_init(*state[:3], cfg.geom)))
     momentum, e_hot, e_cold = [], [], []
@@ -66,6 +67,7 @@ if __name__ == "__main__":
             momentum.append(s["dpz"]); e_hot.append(s["e_hot"]); e_cold.append(s["e_cold"])
         done += chunk
     driver_common.final_report(sim, total_errs, total_cols, start, args.outdir)
+    driver_common.sampling_finish(sim, cfg, args)
     outputs.write_momentum_energy_csv(momentum, e_cold, e_hot, os.path.join(args.outdir, "momentum_energy.csv"))
     import mpmath
     for series in (momentum, e_cold, e_hot):

@@ -228,6 +228,41 @@ int64_t amc_get_step_index(const amc_handle *h);
  * states are bit-identical -- the check that replaces reading 8 GB of state back at 100 M particles. */
 int amc_state_digest(amc_handle *h, uint64_t out[3]);
 
+/* Field sampling: per-cell moments of the particle state, accumulated on the device.  The sampling grid is the
+ * handle's collision-cell grid (a slab handle: the global grid, x and y of its own tables, z of gz_edge); a particle
+ * goes to the cell with edge[a][k] <= v < edge[a][k+1] on every axis (the owner cell of the sort), cells are numbered
+ * x-major, z-minor, and a particle outside the grid on any axis only counts in n_outside.  Ghost copies of a slab
+ * handle are skipped, so the element-wise sum (mod 2^64) of the raw arrays of all ranks equals the single-domain
+ * run's array bit for bit.  Per cell AMC_SAMPLE_WORDS uint64 words:
+ *   [0] particles;  [1..6] sum vx, sum vy, sum vz;  [7..12] sum vx^2, sum vy^2, sum vz^2 (fp64 products)
+ * every sum as two signed 64-bit fixed-point limbs (high, low): one particle adds i1 = rint(v * 2^S1) to the high
+ * limb and i2 = rint((v - i1 * 2^-S1) * 2^S2) to the low limb (round half to even), S1/S2 = AMC_SAMPLE_V1/_V2 for
+ * the velocities and AMC_SAMPLE_Q1/_Q2 for the squares; the sum decodes as high * 2^-S1 + low * 2^-S2.  Integer
+ * adds make the words independent of thread order and of the split of the particles over ranks.  Headroom: 10^6
+ * samples x 10^3 particles per cell at |v| <= 10^4 m/s keep every limb inside the signed 64-bit range (worst case:
+ * 5.2e18 in a velocity high limb, 6.4e18 in a square high limb, 5.4e17 in a low limb).
+ * A sample is taken on the state at the end of a timestep (what amc_get_state returns after amc_step): by amc_step /
+ * amc_slab_step after every step whose index s (amc_get_step_index numbering) has s >= first_step and
+ * (s - first_step) % every == 0, and by amc_sample_now.  Sampling changes no state, counter, histogram or digest;
+ * while it is disabled (the default) no launch and no memory is added.  Memory: 8 * AMC_SAMPLE_WORDS bytes per cell.
+ *   amc_sample_enable   allocate and zero the accumulators; every = 0: on demand only (amc_sample_now)
+ *   amc_sample_disable  free them
+ *   amc_sample_get_raw  acc: [cells][AMC_SAMPLE_WORDS] (nullable), samples taken, particles outside the grid
+ *   amc_sample_set_raw  resume from amc_sample_get_raw's values (sampling must be enabled)
+ *   amc_last_sample_ms  device time of the sampling kernel, summed over the samples of the last amc_step /
+ *                       amc_slab_step / amc_sample_now call (the sample is part of [3] of amc_last_timing) */
+#define AMC_SAMPLE_WORDS 13
+#define AMC_SAMPLE_V1 19
+#define AMC_SAMPLE_V2 49
+#define AMC_SAMPLE_Q1 6
+#define AMC_SAMPLE_Q2 36
+int amc_sample_enable(amc_handle *h, int32_t every, int64_t first_step);
+int amc_sample_disable(amc_handle *h);
+int amc_sample_now(amc_handle *h);
+int amc_sample_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_samples, uint64_t *n_outside);
+int amc_sample_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_samples, uint64_t n_outside);
+int amc_last_sample_ms(amc_handle *h, double *ms);
+
 /* set the step counter that keys the device RNG (default: counts amc_step / amc_walls calls from 0) */
 int amc_set_step_index(amc_handle *h, int64_t step);
 
