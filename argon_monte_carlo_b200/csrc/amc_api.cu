@@ -44,12 +44,9 @@ struct amc_handle {
     int n_buckets = 0;          // padded owner cells + OUT
     bool have_prior = false;
     int64_t step_index = 0;
-    int pdl = 3;                // programmatic dependent launches (launch_pdl; AMC_PDL=0 turns them off)
     int pair_grid = 148 * 5;    // persistent CTAs of k_pairs_group: SMs x resident CTAs per SM
     int pair_grid_fused = 148;  // the same for the fused (in-kernel hand-over) variant
-    int det_grid = 148 * 4;     // persistent CTAs of k_detect
     int det_grid_tma = 148 * 4; // persistent CTAs of k_detect_tma
-    int detect_tma = 2;         // 2 (default) / 1: the two shapes of k_detect_tma (8 CTAs x 128 threads / AMC_DETECT=tma6: 6 x 192), 0: k_detect<false> (AMC_DETECT=ldg)
     int32_t sweep_pass = 0;     // tag of the last pass of the event-driven cube sweep (P::sw_pass)
     // host-RNG parity mode: pending hits of the last amc_wall_hits_pending call
     int32_t *d_pend_count = nullptr, *d_pend_slot = nullptr, *d_pend_id = nullptr;
@@ -61,10 +58,10 @@ struct amc_handle {
     // timing
     std::vector<cudaEvent_t> events;
     double last_ms[5] = {0, 0, 0, 0, 0};
-    std::vector<cudaEvent_t> det_events; // two per step of the last amc_step chunk: around k_detect
+    std::vector<cudaEvent_t> det_events; // two per step of the last amc_step chunk: around k_detect_tma
     int det_slot = -1;                   // step of the chunk run_pairs is recording for (-1: none)
     int slab_phase = 0;                  // slab mode: PH_* bits of the step between amc_slab_advect and amc_slab_sort
-    bool slab_det_pending = false;       // slab mode: events around k_detect recorded, not yet read
+    bool slab_det_pending = false;       // slab mode: events around k_detect_tma recorded, not yet read
     double last_detect_ms = 0;
     std::vector<cudaEvent_t> sc_events;  // two per step of the last amc_step chunk: around k_scatter_advect
     double last_scatter_ms = 0;
@@ -329,19 +326,16 @@ static int create_impl(amc_handle *h, const amc_config *cfg, int device)
         p.det_thr = std::nextafterf((float)thr, INFINITY);
         p.det_w = std::nextafterf((float)(1.05 * std::sqrt((double)p.det_thr)), INFINITY);
     }
-    {
-        // serial sweep of the cube stage: event-driven unless AMC_CUBE_SWEEP=serial asks for the plain one-CTA walk over
-        // every cell (kept as the cross-check and as the fall-back for a column that overflows its list)
-        const char *mode = getenv("AMC_CUBE_SWEEP");
-        if (cfg->pp_mode == AMC_PP_SWEEP && !(mode && strcmp(mode, "serial") == 0)) {
-            const int64_t ncols = (int64_t)cfg->nc[0] * cfg->nc[1];
-            p.sw_colcap = (int32_t)std::min<int64_t>(h->cap, std::max<int64_t>(512, 6 * h->cap / ncols + 64));
-            if (const char *cc = getenv("AMC_SWEEP_COLCAP")) p.sw_colcap = std::max(1, atoi(cc)); /* tests: force the hand-over to the plain sweep */
-            ALLOC(p.sw_col, (size_t)ncols * p.sw_colcap); ALLOC(p.sw_col_n, ncols);
-            ALLOC(p.sw_tag, h->cap); ALLOC(p.sw_ml, h->cap); ALLOC(p.sw_xs, h->cap); ALLOC(p.sw_ys, h->cap);
-            ALLOC(p.sw_state, 2);
-            CK(cudaMemset(p.sw_tag, 0, h->cap * sizeof(int32_t)));
-        }
+    if (cfg->pp_mode == AMC_PP_SWEEP) {
+        // event-driven serial sweep of the cube stage; the plain one-CTA walk over every cell (k_cube_sweep) takes
+        // over a pass in which a column overflows its list
+        const int64_t ncols = (int64_t)cfg->nc[0] * cfg->nc[1];
+        p.sw_colcap = (int32_t)std::min<int64_t>(h->cap, std::max<int64_t>(512, 6 * h->cap / ncols + 64));
+        if (const char *cc = getenv("AMC_SWEEP_COLCAP")) p.sw_colcap = std::max(1, atoi(cc)); /* tests: force the hand-over to the plain sweep */
+        ALLOC(p.sw_col, (size_t)ncols * p.sw_colcap); ALLOC(p.sw_col_n, ncols);
+        ALLOC(p.sw_tag, h->cap); ALLOC(p.sw_ml, h->cap); ALLOC(p.sw_xs, h->cap); ALLOC(p.sw_ys, h->cap);
+        ALLOC(p.sw_state, 2);
+        CK(cudaMemset(p.sw_tag, 0, h->cap * sizeof(int32_t)));
     }
     p.esc_cap = (int32_t)std::min<int64_t>(std::max<int64_t>(h->cap / 64, 4096), 1 << 22);
     ALLOC(p.esc_count, 1); ALLOC(p.esc_slot, p.esc_cap); ALLOC(p.esc_cell, (size_t)p.esc_cap * 8); ALLOC(p.esc_next, (size_t)p.esc_cap * 8);
@@ -369,23 +363,10 @@ static int create_impl(amc_handle *h, const amc_config *cfg, int device)
             h->pair_grid_fused = std::max(1, sms * std::max(per_sm_fused, 1));
         }
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pairs_group<false>, PAIR_THREADS, 0));
-        if (const char *pc = getenv("AMC_PAIR_CTAS")) per_sm = std::max(1, std::min(per_sm, atoi(pc))); /* experiments: fewer CTAs per SM than fit */
         h->pair_grid = std::max(1, sms * std::max(per_sm, 1));
-        CK(cudaFuncSetAttribute(k_detect<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_detect<false>, DET_THREADS, 0));
-        h->det_grid = std::max(1, sms * std::max(per_sm, 1));
-        if (const char *pd = getenv("AMC_PDL")) h->pdl = atoi(pd); /* bit 0: colour groups 1-7 behind the group before, bit 1: k_scan_sums / k_scan_add behind k_scan_tiles; 0 = plain launches (A/B) */
-        const char *dm = getenv("AMC_DETECT");
-        h->detect_tma = dm && strcmp(dm, "ldg") == 0 ? 0 : (dm && strcmp(dm, "tma6") == 0 ? 1 : 2);
-        if (h->detect_tma == 1) {
-            CK(cudaFuncSetAttribute(k_detect_tma<192, 2, 6, 64, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_detect_tma<192, 2, 6, 64, 1>, 192, 0));
-        } else if (h->detect_tma == 2) {
-            CK(cudaFuncSetAttribute(k_detect_tma<128, 3, 8, 32, 2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_detect_tma<128, 3, 8, 32, 2>, 128, 0));
-        }
+        CK(cudaFuncSetAttribute(k_detect_tma<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_detect_tma<false>, DET_THREADS, 0));
         h->det_grid_tma = std::max(1, sms * std::max(per_sm, 1));
-        if (getenv("AMC_DEBUG")) fprintf(stderr, "amc: detect mode %d, %d CTAs per SM\n", h->detect_tma, per_sm);
         ALLOC(p.mv_spill, (size_t)std::max(h->pair_grid, 1) * AMC_MAX_MEMBERS * 3);
     }
     CK(cudaDeviceSynchronize());
@@ -520,7 +501,7 @@ static int sort_scatter(amc_handle *h, int64_t *launches)
 }
 
 // bookkeeping of one pair pass that depends on the sorted layout only through cell_start / band_count (not on the
-// particle arrays): reset of the escaped list and of the worklists, list of the cells k_detect has to look at
+// particle arrays): reset of the escaped list and of the worklists, list of the cells k_detect_tma has to look at
 static int prepare_pairs(amc_handle *h, cudaStream_t st)
 {
     P &p = h->p;
@@ -534,14 +515,10 @@ static int prepare_pairs(amc_handle *h, cudaStream_t st)
     return AMC_OK;
 }
 
-// the detection pass of a timestep: candidates staged by bulk copies (k_detect_tma, the default; measured on B200 at
-// 12.5 M particles: 0.1845 ms in the 8-CTA shape, 0.1975 ms in the 6-CTA shape) or loaded by the threads
-// (k_detect<false>, AMC_DETECT=ldg, 0.1851 ms: kept as the cross-check)
+// the detection pass of a timestep: candidates staged by bulk copies (DESIGN section 5)
 static void launch_detect(amc_handle *h)
 {
-    if (h->detect_tma == 1) k_detect_tma<192, 2, 6, 64, 1><<<h->det_grid_tma, 192, 0, h->stream>>>(h->p);
-    else if (h->detect_tma == 2) k_detect_tma<128, 3, 8, 32, 2><<<h->det_grid_tma, 128, 0, h->stream>>>(h->p);
-    else k_detect<false><<<h->det_grid, DET_THREADS, 0, h->stream>>>(h->p);
+    k_detect_tma<false><<<h->det_grid_tma, DET_THREADS, 0, h->stream>>>(h->p);
 }
 
 // launch `kernel` programmatically dependent on the kernel before it in the stream (griddepcontrol, see pdl_trigger /
@@ -561,22 +538,19 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, c
 static int run_pairs(amc_handle *h, int64_t *launches, bool prepared = false)
 {
     P &p = h->p;
-    if (p.pp_mode == AMC_PP_SWEEP) {
-        if (p.sw_col) { /* event-driven sweep: detection over all columns, then the flagged cells in sweep order */
-            if (h->sweep_pass == 0x7fffffff) { /* pass tags exhausted: start over with clean tags */
-                CK(cudaMemsetAsync(p.sw_tag, 0, h->cap * sizeof(int32_t), h->stream));
-                h->sweep_pass = 0;
-            }
-            p.sw_pass = ++h->sweep_pass;
-            const int ncell = p.nc[0] * p.nc[1] * p.nc[2];
-            CK(cudaMemsetAsync(p.cell_active, 0, (size_t)((ncell + 31) / 32) * sizeof(int32_t), h->stream));
-            CK(cudaMemsetAsync(p.sw_state, 0, 2 * sizeof(unsigned long long), h->stream));
-            k_sweep_detect<<<p.nc[0] * p.nc[1], SWD_THREADS, 0, h->stream>>>(p);
-            k_sweep_events<<<1, SWE_THREADS, 0, h->stream>>>(p);
-            if (launches) *launches += 2;
+    if (p.pp_mode == AMC_PP_SWEEP) { /* event-driven sweep: detection over all columns, then the flagged cells in sweep order */
+        if (h->sweep_pass == 0x7fffffff) { /* pass tags exhausted: start over with clean tags */
+            CK(cudaMemsetAsync(p.sw_tag, 0, h->cap * sizeof(int32_t), h->stream));
+            h->sweep_pass = 0;
         }
-        k_cube_sweep<<<1, SWEEP_THREADS, 0, h->stream>>>(p); /* with the event-driven sweep: only when a column list overflowed */
-        if (launches) *launches += 1;
+        p.sw_pass = ++h->sweep_pass;
+        const int ncell = p.nc[0] * p.nc[1] * p.nc[2];
+        CK(cudaMemsetAsync(p.cell_active, 0, (size_t)((ncell + 31) / 32) * sizeof(int32_t), h->stream));
+        CK(cudaMemsetAsync(p.sw_state, 0, 2 * sizeof(unsigned long long), h->stream));
+        k_sweep_detect<<<p.nc[0] * p.nc[1], SWD_THREADS, 0, h->stream>>>(p);
+        k_sweep_events<<<1, SWE_THREADS, 0, h->stream>>>(p);
+        k_cube_sweep<<<1, SWEEP_THREADS, 0, h->stream>>>(p); /* returns at once unless a column list overflowed */
+        if (launches) *launches += 3;
     } else {
         if (!prepared) {
             int rc = prepare_pairs(h, h->stream);
@@ -587,22 +561,21 @@ static int run_pairs(amc_handle *h, int64_t *launches, bool prepared = false)
         launch_detect(h);
         if (h->det_slot >= 0) CK(cudaEventRecord(h->det_events[2 * h->det_slot + 1], h->stream));
         unsigned grid = (unsigned)std::min<int64_t>((int64_t)h->pair_grid, std::max<int64_t>(ncell / 8, 1));
-        for (int g = 0; g < 8; g++) {
-            if (g > 0 && (h->pdl & 1)) CK(launch_pdl(k_pairs_group<false>, dim3(grid), dim3(PAIR_THREADS), h->stream, p, g));
-            else k_pairs_group<false><<<grid, PAIR_THREADS, 0, h->stream>>>(p, g);
-        }
+        k_pairs_group<false><<<grid, PAIR_THREADS, 0, h->stream>>>(p, 0);
+        for (int g = 1; g < 8; g++) CK(launch_pdl(k_pairs_group<false>, dim3(grid), dim3(PAIR_THREADS), h->stream, p, g));
         if (launches) *launches += 11;
     }
     CK(cudaGetLastError());
     return AMC_OK;
 }
 
-static int ensure_events(amc_handle *h, size_t count)
+// grow one of the handle's event pools to `count` events
+static int ensure_events(amc_handle *h, std::vector<cudaEvent_t> &pool, size_t count)
 {
-    while (h->events.size() < count) {
+    while (pool.size() < count) {
         cudaEvent_t e;
         CK(cudaEventCreate(&e));
-        h->events.push_back(e);
+        pool.push_back(e);
     }
     return AMC_OK;
 }
@@ -623,11 +596,8 @@ static void sample_reset_timing(amc_handle *h)
 // grid_n: slots the launch covers; launches (nullable) counts the kernel launch
 static int launch_sample(amc_handle *h, int64_t grid_n, int64_t *launches)
 {
-    while (h->sample_events.size() < (size_t)(2 * h->sample_slot + 2)) {
-        cudaEvent_t e;
-        CK(cudaEventCreate(&e));
-        h->sample_events.push_back(e);
-    }
+    int rc = ensure_events(h, h->sample_events, (size_t)(2 * h->sample_slot + 2));
+    if (rc != AMC_OK) return rc;
     const P &p = h->p;
     SampleArgs sa;
     sa.acc = h->d_sample;
@@ -757,18 +727,10 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
     }
     while (done < n_steps) {
         int chunk = std::min(n_steps - done, h->stats_cap);
-        int rc = ensure_events(h, (size_t)chunk * 4 + 1);
-        if (rc != AMC_OK) return rc;
-        while (h->det_events.size() < (size_t)chunk * 2) {
-            cudaEvent_t e;
-            CK(cudaEventCreate(&e));
-            h->det_events.push_back(e);
-        }
-        while (h->sc_events.size() < (size_t)chunk * 2) {
-            cudaEvent_t e;
-            CK(cudaEventCreate(&e));
-            h->sc_events.push_back(e);
-        }
+        int rc;
+        if ((rc = ensure_events(h, h->events, (size_t)chunk * 4 + 1)) != AMC_OK) return rc;
+        if ((rc = ensure_events(h, h->det_events, (size_t)chunk * 2)) != AMC_OK) return rc;
+        if ((rc = ensure_events(h, h->sc_events, (size_t)chunk * 2)) != AMC_OK) return rc;
         CK(cudaMemsetAsync(h->d_stats, 0, chunk * sizeof(StatsDev), h->stream));
         CK(cudaEventRecord(h->events[0], h->stream));
         bool closed_prev = true; // the step before this one ended with its own recapture launch
@@ -793,13 +755,8 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
                     CK(cudaEventRecord(h->events[4 * s + 1], h->stream));
                     int m = h->n_buckets, ntiles = (m + SCAN_TILE - 1) / SCAN_TILE;
                     k_scan_tiles<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.band_count, p.rest_count, p.cell_start, h->d_tile_sums, m);
-                    if (h->pdl & 2) {
-                        CK(launch_pdl(k_scan_sums, dim3(1), dim3(SCAN_THREADS), h->stream, h->d_tile_sums, ntiles));
-                        CK(launch_pdl(k_scan_add, dim3(ntiles), dim3(SCAN_THREADS), h->stream, p.cell_start, (const int32_t *)h->d_tile_sums, m, (int32_t)h->n));
-                    } else {
-                        k_scan_sums<<<1, SCAN_THREADS, 0, h->stream>>>(h->d_tile_sums, ntiles);
-                        k_scan_add<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.cell_start, h->d_tile_sums, m, (int32_t)h->n);
-                    }
+                    CK(launch_pdl(k_scan_sums, dim3(1), dim3(SCAN_THREADS), h->stream, h->d_tile_sums, ntiles));
+                    CK(launch_pdl(k_scan_add, dim3(ntiles), dim3(SCAN_THREADS), h->stream, p.cell_start, (const int32_t *)h->d_tile_sums, m, (int32_t)h->n));
                     // the bookkeeping of the pair pass needs the scan, not the scattered particles: it runs beside the scatter
                     CK(cudaEventRecord(h->ev_fork, h->stream));
                     CK(cudaStreamWaitEvent(h->aux, h->ev_fork, 0));
@@ -959,7 +916,7 @@ extern "C" int amc_seed_relax(amc_handle *h, int32_t max_rounds, int64_t *n_redr
         if ((rc = sort_scatter(h, nullptr)) != AMC_OK) return rc;
         if ((rc = prepare_pairs(h, h->stream)) != AMC_OK) return rc;
         CK(cudaMemsetAsync(p.rank, 0, h->n * sizeof(int32_t), h->stream));
-        k_detect<true><<<h->det_grid, DET_THREADS, 0, h->stream>>>(p);
+        k_detect_tma<true><<<h->det_grid_tma, DET_THREADS, 0, h->stream>>>(p);
         if (round < max_rounds) k_seed_redraw<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, h->init_spec, (uint32_t)(round + 1));
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(h->h_stats, h->d_stats, sizeof(StatsDev), cudaMemcpyDeviceToHost, h->stream));
@@ -1387,15 +1344,8 @@ extern "C" int amc_slab_pairs_begin(amc_handle *h, int32_t pre_round)
     if (rc != AMC_OK) return rc;
     P &p = h->p;
     p.group_done = -1;
-    k_pp_begin<<<1, 256, 0, h->stream>>>(p);
-    CK(cudaMemsetAsync(p.wl_count, 0, AMC_WL_COUNTERS * sizeof(int32_t), h->stream));
-    int ncell = p.nc[0] * p.nc[1] * p.nc[2];
-    CK(cudaMemsetAsync(p.cell_active, 0, (size_t)p.wl_stride * 8 * sizeof(int32_t), h->stream));
-    CK(cudaMemsetAsync(p.cell_n, 0, (size_t)p.wl_stride * 8 * sizeof(int32_t), h->stream));
-    k_build_worklist<<<grid_for(ncell, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p);
-    if (h->det_events.size() < 2) {
-        for (int k = 0; k < 2; k++) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->det_events.push_back(e); }
-    }
+    if ((rc = prepare_pairs(h, h->stream)) != AMC_OK) return rc;
+    if ((rc = ensure_events(h, h->det_events, 2)) != AMC_OK) return rc;
     CK(cudaEventRecord(h->det_events[0], h->stream));
     if (h->n) launch_detect(h);
     CK(cudaEventRecord(h->det_events[1], h->stream));
@@ -1602,12 +1552,8 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
         // the count changes by a few hundred per step (migration); the launches of this chunk cover a generous bound
         p.n_hint = std::min<int64_t>(h->cap, h->n + h->n / 32 + 2 * (int64_t)h->xf_total + 4 * (int64_t)p.foreign_cap);
         const unsigned full = grid_for(p.n_hint, ADVECT_THREADS);
-        if ((rc = ensure_events(h, (size_t)chunk * 4 + 1)) != AMC_OK) { p.n_dev = nullptr; return rc; }
-        while (h->det_events.size() < (size_t)chunk * 2) {
-            cudaEvent_t e;
-            CK(cudaEventCreate(&e));
-            h->det_events.push_back(e);
-        }
+        if ((rc = ensure_events(h, h->events, (size_t)chunk * 4 + 1)) != AMC_OK) { p.n_dev = nullptr; return rc; }
+        if ((rc = ensure_events(h, h->det_events, (size_t)chunk * 2)) != AMC_OK) { p.n_dev = nullptr; return rc; }
         CK(cudaMemsetAsync(h->d_stats, 0, chunk * sizeof(StatsDev), h->stream));
         CK(cudaEventRecord(h->events[0], h->stream));
         for (int s = 0; s < chunk; s++) {
@@ -1642,7 +1588,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
             launch_detect(h);
             CK(cudaEventRecord(h->det_events[2 * s + 1], h->stream));
             h->last_launches += 12;
-            if (p.nranks > 1 && pgrid >= 2 * BND_HEAD_CTAS && !getenv("AMC_SLAB_UNFUSED")) {
+            if (p.nranks > 1 && pgrid >= 2 * BND_HEAD_CTAS) {
                 // the hand-over rides inside the group launches (k_pairs_group, fused): records of group g are sent by the
                 // last CTA of launch g and applied at the head of launch g + 1 while the cells away from the cuts run
                 uint32_t prev = 0;
@@ -1652,7 +1598,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
                     h->last_launches += 1;
                 }
                 const bool trace = getenv("AMC_SLAB_TRACE") && s == chunk - 1;
-                if (trace) while (h->grp_events.size() < 10) { cudaEvent_t e; CK(cudaEventCreate(&e)); h->grp_events.push_back(e); }
+                if (trace && (rc = ensure_events(h, h->grp_events, 10)) != AMC_OK) { p.n_dev = nullptr; return rc; }
                 for (int g = 0; g < 8; g++) {
                     p.bnd_seq_apply = prev;
                     p.bnd_seq = ++h->bnd_seq;

@@ -4,13 +4,12 @@
 //   k_scatter_advect  the timestep itself on the way to the sorted slot                         (HBM streaming)
 //   k_build_worklist  reference cells with >= 2 candidates -> detection list                    (tiny)
 //   k_detect_tma      neighbour search over every reference cell, all colour groups at once; candidates staged by
-//                     cp.async.bulk + mbarrier                                                   (issue; 33 B/particle)
-//   k_detect          the same with the candidates loaded by the threads (cross-check; <true>: overlap-free seeding)
+//                     cp.async.bulk + mbarrier; <true>: overlap-free seeding                     (issue; 33 B/particle)
 //   k_pairs_group     ordered resolution of the flagged / activated cells of one colour group   (latency)
 //   k_recapture_list  closing recapture over the slots a collision touched                      (tiny)
 //   k_advect, k_scatter, k_recapture_post   the same step as separate in-place passes: phase-level parity entry points
 //   k_sweep_detect, k_sweep_events   the serial lexicographic cell sweep of the cube stage, event-driven  (latency)
-//   k_cube_sweep      the same sweep as a plain walk over every cell (cross-check, fall-back)   (latency)
+//   k_cube_sweep      the same sweep as a plain walk over every cell (fall-back when a column list overflows)  (latency)
 //   k_pack_pos, k_unpack_pos   the C ABI's separate arrays <-> the 32-byte position records
 //   k_case_*          per-case wall kernels for the host-RNG parity mode
 //   k_init_synthetic  synthetic Maxwellian initial state
@@ -19,20 +18,12 @@
 #include "amc_device.cuh"
 
 #define ADVECT_THREADS 256
-#ifndef PAIR_THREADS
 #define PAIR_THREADS 128
-#endif
 #define AMC_MV_CAP 32 /* particles one cell visit can move (reference scale: 2-6) */
 #define WALK_K 3 /* chains a thread of cell_process walks side by side */
-#ifndef PAIR_K
 #define PAIR_K 3 /* candidates a thread of k_pairs_group has in flight during the gather */
-#endif
-#ifndef PAIR_OCC
 #define PAIR_OCC 6 /* resident CTAs per SM of k_pairs_group: a colour-group launch lasts one visit if the group's worklist fits the grid, two if not */
-#endif
-#ifndef SWEEP_THREADS
 #define SWEEP_THREADS 512
-#endif
 
 // Programmatic dependent launch (griddepcontrol; SASS PREEXIT / ACQBULK): a kernel launched with
 // cudaLaunchAttributeProgrammaticStreamSerialization may become resident while the kernel before it in the stream still
@@ -1157,32 +1148,28 @@ __global__ void __launch_bounds__(ADVECT_THREADS) k_build_worklist(const __grid_
 // rounding bound (det_thr, amc_api.cu), and anything unusual (more candidates than the CTA holds, a
 // full slab) flags the cell.  False positives cost one exact visit; misses are impossible.
 //
-// Per cell: candidates are streamed from HBM once (24 B each; the loads of the NEXT cell are in flight
-// while the current one is searched).  Members are hashed into a 2-D table of bins over (x, y), each
-// >= 1.05 filter radii wide: at gas density a bin holds 0.07 particles, so a member only looks at its own
-// bin and the four forward neighbours and almost never finds anything to test.  Table entries carry the
-// visit number in their upper half, so the table is never cleared.  Two barriers per cell.
+// Per cell: the candidates are 8 runs of consecutive position records (the owner cell, the band prefixes of its 7
+// low-side neighbours), so the header warp hands each run to cp.async.bulk (one 1-D bulk copy per run, SASS UBLKCP) and
+// the records land in shared memory while the CTA searches the previous cell; an mbarrier with a transaction count tells
+// the CTA when all of them are there.  No thread computes a candidate's slot (det_slot) or issues a global load for it,
+// and nothing of the next cell lives in registers during the search.  Members are hashed into a 2-D table of bins over
+// (x, y), >= 1.05 filter radii wide along x and twice that along y: at gas density a bin holds about 0.14 particles,
+// so a member only looks at its own bin and the four forward neighbours and almost never finds anything to test.
+// Table entries carry the visit number in their upper half, so the table is never cleared.  Two barriers per cell.
+// 128 threads x 3 candidates at 64 registers and 27.9 KB of shared memory: 8 CTAs per SM.
 #define DET_THREADS 128
 #define DET_K 3     /* candidates per thread: cells with more than DET_K * DET_THREADS candidates are flagged */
 #define DET_CAND (DET_K * DET_THREADS)
-#ifndef DET_NB
 #define DET_NB 64   /* bins along x, at most */
-#endif
-#ifndef DET_NBY
-#define DET_NBY 64  /* bins along y, at most */
-#define DET_YF 1.0f /* width of a y bin in units of the minimal bin width */
-#endif
-#ifndef DET_OCC
 #define DET_OCC 8   /* resident CTAs per SM the kernel is compiled for */
-#endif
-#define DET_ROW (DET_NBY + 2)               /* one empty bin on either side of a row */
-#define DET_TAB ((DET_NB + 1) * DET_ROW)    /* one empty row behind the last */
 
 struct DetShared {
-    static constexpr int NBX = DET_NB, NBY = DET_NBY, ROW = DET_ROW;
-    static constexpr float YF = DET_YF;
-    unsigned int head[DET_TAB];      /* (visit tag << 16) | (candidate index + 1) of the last member hashed into the bin */
+    static constexpr int NBX = DET_NB, NBY = 32;           /* bins along x / y, at most */
+    static constexpr float YF = 2.0f;                       /* width of a y bin in units of the minimal bin width */
+    static constexpr int ROW = NBY + 2, TAB = (NBX + 1) * ROW; /* one empty bin on either side of a row, one empty row behind the last */
+    unsigned int head[TAB];          /* (visit tag << 16) | (candidate index + 1) of the last member hashed into the bin */
     float4 tile[DET_CAND];           /* by candidate index: cell-relative fp32 position; .w = older member of the same bin (index + 1 as integer bits), 0 = none */
+    __align__(128) PosRec raw[DET_CAND]; /* records of the cell about to be searched: written by the bulk copies only */
     __align__(16) int hdr[2][AMC_WI];
     int rbeg[2][8], rcum[2][9];
     float inv_wx[2], inv_wy[2];
@@ -1190,11 +1177,11 @@ struct DetShared {
     int nmem[2];
     int nhit[2];
     unsigned int hit[2][AMC_MAX_HITS]; /* candidate indices of the pairs that passed the filter: (self << 16) | other */
+    __align__(8) unsigned long long bar; /* mbarrier: one arrival (the header warp's expect_tx) + the bytes of the copies */
 };
 
 // header warp: make the work item `v` (one int per lane) the header in buffer `buf`
-template <class SH>
-__device__ __forceinline__ void det_publish(const P &p, SH &S, int buf, int v, int lane)
+__device__ __forceinline__ void det_publish(const P &p, DetShared &S, int buf, int v, int lane)
 {
     S.hdr[buf][lane] = v;
     __syncwarp();
@@ -1207,7 +1194,7 @@ __device__ __forceinline__ void det_publish(const P &p, SH &S, int buf, int v, i
         if (lane < 2) { /* lane 0: bins along x, lane 1: along y */
             const double *d = reinterpret_cast<const double *>(&S.hdr[buf][20]);
             float wd = (float)(d[2 * lane + 1] - d[2 * lane]);
-            int nb = lane == 0 ? (int)fminf((float)SH::NBX, floorf(wd / p.det_w)) : (int)fminf((float)SH::NBY, floorf(wd / (SH::YF * p.det_w)));
+            int nb = lane == 0 ? (int)fminf((float)DetShared::NBX, floorf(wd / p.det_w)) : (int)fminf((float)DetShared::NBY, floorf(wd / (DetShared::YF * p.det_w)));
             if (nb < 1) nb = 1;
             if (lane == 0) { S.nbx[buf] = nb; S.inv_wx[buf] = (float)nb / wd; S.rcum[buf][0] = 0; }
             else { S.nby[buf] = nb; S.inv_wy[buf] = (float)nb / wd; }
@@ -1217,8 +1204,7 @@ __device__ __forceinline__ void det_publish(const P &p, SH &S, int buf, int v, i
 
 // slot of candidate t of the work item in buffer `buf`: the owner cell's own particles first, then the
 // band prefixes of the 7 low-side neighbours
-template <class SH>
-__device__ __forceinline__ int det_slot(const SH &S, int buf, int t)
+__device__ __forceinline__ int det_slot(const DetShared &S, int buf, int t)
 {
     if (t < S.rcum[buf][1]) return S.rbeg[buf][0] + t;
     int nb = 1;
@@ -1235,8 +1221,8 @@ __device__ __noinline__ void det_seed_mark(const P &p, const int sa, const int s
     if (overlap(p, A.pos[sa].x, A.pos[sa].y, A.pos[sa].z, A.pos[sb].x, A.pos[sb].y, A.pos[sb].z))
         if (atomicExch(&p.rank[A.pos[sa].id > A.pos[sb].id ? sa : sb], 1) == 0) atomicAdd(&p.stats->pp, 1ull);
 }
-// A cell with more candidates than the table holds is searched pair by pair on the fp64 positions (one-time work at
-// initialisation; the timestep leaves such cells to the ordered resolution).
+// A cell with more candidates than the tile holds is not copied; seeding searches it pair by pair on the fp64 positions
+// (one-time work at initialisation; the timestep leaves such cells to the ordered resolution).
 __device__ __noinline__ void det_seed_big_cell(const P &p, const DetShared &S, const int cur, const int total)
 {
     const Arrays &A = p.a;
@@ -1255,53 +1241,95 @@ __device__ __noinline__ void det_seed_big_cell(const P &p, const DetShared &S, c
     }
 }
 
-template <bool SEED> /* SEED: the marking variant of amc_seed_relax; the detection pass of a timestep is k_detect<false> */
-__global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect(const __grid_constant__ P p)
+__device__ __forceinline__ uint32_t smem_u32(const void *q) { return (uint32_t)__cvta_generic_to_shared(q); }
+__device__ __forceinline__ void mbar_init(unsigned long long *bar, const int count)
+{
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, const uint32_t bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, const uint32_t bytes, unsigned long long *bar)
+{
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+                 "l"(__cvta_generic_to_global(src)), "r"(bytes), "r"(smem_u32(bar))
+                 : "memory");
+}
+// false when the phase did not complete within ~1 s (a byte count that does not match the copies): the caller reports it
+__device__ __forceinline__ bool mbar_wait(unsigned long long *bar, const uint32_t parity)
+{
+    for (unsigned int spins = 0; spins < (1u << 22); spins++) {
+        uint32_t ok;
+        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
+                     : "=r"(ok)
+                     : "r"(smem_u32(bar)), "r"(parity)
+                     : "memory");
+        if (ok) return true;
+    }
+    return false;
+}
+
+// header warp: start the bulk copies of the candidates of the work item in header buffer `buf` (published and
+// barrier-separated from here).  A cell with more candidates than the tile holds is not copied: it is flagged unseen.
+__device__ __forceinline__ void det_fetch(const P &p, DetShared &S, const int buf, const int lane)
+{
+    const int total = S.rcum[buf][8];
+    const bool fits = total <= DET_CAND;
+    if (lane == 0) {
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); /* the threads' reads of S.raw (behind a barrier) before the engine's writes */
+        mbar_expect_tx(&S.bar, fits ? (uint32_t)total * (uint32_t)sizeof(PosRec) : 0u);
+    }
+    __syncwarp();
+    if (fits && lane < 8) {
+        const int beg = S.rcum[buf][lane], len = S.rcum[buf][lane + 1] - beg;
+        if (len > 0) bulk_g2s(&S.raw[beg], p.a.pos + S.rbeg[buf][lane], (uint32_t)len * (uint32_t)sizeof(PosRec), &S.bar);
+    }
+}
+
+template <bool SEED> /* SEED: the marking variant of amc_seed_relax; the detection pass of a timestep is k_detect_tma<false> */
+__global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect_tma(const __grid_constant__ P p)
 {
     __shared__ DetShared S;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const Arrays &A = p.a;
     const int nwork = *p.dl_count;
     const int stride = gridDim.x;
     int w = blockIdx.x;
     if (w >= nwork) return;
-    for (int c = tid; c < DET_TAB; c += DET_THREADS) S.head[c] = 0;
+    for (int c = tid; c < DetShared::TAB; c += DET_THREADS) S.head[c] = 0;
     if (tid < 2) { S.nmem[tid] = 0; S.nhit[tid] = 0; }
-    // the header bookkeeping rides on the last warp: it has the fewest candidates to handle (the tail of the list)
-    const bool hw = warp == DET_THREADS / 32 - 1;
-    int hn = 0; /* header warp: the work item after the one published in the other buffer */
+    if (tid == 0) mbar_init(&S.bar, 1);
+    const bool hw = warp == DET_THREADS / 32 - 1; /* header warp: the tail of the candidate list, least to do */
+    int hn = 0;
     if (hw) {
         det_publish(p, S, 0, p.dl[(size_t)w * AMC_WI + lane], lane);
         if (w + stride < nwork) hn = p.dl[(size_t)(w + stride) * AMC_WI + lane];
     }
     __syncthreads();
-    double cx[DET_K], cy[DET_K], cz[DET_K];
-#pragma unroll
-    for (int k = 0; k < DET_K; k++) {
-        int t = tid + k * DET_THREADS;
-        if (t < S.rcum[0][8]) {
-            int s = det_slot(S, 0, t);
-            const PosRec r = A.pos[s];
-            cx[k] = r.x; cy[k] = r.y; cz[k] = r.z;
-        }
-    }
+    if (hw) det_fetch(p, S, 0, lane);
     unsigned int tests = 0;
     unsigned long long nref = 0; /* header warp, lane 0 */
     const float thr = p.det_thr;
     unsigned int tagw = 0;
+    uint32_t phase = 0;
+    bool stuck = false;
     for (int it = 0; w < nwork; it++, w += stride) {
         const int cur = it & 1, nxt = cur ^ 1;
         tagw += 0x10000u;
-        if (tagw == 0) { /* visit tags exhausted (65535 cells in this CTA): start over with a clean table */
+        if (tagw == 0) { /* visit tags exhausted: start over with a clean table */
             __syncthreads();
-            for (int c = tid; c < DET_TAB; c += DET_THREADS) S.head[c] = 0;
+            for (int c = tid; c < DetShared::TAB; c += DET_THREADS) S.head[c] = 0;
             tagw = 0x10000u;
             __syncthreads();
         }
-        // ---- hash the members of the current cell
         const int total = S.rcum[cur][8];
-        bool hit = total > DET_CAND;
-        if (SEED && hit) det_seed_big_cell(p, S, cur, total);
+        const bool big = total > DET_CAND;
+        bool hit = big;
+        if (SEED && big) det_seed_big_cell(p, S, cur, total);
+        if (!mbar_wait(&S.bar, phase)) stuck = true; /* the records of this cell are in S.raw */
+        phase ^= 1u;
+        // ---- hash the members of the current cell
         float fx[DET_K], fy[DET_K], fz[DET_K];
         int bin[DET_K], older[DET_K];
         {
@@ -1313,13 +1341,14 @@ __global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect(const __grid_co
             int nm = 0;
 #pragma unroll
             for (int k = 0; k < DET_K; k++) {
-                int t = tid + k * DET_THREADS;
+                const int t = tid + k * DET_THREADS;
                 bin[k] = -1;
-                if (t < total) {
-                    double x = cx[k], y = cy[k], z = cz[k];
+                if (t < total && !big) {
+                    const double2 xy = *reinterpret_cast<const double2 *>(&S.raw[t]);
+                    const double x = xy.x, y = xy.y, z = S.raw[t].z;
                     if (t < own || (lox < x && x < hix && loy < y && y < hiy && loz < z && z < hiz)) { /* Pore:527-530 */
                         fx[k] = (float)(x - lox); fy[k] = (float)(y - loy); fz[k] = (float)(z - loz);
-                        int b = min(nbx1, (int)(fx[k] * inv_wx)) * DET_ROW + min(nby1, (int)(fy[k] * inv_wy)) + 1;
+                        int b = min(nbx1, (int)(fx[k] * inv_wx)) * DetShared::ROW + min(nby1, (int)(fy[k] * inv_wy)) + 1;
                         unsigned int prev = atomicExch(&S.head[b], tagw | (unsigned int)(t + 1)) ^ tagw;
                         prev = prev < 0x10000u ? prev : 0u;
                         S.tile[t] = make_float4(fx[k], fy[k], fz[k], __uint_as_float(prev));
@@ -1337,22 +1366,8 @@ __global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect(const __grid_co
             if (wn + stride < nwork) hn = p.dl[(size_t)(wn + stride) * AMC_WI + lane];
         }
         __syncthreads();
-        // ---- the next cell's candidates start their trip from HBM now
-        if (wn < nwork) {
-            // all slots first, then all loads: the nine loads leave together instead of queueing behind the shared-memory
-            // reads of the next candidate's slot computation (measured: 0.217 -> 0.193 ms)
-            const int ntot = S.rcum[nxt][8];
-            int sl[DET_K];
-#pragma unroll
-            for (int k = 0; k < DET_K; k++) {
-                const int t = tid + k * DET_THREADS;
-                sl[k] = t < ntot ? det_slot(S, nxt, t) : -1;
-            }
-            const PosRec *ap = A.pos;
-#pragma unroll
-            for (int k = 0; k < DET_K; k++)
-                if (sl[k] >= 0) { const PosRec r = ap[sl[k]]; cx[k] = r.x; cy[k] = r.y; cz[k] = r.z; }
-        }
+        // ---- every thread is done with S.raw: the next cell's records start their trip from HBM now
+        if (hw && wn < nwork) det_fetch(p, S, nxt, lane);
         // ---- search: the older members of the own bin and everything in the four forward neighbour bins
 #pragma unroll
         for (int k = 0; k < DET_K; k++) {
@@ -1360,10 +1375,9 @@ __global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect(const __grid_co
             const int b = bin[k];
             unsigned int c[5];
             c[0] = (unsigned int)older[k];
-            c[1] = S.head[b + 1] ^ tagw; c[2] = S.head[b + DET_ROW - 1] ^ tagw;
-            c[3] = S.head[b + DET_ROW] ^ tagw; c[4] = S.head[b + DET_ROW + 1] ^ tagw;
+            c[1] = S.head[b + 1] ^ tagw; c[2] = S.head[b + DetShared::ROW - 1] ^ tagw;
+            c[3] = S.head[b + DetShared::ROW] ^ tagw; c[4] = S.head[b + DetShared::ROW + 1] ^ tagw;
             if (c[0] == 0 && min(min(c[1], c[2]), min(c[3], c[4])) >= 0x10000u) continue;
-            // the non-empty chains (indices < 512) are packed into one word and walked in a single loop
             unsigned long long pend = c[0];
             int sh = c[0] ? 9 : 0;
 #pragma unroll
@@ -1405,245 +1419,6 @@ __global__ void __launch_bounds__(DET_THREADS, DET_OCC) k_detect(const __grid_co
             }
         }
         if (tid == DET_THREADS - 1) { S.nmem[nxt] = 0; S.nhit[nxt] = 0; }
-        const int any = __syncthreads_or(hit);
-        if (hw) {
-            const int *h = S.hdr[cur];
-            const int cell = h[0], kx = h[1], ky = h[2], kz = h[3];
-            const int g = ((kx & 1) << 2) | ((ky & 1) << 1) | ((kz + p.zoff) & 1);
-            const size_t ci = (size_t)g * p.wl_stride + cell;
-            if (any) {
-                int idx = 0;
-                if (lane == 0) { p.cell_active[ci] = 1; idx = atomicAdd(&p.wl_count[g], 1); }
-                idx = __shfl_sync(0xffffffffu, idx, 0);
-                p.wl[((size_t)g * p.wl_stride + idx) * AMC_WI + lane] = h[lane];
-                // the pairs that passed the filter, as slots: the resolution tests just these (exactly) instead of
-                // searching the cell again; -1 = search (cell flagged for another reason, or too many pairs)
-                const int nh = S.nhit[cur];
-                const bool listed = total <= DET_CAND && nh >= 1 && nh <= AMC_MAX_HITS;
-                int32_t *wh = p.wl_hit + ((size_t)g * p.wl_stride + idx) * AMC_HIT_REC;
-                if (lane == 0) wh[0] = listed ? nh : -1;
-                if (listed && lane < 2 * nh) {
-                    const unsigned int hv = S.hit[cur][lane >> 1];
-                    wh[1 + lane] = det_slot(S, cur, (lane & 1) ? (int)(hv & 0xffffu) : (int)(hv >> 16));
-                }
-            } else if (lane == 0) {
-                const int nm = S.nmem[cur];
-                p.cell_n[ci] = nm;
-                nref += (unsigned long long)nm * (nm - 1) / 2;
-            }
-        }
-    }
-    tests = __reduce_add_sync(0xffffffffu, tests);
-    if (lane == 0 && tests) atomicAdd(&p.stats->checks_exec, (unsigned long long)tests);
-    if (hw && lane == 0 && nref) atomicAdd(&p.stats->checks_ref, nref);
-}
-
-// ------------------------------------------------------------------------------------------------
-// The same detection pass with the candidates staged by the copy engine instead of by the threads.  The candidates
-// of a reference cell are 8 runs of consecutive position records (the owner cell, the band prefixes of its 7 low-side
-// neighbours), so the header warp hands each run to cp.async.bulk (one 1-D bulk copy per run, SASS UBLKCP) and the
-// records land in shared memory while the CTA searches the previous cell; an mbarrier with a transaction count
-// tells the CTA when all of them are there.  No thread computes a candidate's slot (det_slot) or issues a global
-// load any more, and nothing of the next cell lives in registers during the search: 192 threads x 2 candidates at
-// 56 registers, 6 CTAs per SM.  Everything else -- membership, fp32 filter, bin table, results -- is k_detect's.
-// Two shapes are built (amc_api.cu picks one, AMC_DETECT): 192 threads x 2 candidates with k_detect's 64 x 64 bin table
-// (37 KB of shared memory: 6 CTAs per SM), and 128 threads x 3 candidates with y bins twice as wide (28 KB: 8 CTAs).
-template <int NBY_, int YF_>
-struct DetSharedT {
-    static constexpr int NBX = DET_NB, NBY = NBY_, ROW = NBY_ + 2, TAB = (DET_NB + 1) * (NBY_ + 2);
-    static constexpr float YF = (float)YF_;
-    unsigned int head[TAB];
-    float4 tile[DET_CAND];
-    __align__(128) PosRec raw[DET_CAND]; /* records of the cell about to be searched: written by the bulk copies only */
-    __align__(16) int hdr[2][AMC_WI];
-    int rbeg[2][8], rcum[2][9];
-    float inv_wx[2], inv_wy[2];
-    int nbx[2], nby[2];
-    int nmem[2];
-    int nhit[2];
-    unsigned int hit[2][AMC_MAX_HITS];
-    __align__(8) unsigned long long bar; /* mbarrier: one arrival (the header warp's expect_tx) + the bytes of the copies */
-};
-
-__device__ __forceinline__ uint32_t smem_u32(const void *q) { return (uint32_t)__cvta_generic_to_shared(q); }
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, const int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, const uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, const uint32_t bytes, unsigned long long *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(__cvta_generic_to_global(src)), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-// false when the phase did not complete within ~1 s (a byte count that does not match the copies): the caller reports it
-__device__ __forceinline__ bool mbar_wait(unsigned long long *bar, const uint32_t parity)
-{
-    for (unsigned int spins = 0; spins < (1u << 22); spins++) {
-        uint32_t ok;
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(ok)
-                     : "r"(smem_u32(bar)), "r"(parity)
-                     : "memory");
-        if (ok) return true;
-    }
-    return false;
-}
-
-// header warp: start the bulk copies of the candidates of the work item in header buffer `buf` (published and
-// barrier-separated from here).  A cell with more candidates than the tile holds is not copied: it is flagged unseen.
-template <class SH>
-__device__ __forceinline__ void det_fetch(const P &p, SH &S, const int buf, const int lane)
-{
-    const int total = S.rcum[buf][8];
-    const bool fits = total <= DET_CAND;
-    if (lane == 0) {
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); /* the threads' reads of S.raw (behind a barrier) before the engine's writes */
-        mbar_expect_tx(&S.bar, fits ? (uint32_t)total * (uint32_t)sizeof(PosRec) : 0u);
-    }
-    __syncwarp();
-    if (fits && lane < 8) {
-        const int beg = S.rcum[buf][lane], len = S.rcum[buf][lane + 1] - beg;
-        if (len > 0) bulk_g2s(&S.raw[beg], p.a.pos + S.rbeg[buf][lane], (uint32_t)len * (uint32_t)sizeof(PosRec), &S.bar);
-    }
-}
-
-template <int TD_THREADS, int TD_K, int TD_OCC, int NBY_, int YF_>
-__global__ void __launch_bounds__(TD_THREADS, TD_OCC) k_detect_tma(const __grid_constant__ P p)
-{
-    static_assert(TD_THREADS * TD_K == DET_CAND, "the tile holds DET_CAND candidates");
-    typedef DetSharedT<NBY_, YF_> SH;
-    __shared__ SH S;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int nwork = *p.dl_count;
-    const int stride = gridDim.x;
-    int w = blockIdx.x;
-    if (w >= nwork) return;
-    for (int c = tid; c < SH::TAB; c += TD_THREADS) S.head[c] = 0;
-    if (tid < 2) { S.nmem[tid] = 0; S.nhit[tid] = 0; }
-    if (tid == 0) mbar_init(&S.bar, 1);
-    const bool hw = warp == TD_THREADS / 32 - 1; /* header warp: the tail of the candidate list, least to do */
-    int hn = 0;
-    if (hw) {
-        det_publish(p, S, 0, p.dl[(size_t)w * AMC_WI + lane], lane);
-        if (w + stride < nwork) hn = p.dl[(size_t)(w + stride) * AMC_WI + lane];
-    }
-    __syncthreads();
-    if (hw) det_fetch(p, S, 0, lane);
-    unsigned int tests = 0;
-    unsigned long long nref = 0; /* header warp, lane 0 */
-    const float thr = p.det_thr;
-    unsigned int tagw = 0;
-    uint32_t phase = 0;
-    bool stuck = false;
-    for (int it = 0; w < nwork; it++, w += stride) {
-        const int cur = it & 1, nxt = cur ^ 1;
-        tagw += 0x10000u;
-        if (tagw == 0) { /* visit tags exhausted: start over with a clean table */
-            __syncthreads();
-            for (int c = tid; c < SH::TAB; c += TD_THREADS) S.head[c] = 0;
-            tagw = 0x10000u;
-            __syncthreads();
-        }
-        const int total = S.rcum[cur][8];
-        const bool big = total > DET_CAND;
-        bool hit = big;
-        if (!mbar_wait(&S.bar, phase)) stuck = true; /* the records of this cell are in S.raw */
-        phase ^= 1u;
-        // ---- hash the members of the current cell
-        float fx[TD_K], fy[TD_K], fz[TD_K];
-        int bin[TD_K], older[TD_K];
-        {
-            const double *bd = reinterpret_cast<const double *>(&S.hdr[cur][20]);
-            const double lox = bd[0], hix = bd[1], loy = bd[2], hiy = bd[3], loz = bd[4], hiz = bd[5];
-            const float inv_wx = S.inv_wx[cur], inv_wy = S.inv_wy[cur];
-            const int nbx1 = S.nbx[cur] - 1, nby1 = S.nby[cur] - 1;
-            const int own = p.det_own_is_member ? S.rcum[cur][1] : 0; /* the owner cell's particles are members by construction */
-            int nm = 0;
-#pragma unroll
-            for (int k = 0; k < TD_K; k++) {
-                const int t = tid + k * TD_THREADS;
-                bin[k] = -1;
-                if (t < total && !big) {
-                    const double2 xy = *reinterpret_cast<const double2 *>(&S.raw[t]);
-                    const double x = xy.x, y = xy.y, z = S.raw[t].z;
-                    if (t < own || (lox < x && x < hix && loy < y && y < hiy && loz < z && z < hiz)) { /* Pore:527-530 */
-                        fx[k] = (float)(x - lox); fy[k] = (float)(y - loy); fz[k] = (float)(z - loz);
-                        int b = min(nbx1, (int)(fx[k] * inv_wx)) * SH::ROW + min(nby1, (int)(fy[k] * inv_wy)) + 1;
-                        unsigned int prev = atomicExch(&S.head[b], tagw | (unsigned int)(t + 1)) ^ tagw;
-                        prev = prev < 0x10000u ? prev : 0u;
-                        S.tile[t] = make_float4(fx[k], fy[k], fz[k], __uint_as_float(prev));
-                        bin[k] = b; older[k] = (int)prev;
-                        nm++;
-                    }
-                }
-            }
-            nm = __reduce_add_sync(0xffffffffu, nm);
-            if (lane == 0 && nm) atomicAdd(&S.nmem[cur], nm);
-        }
-        const int wn = w + stride;
-        if (hw && wn < nwork) {
-            det_publish(p, S, nxt, hn, lane);
-            if (wn + stride < nwork) hn = p.dl[(size_t)(wn + stride) * AMC_WI + lane];
-        }
-        __syncthreads();
-        // ---- every thread is done with S.raw: the next cell's records start their trip from HBM now
-        if (hw && wn < nwork) det_fetch(p, S, nxt, lane);
-        // ---- search: the older members of the own bin and everything in the four forward neighbour bins
-#pragma unroll
-        for (int k = 0; k < TD_K; k++) {
-            if (bin[k] < 0) continue;
-            const int b = bin[k];
-            unsigned int c[5];
-            c[0] = (unsigned int)older[k];
-            c[1] = S.head[b + 1] ^ tagw; c[2] = S.head[b + SH::ROW - 1] ^ tagw;
-            c[3] = S.head[b + SH::ROW] ^ tagw; c[4] = S.head[b + SH::ROW + 1] ^ tagw;
-            if (c[0] == 0 && min(min(c[1], c[2]), min(c[3], c[4])) >= 0x10000u) continue;
-            unsigned long long pend = c[0];
-            int sh = c[0] ? 9 : 0;
-#pragma unroll
-            for (int n = 1; n < 5; n++)
-                if (c[n] < 0x10000u) { pend |= (unsigned long long)c[n] << sh; sh += 9; }
-            const unsigned long long all = pend;
-            const float ax = fx[k], ay = fy[k], az = fz[k];
-            float dmin = 3.0e38f;
-            for (unsigned int e = 0;;) {
-                if (e == 0) {
-                    if (pend == 0) break;
-                    e = (unsigned int)pend & 511u;
-                    pend >>= 9;
-                }
-                float4 q = S.tile[e - 1];
-                float ex = q.x - ax, ey = q.y - ay, ez = q.z - az;
-                dmin = fminf(dmin, fmaf(ez, ez, fmaf(ey, ey, ex * ex)));
-                tests++;
-                e = __float_as_uint(q.w);
-            }
-            if (dmin < thr) { /* rare: walk the chains once more and remember the pairs for the ordered resolution */
-                hit = true;
-                pend = all;
-                for (unsigned int e = 0;;) {
-                    if (e == 0) {
-                        if (pend == 0) break;
-                        e = (unsigned int)pend & 511u;
-                        pend >>= 9;
-                    }
-                    float4 q = S.tile[e - 1];
-                    float ex = q.x - ax, ey = q.y - ay, ez = q.z - az;
-                    if (fmaf(ez, ez, fmaf(ey, ey, ex * ex)) < thr) {
-                        const int hh = atomicAdd(&S.nhit[cur], 1);
-                        if (hh < AMC_MAX_HITS) S.hit[cur][hh] = ((unsigned int)(tid + k * TD_THREADS) << 16) | (e - 1);
-                    }
-                    e = __float_as_uint(q.w);
-                }
-            }
-        }
-        if (tid == TD_THREADS - 1) { S.nmem[nxt] = 0; S.nhit[nxt] = 0; }
         const int any = __syncthreads_or(hit);
         if (hw) {
             const int *h = S.hdr[cur];
@@ -1922,7 +1697,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS) k_cube_sweep(const __grid_const
     const int tid = threadIdx.x;
     const Arrays &A = p.a;
     int32_t *lx = p.key, *lxy = p.rank;
-    if (p.sw_col && !p.sw_state[0]) return; /* the event-driven sweep (k_sweep_detect / k_sweep_events) did this pass */
+    if (!p.sw_state[0]) return; /* the event-driven sweep (k_sweep_detect / k_sweep_events) did this pass */
     if (tid == 0) { S.nexec = 0; S.nref = 0; }
     for (int c = tid; c < AMC_XBINS + 2; c += SWEEP_THREADS) S.head[c] = 0;
     for (int xl = 0; xl < p.nc[0]; xl++) {

@@ -108,3 +108,18 @@ def test_overlap_free_seeding(oracle):
     first = sim.step(1)[0]
     assert first["pp_collisions"] < 600                  # steady state ~260 per step; the un-relaxed start resolves ~1,070
     sim.close()
+
+
+def test_seed_relax_pinned():
+    """amc_seed_relax at 557,649 particles, seed 17: positions re-drawn and the state digest afterwards.  The values were
+    recorded on a B200 with the earlier seeding kernel, which loaded the candidates with the threads; the seeding variant
+    of the bulk-copy detection kernel has to mark the same particles in every round."""
+    from argon_monte_carlo_b200 import amc, config, init_state
+    cfg = config.pore_config(True)
+    n = cfg.num_molecules
+    assert n == 557649
+    sim = amc.Simulation(cfg, seed=17, max_particles=n)
+    sim.init_synthetic(init_state.pore_spec(cfg, 17))
+    assert sim.seed_relax(8) == (1115, 0)
+    assert sim.state_digest() == (6298284287226869198, 17013363693960920395, 557649)
+    sim.close()

@@ -95,15 +95,10 @@ def test_temp_host_rng_matches_oracle_and_shipped_csv(oracle, temp_cfg):
     sim.close()
 
 
-@pytest.mark.parametrize("detect", ["default", "ldg", "tma6"])
-def test_temp_device_rng_bit_exact(oracle, temp_cfg, temp_init, detect, monkeypatch):
-    """Energized pore with the device RNG, three timesteps against the oracle.  `detect` selects the shape of the
-    detection pass (read by amc_create): default = candidates staged by cp.async.bulk, 8 CTAs per SM; tma6 = the 6-CTA
-    shape with the full bin table; ldg = candidates loaded by the threads.  All three must give the oracle's state."""
+def test_temp_device_rng_bit_exact(oracle, temp_cfg, temp_init):
+    """Energized pore with the device RNG, three timesteps against the oracle."""
     from argon_monte_carlo_b200 import amc, config
     from oracle import steps
-    if detect != "default":
-        monkeypatch.setenv("AMC_DETECT", detect)
     cheb = config.gap_energy_chebyshev(temp_cfg, 16)
     st = oracle.ParticleState(*temp_init)
     sim = amc.Simulation(temp_cfg, taps=amc.TAP_WALL_BITS | amc.TAP_PAIRS, seed=17, cheb=cheb)
@@ -123,15 +118,13 @@ def test_temp_device_rng_bit_exact(oracle, temp_cfg, temp_init, detect, monkeypa
     sim.close()
 
 
-@pytest.mark.parametrize("sweep", ["events", "serial", "handover"])
+@pytest.mark.parametrize("sweep", ["events", "handover"])
 def test_cube_steps_bit_exact(oracle, cube_cfg, cube_init, sweep, monkeypatch):
     """Open_Air_Cube_MC.py as shipped, serial cell sweep (Cube:232-336).  events: the event-driven sweep
-    (k_sweep_detect / k_sweep_events, the default); serial: the plain one-CTA walk over all 3,375 cells
-    (AMC_CUBE_SWEEP=serial); handover: column lists too small for the gas, so every pass is handed to the plain walk."""
+    (k_sweep_detect / k_sweep_events); handover: column lists too small for the gas, so every pass is handed to the
+    plain one-CTA walk over all 3,375 cells (k_cube_sweep)."""
     from argon_monte_carlo_b200 import amc
     from oracle import steps
-    if sweep == "serial":
-        monkeypatch.setenv("AMC_CUBE_SWEEP", "serial")
     if sweep == "handover":
         monkeypatch.setenv("AMC_SWEEP_COLCAP", "16")
     st = oracle.ParticleState(*cube_init)
@@ -176,29 +169,3 @@ def test_multi_step_call_equals_single_steps(oracle, temp_cfg, temp_init):
     for k in KEYS:
         assert np.array_equal(ga[k], gb[k]) and np.array_equal(ga[k], getattr(st, k)), k
     a.close(); b.close()
-
-
-def test_dependent_launches_do_not_change_results(temp_cfg, temp_init, monkeypatch):
-    """The colour-group launches and the scan kernels are launched programmatically dependent on the kernel before
-    them (AMC_PDL, read by amc_create; DESIGN section 4).  Plain stream-ordered launches (AMC_PDL=0) must give the same
-    counters and the same state, bit for bit, over a multi-step call."""
-    from argon_monte_carlo_b200 import amc, config
-    cheb = config.gap_energy_chebyshev(temp_cfg, 16)
-    runs = []
-    for pdl in (None, "0"):
-        if pdl is None:
-            monkeypatch.delenv("AMC_PDL", raising=False)
-        else:
-            monkeypatch.setenv("AMC_PDL", pdl)
-        sim = amc.Simulation(temp_cfg, seed=11, cheb=cheb)
-        sim.set_state(*temp_init)
-        stats = sim.step(6)
-        runs.append((stats, sim.get_state(), sim.state_digest()))
-        sim.close()
-    (sa, ga, da), (sb, gb, db) = runs
-    for x, y in zip(sa, sb):
-        for k in ("collisions", "oob_after_walls", "oob_after_pp", "completed_paths", "dpz", "e_cold", "e_hot"):
-            assert x[k] == y[k], k
-    assert da == db
-    for k in KEYS:
-        assert np.array_equal(ga[k], gb[k]), k
