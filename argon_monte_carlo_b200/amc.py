@@ -92,12 +92,20 @@ EXPORTS = ("amc_create", "amc_destroy", "amc_last_error", "amc_abi_version", "am
            "amc_slab_group", "amc_slab_apply", "amc_slab_finish", "amc_slab_get_owned", "amc_state_digest",
            "amc_slab_p2p_setup", "amc_slab_p2p_connect", "amc_slab_step", "amc_wall_operator", "amc_seed_relax", "amc_last_scatter_ms",
            "amc_sample_enable", "amc_sample_disable", "amc_sample_now", "amc_sample_get_raw", "amc_sample_set_raw",
-           "amc_last_sample_ms")
+           "amc_last_sample_ms", "amc_surface_enable", "amc_surface_disable", "amc_surface_layout", "amc_surface_get_raw",
+           "amc_surface_set_raw")
 
 # field sampling (include/amc.h): words per cell and the binary scales of the fixed-point limbs
 SAMPLE_WORDS = 13
 SAMPLE_V1, SAMPLE_V2 = 19, 49     # velocity sums: high / low limb
 SAMPLE_Q1, SAMPLE_Q2 = 6, 36      # sums of squares: high / low limb
+
+# surface recording (include/amc.h): words per wall element and the binary scales of the fixed-point limbs
+SURF_WORDS = 9
+SURF_V1, SURF_V2 = 16, 46         # velocity-change sums: high / low limb
+SURF_E1, SURF_E2 = 90, 120        # energy sums: high / low limb
+SIDE_CASES = (0, 5, 8, 9)         # cylinder slots of Pore (0, 5, 8) and Temp (1, 4, 6H, 6C)
+PLUS_Z_CASES = (1, 3, 6)          # planes whose normal into the gas is +z (2A / 3C / 5B, Pore 1 / 3 / 6); others: -z
 
 
 def load_library():
@@ -239,6 +247,133 @@ def merge_sample_ranks(parts):
     return acc, ns.pop(), sum(int(p[2]) for p in parts) & ((1 << 64) - 1)
 
 
+class SurfaceLayout:
+    """The wall elements of a handle (amc_surface_layout): per case its bin type -- "side" (z layers of `zedge`),
+    "annulus" (bounds `rsq`), "face" (cube face: in-plane owner cells) or None (no elements) -- and the case-major
+    offsets[NUM_CASES + 1]."""
+
+    def __init__(self, kind, grid, R_oa=None):
+        self.kind = kind
+        self.edges = [np.asarray(e, dtype=np.float64) for e in grid.edge]
+        self.nc = tuple(len(e) - 1 for e in self.edges)
+        self.zedge = self.edges[2]
+        x = self.edges[0]
+        self.dr = float((x[-1] - x[0]) / float(len(x) - 1))
+        self.nann = 0 if kind == KIND_CUBE else int(math.ceil(float(R_oa) / self.dr))
+        k = np.arange(self.nann + 1, dtype=np.float64)
+        self.rsq = (k * self.dr) * (k * self.dr)
+        self.types, counts = [], []
+        for c in range(NUM_CASES):
+            if kind == KIND_CUBE:
+                t = "face" if c < 6 else None
+                n = self.nc[self.face_axes(c)[1]] * self.nc[self.face_axes(c)[2]] if t else 0
+            elif kind == KIND_PORE and c == 9:
+                t, n = None, 0
+            elif c in SIDE_CASES:
+                t, n = "side", self.nc[2]
+            else:
+                t, n = "annulus", self.nann
+            self.types.append(t)
+            counts.append(n)
+        self.offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+
+    @staticmethod
+    def face_axes(c):
+        """(normal axis a, in-plane axes b1 < b2) of cube case c."""
+        a = c >> 1
+        return a, (1 if a == 0 else 0), (1 if a == 2 else 2)
+
+    @property
+    def n_elements(self):
+        return int(self.offsets[-1])
+
+
+def surface_layout_of(cfg, kind, grid):
+    """NumPy restatement of amc_surface_layout for a handle of `kind` on `grid` (a slab run: the global grid)."""
+    return SurfaceLayout(kind, grid, None if kind == KIND_CUBE else cfg.geom.R_oa)
+
+
+def _bin_of(tab, v):
+    """k with tab[k] <= v < tab[k+1], or -1 (NaN and anything outside the table)."""
+    tab = np.asarray(tab, dtype=np.float64)
+    k = np.searchsorted(tab, v, side="right") - 1
+    with np.errstate(invalid="ignore"):
+        ok = (v >= tab[0]) & (v < tab[-1])
+    return np.where(ok, k, -1)
+
+
+def surface_moments_of_hits(hits, layout, geom=None):
+    """NumPy restatement of the surface accumulators: hits = dict of arrays "case", "col" [n, 3] (contact point),
+    "v_in", "v_out" [n, 3], "dE" (the energy the gas gained), one entry per hit the wall phases applied, plus hits
+    that apply nothing (col NaN: the reference's floating-point error path).  geom: the config's geometry (cylinder
+    radii; not needed for the cube).  Returns (acc [elements][SURF_WORDS] uint64, outside [NUM_CASES] uint64) with
+    the binning and the IEEE expressions of include/amc.h."""
+    case = np.asarray(hits["case"], dtype=np.int64)
+    col = np.asarray(hits["col"], dtype=np.float64).reshape(-1, 3)
+    dv = np.asarray(hits["v_out"], dtype=np.float64).reshape(-1, 3) - np.asarray(hits["v_in"], dtype=np.float64).reshape(-1, 3)
+    dE = np.asarray(hits["dE"], dtype=np.float64)
+    n = len(case)
+    elem = np.full(n, -1, dtype=np.int64)
+    w = np.zeros((n, 3), dtype=np.float64)
+    cx, cy, cz = col[:, 0], col[:, 1], col[:, 2]
+    dvx, dvy, dvz = dv[:, 0], dv[:, 1], dv[:, 2]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        for c in range(NUM_CASES):
+            m = case == c
+            t = layout.types[c]
+            if not m.any() or t is None:
+                continue
+            if t == "face":
+                a, b1, b2 = layout.face_axes(c)
+                w[m, 0] = dv[m, a] if c & 1 else -dv[m, a]
+                w[m, 1], w[m, 2] = dv[m, b1], dv[m, b2]
+                o1, o2 = _bin_of(layout.edges[b1], col[m, b1]), _bin_of(layout.edges[b2], col[m, b2])
+                e = np.where((o1 >= 0) & (o2 >= 0), o1 * layout.nc[b2] + o2, -1)
+            elif t == "side":
+                Rc = float(geom.R_oa_c if c == 0 else (geom.R_g_c if c == 5 else geom.R_p_c))
+                ex, ey = cx[m] / Rc, cy[m] / Rc
+                w[m, 0] = -(dvx[m] * ex + dvy[m] * ey)
+                w[m, 1] = dvz[m]
+                w[m, 2] = dvy[m] * ex - dvx[m] * ey
+                e = _bin_of(layout.zedge, cz[m])
+            else:
+                r2 = cx[m] * cx[m] + cy[m] * cy[m]
+                r = np.sqrt(r2)
+                ex = np.where(r > 0.0, cx[m] / r, 1.0)
+                ey = np.where(r > 0.0, cy[m] / r, 0.0)
+                w[m, 0] = dvz[m] if c in PLUS_Z_CASES else -dvz[m]
+                w[m, 1] = dvx[m] * ex + dvy[m] * ey
+                w[m, 2] = dvy[m] * ex - dvx[m] * ey
+                e = _bin_of(layout.rsq, r2)
+            elem[m] = np.where(e >= 0, layout.offsets[c] + e, -1)
+    inside = elem >= 0
+    outside = np.bincount(case[~inside], minlength=NUM_CASES).astype(np.uint64)
+    acc = np.zeros((layout.n_elements, SURF_WORDS), dtype=np.uint64)
+    el = elem[inside]
+    acc[:, 0] = np.bincount(el, minlength=layout.n_elements).astype(np.uint64)
+    cols = [sample_limbs(w[inside, j], SURF_V1, SURF_V2) for j in range(3)] + [sample_limbs(dE[inside], SURF_E1, SURF_E2)]
+    with np.errstate(over="ignore"):
+        for j, (i1, i2) in enumerate(cols):
+            np.add.at(acc[:, 1 + 2 * j], el, i1.view(np.uint64))
+            np.add.at(acc[:, 2 + 2 * j], el, i2.view(np.uint64))
+    return acc, outside
+
+
+def merge_surface_ranks(parts):
+    """Raw surface arrays of the ranks of one run (each (acc, n_steps, outside)): element-wise sums mod 2^64; every
+    rank recorded the same wall phases."""
+    parts = list(parts)
+    ns = {int(p[1]) for p in parts}
+    if len(ns) != 1:
+        raise AmcError("ranks disagree on the number of wall phases recorded: %s" % sorted(ns))
+    acc, out = parts[0][0].copy(), parts[0][2].copy()
+    with np.errstate(over="ignore"):
+        for p in parts[1:]:
+            acc += p[0]
+            out += p[2]
+    return acc, ns.pop(), out
+
+
 def combine_digests(parts):
     """Sum of per-rank digests (mod 2^64 per component)."""
     m = (1 << 64) - 1
@@ -305,6 +440,7 @@ class Simulation:
         self.sample_grid = grid     # a slab rank's handle samples the global grid (slab.SlabRank sets it)
         self.sampling = None    # (every, first_step) while field sampling is enabled
         self.host_steps = 0     # timesteps taken by step_host_rng (the index the sampling schedule of that path uses)
+        self.surface_on = False  # surface recording enabled (amc_surface_enable)
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -523,6 +659,41 @@ class Simulation:
         self._check(self.lib.amc_last_sample_ms(self.h, C.byref(v)), "amc_last_sample_ms")
         return float(v.value)
 
+    # ------------------------------------------------------------------ surface recording
+    def surface_enable(self):
+        """Record every wall interaction into per-element accumulators (amc_surface_enable); zeroes them."""
+        self._check(self.lib.amc_surface_enable(self.h), "amc_surface_enable")
+        self.surface_on = True
+
+    def surface_disable(self):
+        self._check(self.lib.amc_surface_disable(self.h), "amc_surface_disable")
+        self.surface_on = False
+
+    def surface_layout(self):
+        """offsets[NUM_CASES + 1] int64: the elements of case c are offsets[c] .. offsets[c+1]."""
+        off = np.zeros(NUM_CASES + 1, dtype=np.int64)
+        self._check(self.lib.amc_surface_layout(self.h, off.ctypes.data_as(c_int64_p)), "amc_surface_layout")
+        return off
+
+    def surface_raw(self):
+        """(acc [elements][SURF_WORDS] uint64, wall phases recorded, outside [NUM_CASES] uint64)."""
+        acc = np.zeros((int(self.surface_layout()[-1]), SURF_WORDS), dtype=np.uint64)
+        out = np.zeros(NUM_CASES, dtype=np.uint64)
+        ns = C.c_uint64(0)
+        u64 = C.POINTER(C.c_uint64)
+        self._check(self.lib.amc_surface_get_raw(self.h, acc.ctypes.data_as(u64), C.byref(ns), out.ctypes.data_as(u64)),
+                    "amc_surface_get_raw")
+        return acc, int(ns.value), out
+
+    def surface_set_raw(self, acc, n_steps, outside):
+        acc = np.ascontiguousarray(acc, dtype=np.uint64)
+        outside = np.ascontiguousarray(outside, dtype=np.uint64)
+        if acc.size != int(self.surface_layout()[-1]) * SURF_WORDS or outside.size != NUM_CASES:
+            raise AmcError("surface accumulators of %d words for a layout of %d elements" % (acc.size, int(self.surface_layout()[-1])))
+        u64 = C.POINTER(C.c_uint64)
+        self._check(self.lib.amc_surface_set_raw(self.h, acc.ctypes.data_as(u64), C.c_uint64(int(n_steps)), outside.ctypes.data_as(u64)),
+                    "amc_surface_set_raw")
+
     # ------------------------------------------------------------------ outputs
     def histograms(self):
         """(counts[4, 200] uint64 in the order total/x/y/z, number of completed paths, sums[4])."""
@@ -580,6 +751,9 @@ class Simulation:
             acc, ns, no = self.sample_raw()
             st.update(sample_acc=acc, sample_n=np.uint64(ns), sample_outside=np.uint64(no),
                       sample_schedule=np.array(self.sampling, dtype=np.int64), host_steps=np.int64(self.host_steps))
+        if self.surface_on:
+            acc, ns, out = self.surface_raw()
+            st.update(surface_acc=acc, surface_n_steps=np.uint64(ns), surface_outside=out)
         if path is not None:
             np.savez(path, **st)
         return st
@@ -608,6 +782,9 @@ class Simulation:
             self.sample_enable(every, first)
             self.sample_set_raw(ck["sample_acc"], int(ck["sample_n"]), int(ck["sample_outside"]))
             self.host_steps = int(ck["host_steps"])
+        if "surface_acc" in ck:         # checkpoints written without surface recording have none of these keys
+            self.surface_enable()
+            self.surface_set_raw(ck["surface_acc"], int(ck["surface_n_steps"]), ck["surface_outside"])
 
     def state_digest(self):
         """(sum0, sum1, count): order-independent checksum of the owned particle state, computed on the device

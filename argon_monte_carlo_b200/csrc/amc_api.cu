@@ -75,6 +75,12 @@ struct amc_handle {
     std::vector<cudaEvent_t> sample_events; // two per sample of the last call: around k_sample
     int sample_slot = 0;                    // samples recorded into sample_events by the current call
     double last_sample_ms = 0;
+    // surface recording (amc_surface_*): accumulators [elements][AMC_SURF_WORDS] + outside[AMC_NUM_CASES]; null: off
+    unsigned long long *d_surf = nullptr;
+    double *d_surf_rsq = nullptr; // annulus bounds, SurfP::rsq
+    SurfP sp = {};                // kernel parameter of the recording kernels (sp.acc = d_surf)
+    uint64_t surf_steps = 0;      // wall phases recorded
+    double surf_dr = 0;           // x cell width of the grid: (edge[0][nc] - edge[0][0]) / nc
     std::string error;
 
     int fail(int code, const std::string &msg)
@@ -183,6 +189,8 @@ extern "C" int amc_destroy(amc_handle *h)
     for (cudaEvent_t e : h->sc_events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->sample_events) cudaEventDestroy(e);
     if (h->d_sample) cudaFree(h->d_sample);
+    if (h->d_surf) cudaFree(h->d_surf);
+    if (h->d_surf_rsq) cudaFree(h->d_surf_rsq);
     if (h->h_stats) cudaFreeHost(h->h_stats);
     if (h->aux) { cudaStreamSynchronize(h->aux); cudaStreamDestroy(h->aux); }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -253,6 +261,7 @@ static int create_impl(amc_handle *h, const amc_config *cfg, int device)
         p.e0[a] = cfg->edge[a][0];
         p.inv_d[a] = (double)cfg->nc[a] / (cfg->edge[a][cfg->nc[a]] - cfg->edge[a][0]);
     }
+    h->surf_dr = (cfg->edge[0][cfg->nc[0]] - cfg->edge[0][0]) / (double)cfg->nc[0];
     if (ncell + 2 > 0x7fffffffLL) return h->fail(AMC_E_INVALID, "too many cells");
     p.ncell_pad = (int32_t)ncell;
     for (int a = 0; a < 3; a++) p.nh[a] = (cfg->nc[a] + 1) / 2;
@@ -704,6 +713,114 @@ extern "C" int amc_last_sample_ms(amc_handle *h, double *ms)
     return AMC_OK;
 }
 
+// ---- surface recording ---------------------------------------------------------------------------
+// elements of every wall case (include/amc.h): z layers for the cylinders, annuli for the planes of Pore / Temp, the
+// in-plane cell pairs for the cube faces; rsq (nullable) receives the annulus bounds
+static void surf_layout(const amc_handle *h, int64_t off[AMC_NUM_CASES + 1], std::vector<double> *rsq)
+{
+    const int64_t nc[3] = {h->cfg.nc[0], h->cfg.nc[1], h->slab ? h->p.gncz : h->cfg.nc[2]};
+    const int32_t kind = h->cfg.kind;
+    const int64_t nann = kind == AMC_KIND_CUBE ? 0 : (int64_t)ceil(h->cfg.geom.R_oa / h->surf_dr);
+    off[0] = 0;
+    for (int c = 0; c < AMC_NUM_CASES; c++) {
+        int64_t n = 0;
+        if (kind == AMC_KIND_CUBE) {
+            const int a = c >> 1;
+            if (c < 6) n = nc[a == 0 ? 1 : 0] * nc[a == 2 ? 1 : 2];
+        } else if (kind == AMC_KIND_PORE && c == AMC_CASE_6C) {
+            n = 0;
+        } else {
+            const bool side = c == AMC_CASE_1 || c == AMC_CASE_4 || c == AMC_CASE_6H || c == AMC_CASE_6C;
+            n = side ? nc[2] : nann;
+        }
+        off[c + 1] = off[c] + n;
+    }
+    if (rsq) {
+        rsq->resize((size_t)nann + 1);
+        for (int64_t k = 0; k <= nann; k++) (*rsq)[k] = ((double)k * h->surf_dr) * ((double)k * h->surf_dr);
+    }
+}
+
+extern "C" int amc_surface_layout(amc_handle *h, int64_t offsets[AMC_NUM_CASES + 1])
+{
+    if (!h || !offsets) return AMC_E_INVALID;
+    surf_layout(h, offsets, nullptr);
+    return AMC_OK;
+}
+
+extern "C" int amc_surface_disable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    if (h->d_surf) CK(cudaFree(h->d_surf));
+    if (h->d_surf_rsq) CK(cudaFree(h->d_surf_rsq));
+    h->d_surf = nullptr; h->d_surf_rsq = nullptr;
+    h->sp = SurfP{};
+    h->surf_steps = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_surface_enable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    int rc = amc_surface_disable(h);
+    if (rc != AMC_OK) return rc;
+    P &p = h->p;
+    int64_t off[AMC_NUM_CASES + 1];
+    std::vector<double> rsq;
+    surf_layout(h, off, &rsq);
+    if (off[AMC_NUM_CASES] > 0x7fffffffLL / AMC_SURF_WORDS) return h->fail(AMC_E_INVALID, "too many surface elements");
+    const size_t words = (size_t)off[AMC_NUM_CASES] * AMC_SURF_WORDS + AMC_NUM_CASES;
+    cudaError_t e = cudaMalloc(&h->d_surf, words * sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMalloc(&h->d_surf_rsq, rsq.size() * sizeof(double));
+    if (e != cudaSuccess) {
+        amc_surface_disable(h);
+        return h->fail(AMC_E_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    }
+    CK(cudaMemsetAsync(h->d_surf, 0, words * sizeof(unsigned long long), h->stream));
+    CK(cudaMemcpyAsync(h->d_surf_rsq, rsq.data(), rsq.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    SurfP &sp = h->sp;
+    for (int c = 0; c <= AMC_NUM_CASES; c++) sp.off[c] = (int32_t)off[c];
+    sp.rsq = h->d_surf_rsq;
+    sp.nann = (int32_t)(rsq.size() - 1);
+    sp.inv_dr = 1.0 / h->surf_dr;
+    if (p.slab) { sp.zedge = p.gz_edge; sp.ncz = p.gncz; sp.ze0 = p.g_e0z; sp.zinv = p.g_inv_dz; }
+    else { sp.zedge = p.edge[2]; sp.ncz = p.nc[2]; sp.ze0 = p.e0[2]; sp.zinv = p.inv_d[2]; }
+    sp.acc = h->d_surf;
+    h->surf_steps = 0;
+    return AMC_OK;
+}
+
+static size_t surf_acc_words(const amc_handle *h) { return (size_t)h->sp.off[AMC_NUM_CASES] * AMC_SURF_WORDS; }
+
+extern "C" int amc_surface_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_steps, uint64_t outside[AMC_NUM_CASES])
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_surf) return h->fail(AMC_E_STATE, "surface recording is not enabled (amc_surface_enable)");
+    CK(cudaSetDevice(h->device));
+    const size_t nw = surf_acc_words(h);
+    if (acc) CK(cudaMemcpyAsync(acc, h->d_surf, nw * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+    if (outside) CK(cudaMemcpyAsync(outside, h->d_surf + nw, AMC_NUM_CASES * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (n_steps) *n_steps = h->surf_steps;
+    return AMC_OK;
+}
+
+extern "C" int amc_surface_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_steps, const uint64_t outside[AMC_NUM_CASES])
+{
+    if (!h || !acc || !outside) return AMC_E_INVALID;
+    if (!h->d_surf) return h->fail(AMC_E_STATE, "surface recording is not enabled (amc_surface_enable)");
+    CK(cudaSetDevice(h->device));
+    const size_t nw = surf_acc_words(h);
+    CK(cudaMemcpyAsync(h->d_surf, acc, nw * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_surf + nw, outside, AMC_NUM_CASES * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->surf_steps = n_steps;
+    return AMC_OK;
+}
+
 extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
 {
     if (!h) return AMC_E_INVALID;
@@ -737,6 +854,7 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
         for (int s = 0; s < chunk; s++) {
             p.stats = h->d_stats + s;
             p.step = h->step_index++;
+            if (h->sp.acc) h->surf_steps++;
             // a sampled step is closed like the last step of a chunk, so the sample sees the state at its end
             const bool sample = sample_due(h, p.step);
             if (h->n > 0) {
@@ -745,7 +863,8 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
                 p.stats_prev = fuse_prev ? h->d_stats + (s - 1) : h->d_stats + s;
                 int phase = PH_DRIFT | PH_WALLS | (has_recap ? PH_RECAP : 0) | (fuse_prev ? PH_RECAP_POST : 0);
                 if (sweep) {
-                    k_advect<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase);
+                    if (h->sp.acc) k_advect_surf<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase, h->sp);
+                    else k_advect<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase);
                     h->last_launches += 1;
                     CK(cudaEventRecord(h->events[4 * s + 1], h->stream));
                 } else { // fused: keys of the post-step positions, then the step itself on the way to the sorted slot
@@ -763,7 +882,8 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
                     if ((rc = prepare_pairs(h, h->aux)) != AMC_OK) return rc;
                     CK(cudaEventRecord(h->ev_join, h->aux));
                     CK(cudaEventRecord(h->sc_events[2 * s], h->stream));
-                    k_scatter_advect<false><<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase);
+                    if (h->sp.acc) k_scatter_advect_surf<false><<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase, h->sp);
+                    else k_scatter_advect<false><<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, phase);
                     CK(cudaEventRecord(h->sc_events[2 * s + 1], h->stream));
                     CK(cudaGetLastError());
                     CK(cudaStreamWaitEvent(h->stream, h->ev_join, 0));
@@ -855,7 +975,11 @@ extern "C" int amc_walls(amc_handle *h, amc_step_stats *stats)
     if (rc != AMC_OK) return rc;
     if ((rc = ensure_prior(h)) != AMC_OK) return rc;
     h->p.step = h->step_index++;
-    if (h->n) k_advect<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, PH_WALLS | PH_LOAD_PRIOR);
+    if (h->sp.acc) h->surf_steps++;
+    if (h->n) {
+        if (h->sp.acc) k_advect_surf<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, PH_WALLS | PH_LOAD_PRIOR, h->sp);
+        else k_advect<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, PH_WALLS | PH_LOAD_PRIOR);
+    }
     return phase_end(h, stats);
 }
 
@@ -960,7 +1084,8 @@ extern "C" int amc_wall_case(amc_handle *h, int32_t c, int64_t *n_hits)
     if (!h->have_prior) return h->fail(AMC_E_STATE, "call amc_drift first");
     int rc = phase_begin(h);
     if (rc != AMC_OK) return rc;
-    if (h->n) k_case_specular<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, c);
+    if (h->sp.acc && c == AMC_CASE_1) h->surf_steps++; /* the first case of a host-RNG wall phase */
+    if (h->n) k_case_specular<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, c, h->sp);
     amc_step_stats st;
     rc = phase_end(h, &st);
     if (n_hits) *n_hits = st.wall_hits[c];
@@ -1028,7 +1153,7 @@ extern "C" int amc_wall_apply_directions(amc_handle *h, int32_t c, int64_t n_hit
         CK(cudaMemcpyAsync(h->d_pend_dirs, dir3, (size_t)n_hits * 3 * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         if (surf_e) CK(cudaMemcpyAsync(h->d_pend_se, surf_e, n_hits * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         k_case_apply<<<grid_for(n_hits, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, c, (int32_t)n_hits, h->d_pend_slot, h->d_pend_dirs,
-                                                                                        h->d_pend_se, h->d_pend_dpz, h->d_pend_de);
+                                                                                        h->d_pend_se, h->d_pend_dpz, h->d_pend_de, h->sp);
         if (dpz) CK(cudaMemcpyAsync(dpz, h->d_pend_dpz, n_hits * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         if (de) CK(cudaMemcpyAsync(de, h->d_pend_de, n_hits * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     }
@@ -1206,6 +1331,7 @@ extern "C" int amc_slab_enable(amc_handle *h, const amc_slab_config *c)
     if (c->cuts[c->rank + 1] - c->cuts[c->rank] != h->cfg.nc[2]) return h->fail(AMC_E_INVALID, "handle z grid does not match its slab");
     if (h->p.wall_bits) return h->fail(AMC_E_INVALID, "AMC_TAP_WALL_BITS is indexed by particle id (global on a slab handle): not available with slabs");
     if (h->d_sample) return h->fail(AMC_E_STATE, "enable sampling after amc_slab_enable (a slab handle samples the global grid)");
+    if (h->d_surf) return h->fail(AMC_E_STATE, "enable surface recording after amc_slab_enable (a slab handle bins on the global grid)");
     CK(cudaSetDevice(h->device));
     P &p = h->p;
     p.slab = 1; p.srank = c->rank; p.nranks = c->nranks; p.zoff = c->cuts[c->rank]; p.gncz = c->gncz;
@@ -1296,6 +1422,7 @@ extern "C" int amc_slab_advect(amc_handle *h)
     CK(cudaMemsetAsync(p.band_count, 0, (h->n_buckets + 2) * sizeof(int32_t), h->stream));
     CK(cudaMemsetAsync(p.rest_count, 0, (h->n_buckets + 1) * sizeof(int32_t), h->stream));
     h->slab_phase = PH_DRIFT | PH_WALLS | (p.kind != AMC_KIND_CUBE ? PH_RECAP : 0);
+    if (h->sp.acc) h->surf_steps++;
     if (h->n) {
         k_keys<true><<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, h->slab_phase);
         if (p.nranks > 1) k_slab_pack<<<dim3(grid_for(p.xf_cap, ADVECT_THREADS), p.nranks), ADVECT_THREADS, 0, h->stream>>>(p, h->slab_phase);
@@ -1320,7 +1447,8 @@ extern "C" int amc_slab_sort(amc_handle *h, int64_t *n_resident)
     k_scan_tiles<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.band_count, p.rest_count, p.cell_start, h->d_tile_sums, m);
     k_scan_sums<<<1, SCAN_THREADS, 0, h->stream>>>(h->d_tile_sums, ntiles);
     k_scan_add<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.cell_start, h->d_tile_sums, m, 0);
-    if (bound) k_scatter_advect<true><<<grid_for(bound, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, h->slab_phase);
+    if (bound && h->sp.acc) k_scatter_advect_surf<true><<<grid_for(bound, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, h->slab_phase, h->sp);
+    else if (bound) k_scatter_advect<true><<<grid_for(bound, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p, h->slab_phase);
     h->last_launches += 4 + (bound ? 1 : 0);
     CK(cudaGetLastError());
     std::swap(p.a, p.b);
@@ -1559,6 +1687,7 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
         for (int s = 0; s < chunk; s++) {
             p.stats = h->d_stats + s;
             p.step = h->step_index++;
+            if (h->sp.acc) h->surf_steps++;
             p.xf_seq = ++h->xf_seq;
             p.parity = (int32_t)(p.xf_seq & 1u);
             // ---- advect (dry run) + packing, all-to-all, unpack, sort
@@ -1577,7 +1706,8 @@ extern "C" int amc_slab_step(amc_handle *h, int32_t n_steps, int32_t pre_round, 
             k_scan_tiles<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.band_count, p.rest_count, p.cell_start, h->d_tile_sums, m);
             k_scan_sums<<<1, SCAN_THREADS, 0, h->stream>>>(h->d_tile_sums, ntiles);
             k_scan_add<<<ntiles, SCAN_THREADS, 0, h->stream>>>(p.cell_start, h->d_tile_sums, m, 0);
-            k_scatter_advect<true><<<full, ADVECT_THREADS, 0, h->stream>>>(p, phase);
+            if (h->sp.acc) k_scatter_advect_surf<true><<<full, ADVECT_THREADS, 0, h->stream>>>(p, phase, h->sp);
+            else k_scatter_advect<true><<<full, ADVECT_THREADS, 0, h->stream>>>(p, phase);
             std::swap(p.a, p.b);
             k_slab_set_n<<<1, 32, 0, h->stream>>>(p, 1);
             CK(cudaEventRecord(h->events[4 * s + 2], h->stream));

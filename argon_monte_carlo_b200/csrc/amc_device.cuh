@@ -218,6 +218,19 @@ struct P {
     unsigned long long *sw_state; /* [0] != 0: a column list overflowed, the plain sweep takes over; [1] pair tests of pass 1 */
 };
 
+// surface recording (amc_surface_*): a kernel parameter of its own, passed only to the recording kernels
+// (k_advect_surf, k_scatter_advect_surf, the host-RNG case kernels), so that P and every other kernel stay as they are
+struct SurfP {
+    unsigned long long *acc; /* [elements][AMC_SURF_WORDS], then outside[AMC_NUM_CASES]; null: not recording */
+    int32_t off[AMC_NUM_CASES + 1]; /* first element of every case (case-major numbering) */
+    const double *rsq;       /* annulus bounds (k * dr) * (k * dr), k = 0 .. nann */
+    int32_t nann;
+    double inv_dr;
+    const double *zedge;     /* z edges of the layout (a slab handle: the global ones) */
+    int32_t ncz;
+    double ze0, zinv;
+};
+
 // ---------------------------------------------------------------- deterministic accumulation
 // Sums that feed printed outputs (momentum / energy per step, free-path means) are accumulated as
 // two 64-bit integer limbs at fixed binary scales: integer adds are associative, so the result does
@@ -240,6 +253,11 @@ __device__ __forceinline__ void acc_add(unsigned long long *acc, double v, doubl
     atomicAdd(&acc[0], (unsigned long long)i1);
     atomicAdd(&acc[1], (unsigned long long)i2);
 }
+
+// surface recording (defined below, after the owner-cell helpers it uses)
+__device__ __noinline__ void surf_record(const P &p, const SurfP &sp, const int c, const double cx, const double cy, const double cz,
+                                         const double dvx, const double dvy, const double dvz, const double dE);
+__device__ __noinline__ void surf_outside(const SurfP &sp, const int c);
 
 // ---------------------------------------------------------------- completed free paths
 // One completed path = one append to each of the reference's four lists (Pore:187-190).  The
@@ -319,24 +337,31 @@ __device__ __forceinline__ void reflect_xy(Part &q, double Rc, double t)
     q.x = col_x + nvx * t; q.y = col_y + nvy * t; q.vx = nvx; q.vy = nvy;
 }
 
-// hit_cylinder_side_wall, Pore:294-348
-template <int MODE = 1>
-__device__ __forceinline__ void pore_side_wall(const P &p, Part &q, double Rc)
+// hit_cylinder_side_wall, Pore:294-348.  SURF: record the hit as wall case c (surf_record)
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ void pore_side_wall(const P &p, Part &q, double Rc, int c = 0, const SurfP *sp = nullptr)
 {
     double t;
-    if (!side_quadratic(q.x, q.y, q.vx, q.vy, Rc, t)) { if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull); return; }
+    if (!side_quadratic(q.x, q.y, q.vx, q.vy, Rc, t)) {
+        if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull);
+        if (SURF && MODE == AMC_LIVE) surf_outside(*sp, c);
+        return;
+    }
     double vx = q.vx, vy = q.vy, vz = q.vz;
     mfp_record<MODE>(p, q.d, q.dx, q.dy, q.dz, q.flag, vx, vy, vz, t);
+    const double cx = q.x - vx * t, cy = q.y - vy * t, cz = q.z - vz * t; /* contact point (the col_x, col_y of reflect_xy) */
     reflect_xy(q, Rc, t);
+    if (SURF && MODE == AMC_LIVE) surf_record(p, *sp, c, cx, cy, cz, q.vx - vx, q.vy - vy, 0.0, 0.0);
     q.d = fabs(sqrt((q.vx * q.vx + q.vy * q.vy) + vz * vz) * t);
     q.dx = fabs(q.vx * t); q.dy = fabs(q.vy * t); q.dz = fabs(vz * t);
 }
 
 // hit_vertical_wall, Pore:257-292
-template <int MODE = 1>
-__device__ __forceinline__ void pore_plane_wall(const P &p, Part &q, double zp)
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ void pore_plane_wall(const P &p, Part &q, double zp, int c = 0, const SurfP *sp = nullptr)
 {
     double t = (q.z - zp) / q.vz;
+    if (SURF && MODE == AMC_LIVE) surf_record(p, *sp, c, q.x - q.vx * t, q.y - q.vy * t, zp, 0.0, 0.0, -q.vz - q.vz, 0.0);
     mfp_record<MODE>(p, q.d, q.dx, q.dy, q.dz, q.flag, q.vx, q.vy, q.vz, t);
     q.d = fabs(sqrt((q.vx * q.vx + q.vy * q.vy) + q.vz * q.vz) * t);
     q.dx = fabs(q.vx * t); q.dy = fabs(q.vy * t); q.dz = fabs(q.vz * t);
@@ -346,23 +371,23 @@ __device__ __forceinline__ void pore_plane_wall(const P &p, Part &q, double zp)
 
 // Pore wall cases 1..6 against the progressively mutated particle (Pore:442-485); returns hit bits.
 // `np.sqrt(x**2 + y**2) > R` is evaluated as `x*x + y*y > gt_R` (exactly equivalent, see P).
-template <int MODE = 1>
-__device__ __forceinline__ uint32_t pore_walls(const P &p, Part &q)
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ uint32_t pore_walls(const P &p, Part &q, const SurfP *sp = nullptr)
 {
     const amc_geom &g = p.g;
     uint32_t bits = 0;
-    if (q.x * q.x + q.y * q.y > p.gt_Roa) { bits |= 1u << 0; pore_side_wall<MODE>(p, q, g.R_oa_c); }
-    if (q.z < 0) { bits |= 1u << 1; pore_plane_wall<MODE>(p, q, 0.0); }
-    if (q.z > g.H) { bits |= 1u << 2; pore_plane_wall<MODE>(p, q, g.H); }
-    if (q.pz > g.z_cold && q.z < g.z_cold && q.x * q.x + q.y * q.y > p.gt_Rp) { bits |= 1u << 3; pore_plane_wall<MODE>(p, q, g.z_cold); }
-    if (q.pz < g.oah && q.z > g.oah && q.x * q.x + q.y * q.y > p.gt_Rp) { bits |= 1u << 4; pore_plane_wall<MODE>(p, q, g.oah); }
+    if (q.x * q.x + q.y * q.y > p.gt_Roa) { bits |= 1u << 0; pore_side_wall<MODE, SURF>(p, q, g.R_oa_c, 0, sp); }
+    if (q.z < 0) { bits |= 1u << 1; pore_plane_wall<MODE, SURF>(p, q, 0.0, 1, sp); }
+    if (q.z > g.H) { bits |= 1u << 2; pore_plane_wall<MODE, SURF>(p, q, g.H, 2, sp); }
+    if (q.pz > g.z_cold && q.z < g.z_cold && q.x * q.x + q.y * q.y > p.gt_Rp) { bits |= 1u << 3; pore_plane_wall<MODE, SURF>(p, q, g.z_cold, 3, sp); }
+    if (q.pz < g.oah && q.z > g.oah && q.x * q.x + q.y * q.y > p.gt_Rp) { bits |= 1u << 4; pore_plane_wall<MODE, SURF>(p, q, g.oah, 4, sp); }
     double pr2 = q.px * q.px + q.py * q.py;
     bool pz_in_gap = q.pz < g.z_gt_pore && q.pz > g.z_gb;
-    if (pz_in_gap && pr2 < p.lt_Rg && q.x * q.x + q.y * q.y > p.gt_Rg) { bits |= 1u << 5; pore_side_wall<MODE>(p, q, g.R_g_c); }
-    if (pr2 > p.gt_Rp && q.z < g.z_gb && pz_in_gap) { bits |= 1u << 6; pore_plane_wall<MODE>(p, q, g.z_gb); }
-    if (pr2 > p.gt_Rp && q.z > g.z_gt_pore && pz_in_gap) { bits |= 1u << 7; pore_plane_wall<MODE>(p, q, g.z_gt_pore); }
+    if (pz_in_gap && pr2 < p.lt_Rg && q.x * q.x + q.y * q.y > p.gt_Rg) { bits |= 1u << 5; pore_side_wall<MODE, SURF>(p, q, g.R_g_c, 5, sp); }
+    if (pr2 > p.gt_Rp && q.z < g.z_gb && pz_in_gap) { bits |= 1u << 6; pore_plane_wall<MODE, SURF>(p, q, g.z_gb, 6, sp); }
+    if (pr2 > p.gt_Rp && q.z > g.z_gt_pore && pz_in_gap) { bits |= 1u << 7; pore_plane_wall<MODE, SURF>(p, q, g.z_gt_pore, 7, sp); }
     if (pr2 < p.lt_Rp && q.x * q.x + q.y * q.y > p.gt_Rp &&
-        ((q.z < g.z_cold && q.z > g.z_gt_pore) || (q.z < g.z_gb && q.z > g.oah))) { bits |= 1u << 8; pore_side_wall<MODE>(p, q, g.R_p_c); }
+        ((q.z < g.z_cold && q.z > g.z_gt_pore) || (q.z < g.z_gb && q.z > g.oah))) { bits |= 1u << 8; pore_side_wall<MODE, SURF>(p, q, g.R_p_c, 8, sp); }
     return bits;
 }
 
@@ -456,16 +481,23 @@ __device__ __forceinline__ void temp_energized(const P &p, Part &q, double t, co
 }
 
 // specular Temp cases: no MFP bookkeeping (Temp:311-347)
-template <int MODE = 1>
-__device__ __forceinline__ void temp_specular(const P &p, int c, Part &q)
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ void temp_specular(const P &p, int c, Part &q, const SurfP *sp = nullptr)
 {
     if (c == AMC_CASE_1) {
         double t;
-        if (!side_quadratic(q.x, q.y, q.vx, q.vy, p.g.R_oa_c, t)) { if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull); return; }
+        if (!side_quadratic(q.x, q.y, q.vx, q.vy, p.g.R_oa_c, t)) {
+            if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull);
+            if (SURF && MODE == AMC_LIVE) surf_outside(*sp, c);
+            return;
+        }
+        const double vx = q.vx, vy = q.vy, cx = q.x - vx * t, cy = q.y - vy * t, cz = q.z - q.vz * t;
         reflect_xy(q, p.g.R_oa_c, t);
+        if (SURF && MODE == AMC_LIVE) surf_record(p, *sp, c, cx, cy, cz, q.vx - vx, q.vy - vy, 0.0, 0.0);
     } else {
         double zp = temp_plane(p.g, c);
         double t = (q.z - zp) / q.vz;
+        if (SURF && MODE == AMC_LIVE) surf_record(p, *sp, c, q.x - q.vx * t, q.y - q.vy * t, zp, 0.0, 0.0, -q.vz - q.vz, 0.0);
         q.vz = -q.vz;
         q.z = zp + t * q.vz;
     }
@@ -562,8 +594,8 @@ __device__ __forceinline__ bool temp_any_mask(const P &p, const Part &q)
 }
 
 // all ten Temp cases on one particle with device RNG (Temp:693-753)
-template <int MODE = 1>
-__device__ __forceinline__ uint32_t temp_walls_device(const P &p, Part &q, int64_t id)
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ uint32_t temp_walls_device(const P &p, Part &q, int64_t id, const SurfP *sp = nullptr)
 {
     uint32_t bits = 0;
     if (!temp_any_mask(p, q)) return 0;
@@ -571,30 +603,55 @@ __device__ __forceinline__ uint32_t temp_walls_device(const P &p, Part &q, int64
     for (int c = 0; c < AMC_NUM_CASES; c++) {
         if (!temp_mask(p, c, q)) continue;
         bits |= 1u << c;
-        if (c <= AMC_CASE_2B) { temp_specular<MODE>(p, c, q); continue; }
+        if (c <= AMC_CASE_2B) { temp_specular<MODE, SURF>(p, c, q, sp); continue; }
         double t, col[3], nrm[3], dir[3], dpz, dE;
-        if (!temp_contact(p.g, c, q, t, col, nrm)) { if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull); continue; }
+        if (!temp_contact(p.g, c, q, t, col, nrm)) {
+            if (MODE == AMC_LIVE) atomicAdd(&p.stats->errors, 1ull);
+            if (SURF && MODE == AMC_LIVE) surf_outside(*sp, c);
+            continue;
+        }
         philox_direction(p, id, c, nrm, dir);
         double Es = c == AMC_CASE_4 ? cheb_eval(p, col[2]) : (temp_is_cold(c) ? p.g.E_cold : p.g.E_hot);
         double alpha = c == AMC_CASE_4 ? p.g.alpha_g : p.g.alpha_c;
+        const double vx = q.vx, vy = q.vy, vz = q.vz;
         temp_energized<MODE>(p, q, t, col, dir, Es, alpha, dpz, dE);
         if (MODE != AMC_LIVE) continue;
+        if (SURF) surf_record(p, *sp, c, col[0], col[1], col[2], q.vx - vx, q.vy - vy, q.vz - vz, dE);
         acc_add(p.stats->dpz, dpz, SC_P1, SC_P1I, SC_P2);
         if (c != AMC_CASE_4) acc_add(temp_is_cold(c) ? p.stats->ecold : p.stats->ehot, dE, SC_E1, SC_E1I, SC_E2);
     }
     return bits;
 }
 
-// Cube: six specular planes, x then y then z, max wall before min wall (Cube:192-226)
-__device__ __forceinline__ uint32_t cube_walls(const P &p, Part &q)
+// contact point of a cube face hit (face of case c on axis c / 2 at coordinate L): (x, y, z) - v * t with the face's own
+// coordinate set to L
+__device__ __forceinline__ void cube_record(const P &p, const SurfP &sp, const int c, const Part &q, const double t, const double L, const double dva)
+{
+    const int a = c >> 1;
+    const double cx = a == 0 ? L : q.x - q.vx * t, cy = a == 1 ? L : q.y - q.vy * t, cz = a == 2 ? L : q.z - q.vz * t;
+    surf_record(p, sp, c, cx, cy, cz, a == 0 ? dva : 0.0, a == 1 ? dva : 0.0, a == 2 ? dva : 0.0, 0.0);
+}
+
+// Cube: six specular planes, x then y then z, max wall before min wall (Cube:192-226).  SURF (live runs only): record
+// every hit at the contact point the same rewind gives, taken on the particle as it stands when its axis is handled
+template <int MODE = 1, bool SURF = false>
+__device__ __forceinline__ uint32_t cube_walls(const P &p, Part &q, const SurfP *sp = nullptr)
 {
     uint32_t bits = 0;
     double *pos[3] = {&q.x, &q.y, &q.z}, *vel[3] = {&q.vx, &q.vy, &q.vz};
 #pragma unroll
     for (int a = 0; a < 3; a++) {
         double L = p.cube[a];
-        if (*pos[a] > L) { double t = (*pos[a] - L) / *vel[a]; *vel[a] = -*vel[a]; *pos[a] = L + t * *vel[a]; bits |= 1u << (2 * a); }
-        if (*pos[a] < 0) { double t = *pos[a] / *vel[a]; *vel[a] = -*vel[a]; *pos[a] = t * *vel[a]; bits |= 1u << (2 * a + 1); }
+        if (*pos[a] > L) {
+            double t = (*pos[a] - L) / *vel[a];
+            if (SURF && MODE == AMC_LIVE) cube_record(p, *sp, 2 * a, q, t, L, -*vel[a] - *vel[a]);
+            *vel[a] = -*vel[a]; *pos[a] = L + t * *vel[a]; bits |= 1u << (2 * a);
+        }
+        if (*pos[a] < 0) {
+            double t = *pos[a] / *vel[a];
+            if (SURF && MODE == AMC_LIVE) cube_record(p, *sp, 2 * a + 1, q, t, 0.0, -*vel[a] - *vel[a]);
+            *vel[a] = -*vel[a]; *pos[a] = t * *vel[a]; bits |= 1u << (2 * a + 1);
+        }
     }
     return bits;
 }
@@ -633,6 +690,71 @@ __device__ __forceinline__ int32_t owner_key(const P &p, double x, double y, dou
     if (o[0] == p.nc[0] || o[1] == p.nc[1] || o[2] == p.nc[2]) return p.ncell_pad;
     return ((o[0] + 1) * p.pnc[1] + (o[1] + 1)) * p.pnc[2] + (o[2] + 1);
 }
+// ---------------------------------------------------------------- surface recording (amc_surface_*)
+// One wall interaction of case c: contact point (cx, cy, cz), velocity change dv = v_out - v_in of the particle, energy
+// dE the gas gained.  The binning, the wall-local components and the limbs are defined in include/amc.h (a NumPy
+// restatement mirrors every expression).  Out of line: the recording instantiations carry one call per wall helper, the
+// streaming kernels none.
+// bin k of v with tab[k] <= v < tab[k+1], 0 <= k < n, or -1 (NaN included); est: estimate of k.  Self-contained rather
+// than owner_axis: a call from here with a pointer of the SurfP parameter would turn the global loads of the shared
+// owner_axis_slow into generic ones in every kernel of the library.
+__device__ __forceinline__ int surf_bin(const double *tab, const int n, const double est, const double v)
+{
+    if (!(v >= tab[0] && v < tab[n])) return -1;
+    int k = min(max(__double2int_rd(est), 0), n - 1);
+    while (v < tab[k]) --k;
+    while (v >= tab[k + 1]) ++k;
+    return k;
+}
+// bin of coordinate v on axis a of the layout's grid (z: the global edges on a slab handle)
+__device__ __forceinline__ int surf_axis_bin(const P &p, const SurfP &sp, const int a, const double v)
+{
+    return a == 2 ? surf_bin(sp.zedge, sp.ncz, (v - sp.ze0) * sp.zinv, v) : surf_bin(p.edge[a], p.nc[a], (v - p.e0[a]) * p.inv_d[a], v);
+}
+__device__ __forceinline__ bool surf_is_side(const int kind, const int c)
+{
+    return kind != AMC_KIND_CUBE && (c == AMC_CASE_1 || c == AMC_CASE_4 || c == AMC_CASE_6H || c == AMC_CASE_6C);
+}
+__device__ __noinline__ void surf_record(const P &p, const SurfP &sp, const int c, const double cx, const double cy, const double cz,
+                                         const double dvx, const double dvy, const double dvz, const double dE)
+{
+    static_assert(AMC_SURF_WORDS == 9 && AMC_SURF_V1 == 16 && AMC_SURF_V2 == 46 && AMC_SURF_E1 == 90 && AMC_SURF_E2 == 120,
+                  "scales of surf_record");
+    int e = -1; /* element inside the case, -1: outside every bin */
+    double dn, d1, d2;
+    if (p.kind == AMC_KIND_CUBE) {
+        const int a = c >> 1, b1 = a == 0 ? 1 : 0, b2 = a == 2 ? 1 : 2;
+        const double col[3] = {cx, cy, cz}, dv[3] = {dvx, dvy, dvz};
+        dn = (c & 1) ? dv[a] : -dv[a]; /* even case: the face at cube[a], normal -e_a; odd: the face at 0, normal +e_a */
+        d1 = dv[b1]; d2 = dv[b2];
+        const int o1 = surf_axis_bin(p, sp, b1, col[b1]), o2 = surf_axis_bin(p, sp, b2, col[b2]);
+        if (o1 >= 0 && o2 >= 0) e = o1 * (b2 == 2 ? sp.ncz : p.nc[b2]) + o2;
+    } else if (surf_is_side(p.kind, c)) {
+        const double Rc = c == AMC_CASE_1 ? p.g.R_oa_c : (c == AMC_CASE_4 ? p.g.R_g_c : p.g.R_p_c);
+        const double ex = cx / Rc, ey = cy / Rc;
+        dn = -(dvx * ex + dvy * ey); d1 = dvz; d2 = dvy * ex - dvx * ey;
+        e = surf_axis_bin(p, sp, 2, cz);
+    } else {
+        const double r2 = cx * cx + cy * cy, r = sqrt(r2);
+        const double ex = r > 0.0 ? cx / r : 1.0, ey = r > 0.0 ? cy / r : 0.0;
+        dn = (c == AMC_CASE_2A || c == AMC_CASE_3C || c == AMC_CASE_5B) ? dvz : -dvz;
+        d1 = dvx * ex + dvy * ey; d2 = dvy * ex - dvx * ey;
+        e = surf_bin(sp.rsq, sp.nann, r * sp.inv_dr, r2);
+    }
+    if (e < 0) { surf_outside(sp, c); return; }
+    unsigned long long *w = sp.acc + (int64_t)(sp.off[c] + e) * AMC_SURF_WORDS;
+    atomicAdd(w, 1ull);
+    acc_add(w + 1, dn, 0x1p16, 0x1p-16, 0x1p46);
+    acc_add(w + 3, d1, 0x1p16, 0x1p-16, 0x1p46);
+    acc_add(w + 5, d2, 0x1p16, 0x1p-16, 0x1p46);
+    acc_add(w + 7, dE, 0x1p90, 0x1p-90, 0x1p120);
+}
+// a hit the case counts but applies nothing to (the reference's floating-point error path)
+__device__ __noinline__ void surf_outside(const SurfP &sp, const int c)
+{
+    atomicAdd(sp.acc + (int64_t)sp.off[AMC_NUM_CASES] * AMC_SURF_WORDS + c, 1ull);
+}
+
 // true when the coordinate lies inside the low-side band of the next cell up on this axis, i.e. the
 // particle can be a member of a reference cell other than its owner cell (Pore:527-529)
 __device__ __forceinline__ bool in_next_band(const double *lo, int nc, int owner, double v)

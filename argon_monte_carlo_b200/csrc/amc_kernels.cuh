@@ -84,7 +84,9 @@ __device__ __forceinline__ int warp_rank(int32_t *counter, int tag)
 //   walls         Pore:442-485 / Temp:693-753 (device RNG) / Cube:192-226
 //   recapture     Pore:354-375 / Temp:560-616
 //   keys          owner cell of the final position + rank inside that cell (counting sort, pass 1)
-__global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect(const __grid_constant__ P p, const int phase)
+// k_advect_surf: the same with the wall interactions recorded (amc_surface_*), launched only while recording is on
+template <bool SURF>
+__device__ __forceinline__ void advect_body(const P &p, const int phase, const SurfP *sp)
 {
     int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= p.n) return;
@@ -116,7 +118,8 @@ __global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect(const __grid_const
         q.px = p.px[s]; q.py = p.py[s]; q.pz = p.pz[s];
     }
     if (phase & PH_WALLS) {
-        uint32_t bits = p.kind == AMC_KIND_PORE ? pore_walls(p, q) : (p.kind == AMC_KIND_TEMP ? temp_walls_device(p, q, id) : cube_walls(p, q));
+        uint32_t bits = p.kind == AMC_KIND_PORE ? pore_walls<AMC_LIVE, SURF>(p, q, sp)
+                                                : (p.kind == AMC_KIND_TEMP ? temp_walls_device<AMC_LIVE, SURF>(p, q, id, sp) : cube_walls<AMC_LIVE, SURF>(p, q, sp));
         if (bits) {
             for (uint32_t b = bits; b; b &= b - 1) atomicAdd(&p.stats->wall_hits[__ffs(b) - 1], 1ull);
         }
@@ -183,6 +186,11 @@ __global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect(const __grid_const
         p.rank[s] = band ? r : ~r;
     }
 }
+__global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect(const __grid_constant__ P p, const int phase) { advect_body<false>(p, phase, nullptr); }
+__global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect_surf(const __grid_constant__ P p, const int phase, const __grid_constant__ SurfP sp)
+{
+    advect_body<true>(p, phase, &sp);
+}
 
 // ------------------------------------------------------------------------------------------------
 // The fused timestep streams the state ONCE through the SM instead of twice: a light first pass finds out
@@ -192,9 +200,10 @@ __global__ void __launch_bounds__(ADVECT_THREADS, 4) k_advect(const __grid_const
 // advance_particle is the per-particle part of a timestep before the pair pass (closing recapture of
 // the previous step, drift, wall cases, recapture; same references as k_advect).  MODE = AMC_DRY is a
 // dry run: same arithmetic and therefore bit-identical positions, but no counters, no completed paths,
-// no path-length bookkeeping -- none of which feeds back into the position.
-template <int MODE>
-__device__ __forceinline__ void advance_particle(const P &p, Part &q, const int32_t id, const int phase)
+// no path-length bookkeeping -- none of which feeds back into the position.  SURF: the live run records the wall
+// interactions (amc_surface_*).
+template <int MODE, bool SURF = false>
+__device__ __forceinline__ void advance_particle(const P &p, Part &q, const int32_t id, const int phase, const SurfP *sp = nullptr)
 {
     // Calm particles (energized pore, ~95 % of the gas): both the position before the drift and the one after it
     // lie in one of three regions in which every wall mask (Temp:693-753), every recapture condition (Temp:594-616)
@@ -239,7 +248,8 @@ __device__ __forceinline__ void advance_particle(const P &p, Part &q, const int3
         }
     }
     if (phase & PH_WALLS) {
-        uint32_t bits = p.kind == AMC_KIND_PORE ? pore_walls<MODE>(p, q) : (p.kind == AMC_KIND_TEMP ? temp_walls_device<MODE>(p, q, id) : cube_walls(p, q));
+        uint32_t bits = p.kind == AMC_KIND_PORE ? pore_walls<MODE, SURF>(p, q, sp)
+                                                : (p.kind == AMC_KIND_TEMP ? temp_walls_device<MODE, SURF>(p, q, id, sp) : cube_walls<MODE, SURF>(p, q, sp));
         if (MODE == AMC_LIVE) {
             for (uint32_t b = bits; b; b &= b - 1) atomicAdd(&p.stats->wall_hits[__ffs(b) - 1], 1ull);
             if (p.wall_bits) p.wall_bits[id] = (uint16_t)bits;
@@ -357,9 +367,10 @@ __global__ void __launch_bounds__(ADVECT_THREADS, SLAB ? KEYS_OCC_SLAB : KEYS_OC
 
 // pass 2: the timestep proper, written straight to the particle's slot in owner-cell order.  Slab mode: the
 // particles unpacked behind the resident ones (slots n .. n + n_in) arrive already advanced; ghosts of the last
-// step and emigrants go to the bucket behind the last cell and are dropped.
-template <bool SLAB>
-__global__ void __launch_bounds__(ADVECT_THREADS, 3) k_scatter_advect(const __grid_constant__ P p, const int phase)
+// step and emigrants go to the bucket behind the last cell and are dropped.  k_scatter_advect_surf: the same with the wall
+// interactions recorded (see k_advect).
+template <bool SLAB, bool SURF>
+__device__ __forceinline__ void scatter_advect_body(const P &p, const int phase, const SurfP *sp)
 {
     int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= (SLAB ? p.cap : p.n)) return;
@@ -370,7 +381,7 @@ __global__ void __launch_bounds__(ADVECT_THREADS, 3) k_scatter_advect(const __gr
     if (SLAB && s >= n0 + *p.n_in) return;
     if (s < n0 && !(SLAB && (q.flag & AMC_FLAG_GHOST))) {
         q.flag &= AMC_FLAG_PATH;
-        advance_particle<AMC_LIVE>(p, q, id, phase);
+        advance_particle<AMC_LIVE, SURF>(p, q, id, phase, sp);
         if (SLAB) {
             const unsigned aux = p.aux[s];
             if (aux & AUX_GHOST_UP) q.flag |= AMC_FLAG_REL_UP;
@@ -393,6 +404,16 @@ __global__ void __launch_bounds__(ADVECT_THREADS, 3) k_scatter_advect(const __gr
             if (j < p.bnd_cap) p.bnd_dirty[0][j] = (int32_t)t; else atomicAdd(p.slab_overflow + 2, 1ull);
         }
     }
+}
+template <bool SLAB>
+__global__ void __launch_bounds__(ADVECT_THREADS, 3) k_scatter_advect(const __grid_constant__ P p, const int phase)
+{
+    scatter_advect_body<SLAB, false>(p, phase, nullptr);
+}
+template <bool SLAB>
+__global__ void __launch_bounds__(ADVECT_THREADS, 3) k_scatter_advect_surf(const __grid_constant__ P p, const int phase, const __grid_constant__ SurfP sp)
+{
+    scatter_advect_body<SLAB, true>(p, phase, &sp);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1988,8 +2009,9 @@ __global__ void __launch_bounds__(SWE_THREADS) k_sweep_events(const __grid_const
 
 // ------------------------------------------------------------------------------------------------
 // host-RNG parity mode (AMC_KIND_TEMP): one wall case at a time (Temp:693-753)
-// specular cases 1, 2a, 2b applied directly; returns the hit count in stats->wall_hits[c]
-__global__ void __launch_bounds__(ADVECT_THREADS) k_case_specular(const __grid_constant__ P p, const int c)
+// specular cases 1, 2a, 2b applied directly; returns the hit count in stats->wall_hits[c].  sp.acc != null: record the
+// hits (amc_surface_*), here and in k_case_apply
+__global__ void __launch_bounds__(ADVECT_THREADS) k_case_specular(const __grid_constant__ P p, const int c, const __grid_constant__ SurfP sp)
 {
     int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= p.n) return;
@@ -1999,7 +2021,8 @@ __global__ void __launch_bounds__(ADVECT_THREADS) k_case_specular(const __grid_c
     if (!temp_mask(p, c, q)) return;
     atomicAdd(&p.stats->wall_hits[c], 1ull);
     if (p.wall_bits) p.wall_bits[p.a.pos[s].id] |= (uint16_t)(1u << c);
-    temp_specular(p, c, q);
+    if (sp.acc) temp_specular<AMC_LIVE, true>(p, c, q, &sp);
+    else temp_specular(p, c, q);
     store_part(p.a, s, q);
 }
 // energized cases: list the hits (slot, id, normal, contact height); order fixed up on the host
@@ -2023,7 +2046,8 @@ __global__ void __launch_bounds__(ADVECT_THREADS) k_case_detect(const __grid_con
 }
 __global__ void __launch_bounds__(ADVECT_THREADS) k_case_apply(const __grid_constant__ P p, const int c, int32_t nh,
                                                                const int32_t *slots, const double *dirs,
-                                                               const double *surf_e, double *out_dpz, double *out_de)
+                                                               const double *surf_e, double *out_dpz, double *out_de,
+                                                               const __grid_constant__ SurfP sp)
 {
     int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= nh) return;
@@ -2035,11 +2059,17 @@ __global__ void __launch_bounds__(ADVECT_THREADS) k_case_apply(const __grid_cons
     atomicAdd(&p.stats->wall_hits[c], 1ull);
     if (p.wall_bits) p.wall_bits[p.a.pos[s].id] |= (uint16_t)(1u << c);
     double t, col[3], nrm[3], dpz, dE;
-    if (!temp_contact(p.g, c, q, t, col, nrm)) { atomicAdd(&p.stats->errors, 1ull); return; }
+    if (!temp_contact(p.g, c, q, t, col, nrm)) {
+        atomicAdd(&p.stats->errors, 1ull);
+        if (sp.acc) surf_outside(sp, c);
+        return;
+    }
     double dir[3] = {dirs[3 * k], dirs[3 * k + 1], dirs[3 * k + 2]};
     double Es = c == AMC_CASE_4 ? surf_e[k] : (temp_is_cold(c) ? p.g.E_cold : p.g.E_hot);
     double alpha = c == AMC_CASE_4 ? p.g.alpha_g : p.g.alpha_c;
+    const double vx = q.vx, vy = q.vy, vz = q.vz;
     temp_energized(p, q, t, col, dir, Es, alpha, dpz, dE);
+    if (sp.acc) surf_record(p, sp, c, col[0], col[1], col[2], q.vx - vx, q.vy - vy, q.vz - vz, dE);
     out_dpz[k] = dpz; out_de[k] = c == AMC_CASE_4 ? 0.0 : dE;
     store_part(p.a, s, q);
 }

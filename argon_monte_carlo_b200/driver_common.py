@@ -27,10 +27,36 @@ def parse_args(default_steps, description, temp=False, argv=None):
                     help="sample density, flow velocity and temperature per collision cell after every K-th timestep "
                          "and write profile_z.csv (default 0: off)")
     ap.add_argument("--sample-start", type=int, default=0, metavar="S", help="first timestep sampled (default 0)")
+    ap.add_argument("--surface-start", type=int, default=None, metavar="S",
+                    help="record wall pressure, shear stress and heat flux per wall element from timestep S to the end "
+                         "and write surface.csv (default: off)")
     args = ap.parse_args(argv)
     if args.sample_every < 0 or args.sample_start < 0:
         ap.error("--sample-every and --sample-start must be >= 0")
+    if args.surface_start is not None and args.surface_start < 0:
+        ap.error("--surface-start must be >= 0")
     return args
+
+
+def surface_chunk(sim, args, done, chunk):
+    """The number of timesteps to take from timestep `done` on, at most `chunk`: a batch never straddles
+    --surface-start, and recording starts when the run reaches it."""
+    s = args.surface_start
+    if s is None:
+        return chunk
+    if done >= s and not sim.surface_on:
+        sim.surface_enable()
+    return s - done if done < s < done + chunk else chunk
+
+
+def surface_finish(sim, cfg, args):
+    """Write surface.csv (one row per wall element) into --outdir if --surface-start was given."""
+    if args.surface_start is None:
+        return
+    if not sim.surface_on:      # the run ended before timestep S: nothing recorded
+        sim.surface_enable()
+    grid = getattr(sim, "sample_grid", cfg.grid)
+    outputs.write_surface_csv(os.path.join(args.outdir, "surface.csv"), outputs.surface_fields(sim.surface_raw(), cfg, grid, sim.kind))
 
 
 def sampling_begin(sim, args):

@@ -146,3 +146,103 @@ def write_axial_profile(path, profile):
         for k in range(len(profile["z_lo"])):
             f.write(",".join(str(int(profile[c][k])) if c == "samples" else "%.17g" % float(profile[c][k])
                              for c in PROFILE_COLUMNS) + "\n")
+
+
+# ---------------------------------------------------------------- wall surfaces (amc_surface_*)
+SURFACE_COLUMNS = ("element", "case", "lo1", "hi1", "lo2", "hi2", "area", "hits", "number_flux", "pressure", "shear_1",
+                   "shear_2", "heat_flux")
+
+
+def decode_surface_sums(acc):
+    """acc [elements][9] uint64 (Simulation.surface_raw) -> (hits [elements], sums [elements, 4]: dv.n, dv.t1, dv.t2
+    in m/s and dE in J) as float64, each sum high * 2^-S1 + low * 2^-S2 of its signed limbs (include/amc.h)."""
+    from .amc import SURF_E1, SURF_E2, SURF_V1, SURF_V2, SURF_WORDS
+    w = np.ascontiguousarray(acc, dtype=np.uint64).reshape(-1, SURF_WORDS).view(np.int64)
+    dec = lambda j, s1, s2: np.ldexp(w[:, j].astype(np.float64), -s1) + np.ldexp(w[:, j + 1].astype(np.float64), -s2)
+    sums = np.stack([dec(1, SURF_V1, SURF_V2), dec(3, SURF_V1, SURF_V2), dec(5, SURF_V1, SURF_V2), dec(7, SURF_E1, SURF_E2)], axis=1)
+    return w[:, 0].view(np.uint64).astype(np.float64), sums
+
+
+def wall_extents(cfg, kind):
+    """Per case the extent of its contact surface along the binned coordinate: cylinders (radius, [(z_lo, z_hi), ...]),
+    planes (z, r_lo, r_hi), from the z and radial conditions of the case masks (Pore:442-485, Temp:693-753).  The
+    open-air side wall has no z condition; particles reach it in the two open-air regions only."""
+    from .amc import KIND_PORE
+    g = cfg.geom
+    oa = [(0.0, g.oah), (g.z_cold, g.H)]
+    if kind == KIND_PORE:
+        return {0: ("side", g.R_oa_c, oa), 1: ("plane", 0.0, 0.0, g.R_oa_c), 2: ("plane", g.H, 0.0, g.R_oa_c),
+                3: ("plane", g.z_cold, g.R_p, g.R_oa_c), 4: ("plane", g.oah, g.R_p, g.R_oa_c),
+                5: ("side", g.R_g_c, [(g.z_gb, g.z_gt_pore)]), 6: ("plane", g.z_gb, g.R_p, g.R_g_c),
+                7: ("plane", g.z_gt_pore, g.R_p, g.R_g_c), 8: ("side", g.R_p_c, [(g.oah, g.z_gb), (g.z_gt_pore, g.z_cold)])}
+    return {0: ("side", g.R_oa_c, oa), 1: ("plane", 0.0, 0.0, g.R_oa_c), 2: ("plane", g.H, 0.0, g.R_oa_c),
+            3: ("plane", g.zc3, g.R_p, g.R_oa_c), 4: ("plane", g.zh3, g.R_p, g.R_oa_c), 5: ("side", g.R_g_c, [(g.zgb_p, g.zgt_m)]),
+            6: ("plane", g.zgb_p, g.R_p_c, g.R_g_c), 7: ("plane", g.zgt_m, g.R_p_c, g.R_g_c),
+            8: ("side", g.R_p_c, [(g.zh3, g.zgb_p)]), 9: ("side", g.R_p_c, [(g.zgt_m, g.zc3)])}
+
+
+def surface_geometry(cfg, layout):
+    """Per element: case, coordinate ranges (lo1, hi1, lo2, hi2: z for cylinders, r for annuli, the two in-plane
+    axes for cube faces; lo2 / hi2 NaN where there is one coordinate) and the area of the contact surface the element
+    covers: radius Rc for cylinders, the shifted planes (zc3 etc.), each clipped to its wall's extent."""
+    n = layout.n_elements
+    case = np.zeros(n, dtype=np.int64)
+    rng = np.full((n, 4), np.nan)
+    area = np.zeros(n)
+    ext = None if layout.kind == 0 else wall_extents(cfg, layout.kind)
+    for c in range(len(layout.types)):
+        a0, a1 = int(layout.offsets[c]), int(layout.offsets[c + 1])
+        if a1 == a0:
+            continue
+        case[a0:a1] = c
+        t = layout.types[c]
+        if t == "face":
+            _, b1, b2 = layout.face_axes(c)
+            L = (cfg.cube_x, cfg.cube_y, cfg.cube_z)
+            e1, e2 = layout.edges[b1], layout.edges[b2]
+            w1 = _overlap(e1[:-1], e1[1:], 0.0, float(L[b1]))
+            w2 = _overlap(e2[:-1], e2[1:], 0.0, float(L[b2]))
+            rng[a0:a1] = np.stack([np.repeat(e1[:-1], len(w2)), np.repeat(e1[1:], len(w2)),
+                                   np.tile(e2[:-1], len(w1)), np.tile(e2[1:], len(w1))], axis=1)
+            area[a0:a1] = np.outer(w1, w2).ravel()
+        elif t == "side":
+            _, Rc, spans = ext[c]
+            z = layout.zedge
+            rng[a0:a1, 0], rng[a0:a1, 1] = z[:-1], z[1:]
+            area[a0:a1] = 2.0 * np.pi * float(Rc) * sum(_overlap(z[:-1], z[1:], float(lo), float(hi)) for lo, hi in spans)
+        else:
+            _, _, rlo, rhi = ext[c]
+            r = np.sqrt(layout.rsq)
+            rng[a0:a1, 0], rng[a0:a1, 1] = r[:-1], r[1:]
+            lo, hi = np.maximum(r[:-1], float(rlo)), np.minimum(r[1:], float(rhi))
+            area[a0:a1] = np.where(hi > lo, np.pi * (hi * hi - lo * lo), 0.0)
+    return case, rng, area
+
+
+def surface_fields(raw, cfg, grid, kind):
+    """Per wall element of raw = (acc, n_steps, outside) (Simulation.surface_raw) on `grid` for a handle of `kind`: the
+    SURFACE_COLUMNS -- case, coordinate ranges and area (surface_geometry), hits, number flux hits / (A n_steps dt)
+    (1 / (m^2 s)), pressure m sum(dv.n) / (A n_steps dt) and the shear components m sum(dv.t) / (A n_steps dt) (Pa),
+    heat flux into the wall -sum(dE) / (A n_steps dt) (W / m^2).  Elements of zero area give NaN rates."""
+    from .amc import surface_layout_of
+    acc, n_steps, _ = raw
+    layout = surface_layout_of(cfg, kind, grid)
+    case, rng, area = surface_geometry(cfg, layout)
+    hits, sums = decode_surface_sums(acc)
+    m = float(cfg.argon_mass)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        denom = np.where(area > 0, area, np.nan) * (float(n_steps) * float(cfg.dt))
+        return {"element": np.arange(layout.n_elements), "case": case, "lo1": rng[:, 0], "hi1": rng[:, 1], "lo2": rng[:, 2],
+                "hi2": rng[:, 3], "area": area, "hits": acc[:, 0].astype(np.uint64), "number_flux": hits / denom,
+                "pressure": m * sums[:, 0] / denom, "shear_1": m * sums[:, 1] / denom, "shear_2": m * sums[:, 2] / denom,
+                "heat_flux": -sums[:, 3] / denom, "n_steps": int(n_steps)}
+
+
+def write_surface_csv(path, fields):
+    """surface.csv: one row per wall element, the SURFACE_COLUMNS (lengths in m, areas in m^2, number flux in
+    1 / (m^2 s), pressure and shear in Pa, heat flux into the wall in W / m^2), floats with 17 significant digits."""
+    ints = ("element", "case", "hits")
+    with open(path, "w") as f:
+        f.write(",".join(SURFACE_COLUMNS) + "\n")
+        for k in range(len(fields["element"])):
+            f.write(",".join(str(int(fields[c][k])) if c in ints else "%.17g" % float(fields[c][k]) for c in SURFACE_COLUMNS) + "\n")

@@ -562,6 +562,26 @@ class SlabSimulation:
     def last_sample_ms(self):
         return [r.sim.last_sample_ms() for r in self.ranks]
 
+    # ------------------------------------------------------------------ surface recording
+    def surface_enable(self):
+        """Surface recording on every local rank (Simulation.surface_enable); a hit is recorded by the rank that owns
+        the particle, on the global grid, so the merged accumulators equal those of the single-domain run bit for bit."""
+        for r in self.ranks:
+            r.sim.surface_enable()
+
+    def surface_disable(self):
+        for r in self.ranks:
+            r.sim.surface_disable()
+
+    def surface_raw(self, reduce=True):
+        """(acc, wall phases recorded, outside) summed over the local ranks and, with a distributed transport and
+        reduce=True, over all processes (element-wise uint64 sums)."""
+        acc, ns, out = amc.merge_surface_ranks([r.sim.surface_raw() for r in self.ranks])
+        if reduce and not isinstance(self.transport, LocalTransport):
+            acc = self.transport.allreduce_u64(acc)
+            out = self.transport.allreduce_u64(out)
+        return acc, ns, out
+
     def histograms(self):
         counts, n, sums = None, 0, None
         for r in self.ranks:

@@ -263,6 +263,61 @@ int amc_sample_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_samples, uint64
 int amc_sample_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_samples, uint64_t n_outside);
 int amc_last_sample_ms(amc_handle *h, double *ms);
 
+/* Surface recording: what the gas does to the walls, per wall element, accumulated on the device as every wall
+ * interaction happens.  The walls are the AMC_CASE_* slots of the handle's kind (Pore 9, Temp 10, Cube 6; a case the
+ * kind does not have has no element), each cut into bins on the handle's sampling grid (that of amc_sample_*; a slab
+ * handle: the global z edges).  c = (cx, cy, cz) is the contact point of a hit:
+ *   cylinders (Pore 0, 5, 8; Temp 1, 4, 6H, 6C; radius Rc = R_oa_c, R_g_c, R_p_c): the z layer k of cz with
+ *     edge[k] <= cz < edge[k+1] (the rows of profile_z.csv)
+ *   planes of Pore / Temp: the annulus k with rsq[k] <= cx*cx + cy*cy < rsq[k+1], rsq[k] = (k*dr) * (k*dr) in fp64,
+ *     dr = (edge_x[nc_x] - edge_x[0]) / nc_x, k < ceil(R_oa / dr)
+ *   cube faces (case 2a: the face x = cube[a], 2a+1: the face x_a = 0): the pair of owner cells (o1, o2) of the two
+ *     in-plane axes b1 < b2, element o1 * nc[b2] + o2
+ * Elements are numbered case-major (amc_surface_layout: offsets[c] .. offsets[c+1]).  A hit in no bin -- a NaN contact,
+ * a contact outside the grid, or the reference's floating-point error path (the case counts a hit and applies nothing)
+ * -- counts in outside[c] instead, so per case the hits of the elements plus outside[c] equal the sum of wall_hits[c].
+ * Contact points: planes (x - vx*t, y - vy*t, zp) with t = (z - zp) / vz before the reflection; cylinders
+ * (x - vx*t, y - vy*t, z - vz*t) with t from the side-wall quadratic; energized cases the contact point of the reference
+ * (Temp:372-375, 440-444); cube faces the same rewind on the particle as it stands when its axis is handled, with the
+ * face's own coordinate set to the face.  With dv = v_out - v_in (fp64, per component) and with n the unit normal from
+ * the wall into the gas, every hit adds, in IEEE fp64 with separate roundings:
+ *   cylinders  ex = cx / Rc, ey = cy / Rc;  dv.n = -(dvx*ex + dvy*ey);  dv.t1 = dvz (t1 = z);  dv.t2 = dvy*ex - dvx*ey
+ *              (t2 = azimuth (-ey, ex, 0))
+ *   annuli     r = sqrt(cx*cx + cy*cy);  ex = cx / r, ey = cy / r (r = 0: ex = 1, ey = 0);  dv.n = s * dvz with
+ *              s = +1 for 2A / 3C / 5B (Pore 1, 3, 6) and -1 for 2B / 3H / 5T (Pore 2, 4, 7);  dv.t1 = dvx*ex + dvy*ey
+ *              (radial);  dv.t2 = dvy*ex - dvx*ey (azimuth)
+ *   cube faces dv.n = -dv_a on the face at cube[a], +dv_a on the face at 0;  dv.t1 = dv_b1, dv.t2 = dv_b2
+ * and dE, the energy the gas gained: the dE of the energized exchange (Temp:377-389) on energized cases -- case 4
+ * included, which the e_cold / e_hot series of amc_step_stats leave out -- and 0 on specular ones.  Per element
+ * AMC_SURF_WORDS uint64 words:
+ *   [0] hits;  [1..2] sum dv.n;  [3..4] sum dv.t1;  [5..6] sum dv.t2 (m/s);  [7..8] sum dE (J)
+ * every sum as two signed 64-bit fixed-point limbs, the scheme of amc_sample_*: S1 / S2 = AMC_SURF_V1 / _V2 for the
+ * velocities, AMC_SURF_E1 / _E2 for the energy.  Headroom: 10^9 hits per element at |v| <= 10^4 m/s (|dv| <= 2*10^4,
+ * |dE| <= 3.4e-18 J for argon) keep every limb inside the signed 64-bit range (worst case: 1.4e18 in a velocity high
+ * limb, 4.2e18 in the energy high limb, 5.4e17 in a low limb).
+ * Recorded wall phases: every timestep of amc_step and amc_slab_step, every amc_slab_advect and amc_walls call, and
+ * every amc_wall_case(h, AMC_CASE_1) (the first case of a host-RNG wall phase); *n_steps counts them, so that rates
+ * are sums / (n_steps * dt).  Not recorded: amc_wall_operator (operator-level parity entry point), and the recapture
+ * (a teleport, not a wall interaction).  A slab handle records a hit on the rank that owns the particle at the start
+ * of the step, so the element-wise sum (mod 2^64) of the raw arrays of all ranks equals the single-domain run's.
+ * Recording changes no state, counter, histogram or digest; while it is disabled (the default) no launch and no memory
+ * is added.  Memory: 8 * AMC_SURF_WORDS bytes per element.
+ *   amc_surface_enable   allocate, zero and start recording (a slab handle: after amc_slab_enable)
+ *   amc_surface_disable  free the accumulators
+ *   amc_surface_layout   offsets[AMC_NUM_CASES + 1]: first element of every case, offsets[AMC_NUM_CASES] = elements
+ *   amc_surface_get_raw  acc: [elements][AMC_SURF_WORDS] (nullable), wall phases recorded, outside (nullable)
+ *   amc_surface_set_raw  resume from amc_surface_get_raw's values (recording must be enabled) */
+#define AMC_SURF_WORDS 9
+#define AMC_SURF_V1 16
+#define AMC_SURF_V2 46
+#define AMC_SURF_E1 90
+#define AMC_SURF_E2 120
+int amc_surface_enable(amc_handle *h);
+int amc_surface_disable(amc_handle *h);
+int amc_surface_layout(amc_handle *h, int64_t offsets[AMC_NUM_CASES + 1]);
+int amc_surface_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_steps, uint64_t outside[AMC_NUM_CASES]);
+int amc_surface_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_steps, const uint64_t outside[AMC_NUM_CASES]);
+
 /* set the step counter that keys the device RNG (default: counts amc_step / amc_walls calls from 0) */
 int amc_set_step_index(amc_handle *h, int64_t step);
 
