@@ -93,12 +93,16 @@ EXPORTS = ("amc_create", "amc_destroy", "amc_last_error", "amc_abi_version", "am
            "amc_slab_p2p_setup", "amc_slab_p2p_connect", "amc_slab_step", "amc_wall_operator", "amc_seed_relax", "amc_last_scatter_ms",
            "amc_sample_enable", "amc_sample_disable", "amc_sample_now", "amc_sample_get_raw", "amc_sample_set_raw",
            "amc_last_sample_ms", "amc_surface_enable", "amc_surface_disable", "amc_surface_layout", "amc_surface_get_raw",
-           "amc_surface_set_raw")
+           "amc_surface_set_raw", "amc_vdf_enable", "amc_vdf_disable", "amc_vdf_layout", "amc_vdf_get_raw", "amc_vdf_set_raw")
 
 # field sampling (include/amc.h): words per cell and the binary scales of the fixed-point limbs
 SAMPLE_WORDS = 13
 SAMPLE_V1, SAMPLE_V2 = 19, 49     # velocity sums: high / low limb
 SAMPLE_Q1, SAMPLE_Q2 = 6, 36      # sums of squares: high / low limb
+
+# velocity distribution (include/amc.h): histograms per z layer (vx, vy, vz, speed) and the largest bin count
+VDF_HISTS = 4
+VDF_MAX_BINS = 4096
 
 # surface recording (include/amc.h): words per wall element and the binary scales of the fixed-point limbs
 SURF_WORDS = 9
@@ -374,6 +378,46 @@ def merge_surface_ranks(parts):
     return acc, ns.pop(), out
 
 
+def vdf_edges(n_bins, v_max):
+    """Bin edges of the velocity components and of the speed (amc_vdf_enable computes the same on the host)."""
+    v = float(v_max)
+    return np.linspace(-v, v, int(n_bins) + 1), np.linspace(0.0, v, int(n_bins) + 1)
+
+
+def vdf_words_of(values, n_bins, lo, hi):
+    """[under, bin 0 .. bin n_bins-1, over] of one histogram: np.histogram over [lo, hi] (last bin closed), values below
+    lo in under, above hi or NaN in over."""
+    values = np.asarray(values, dtype=np.float64)
+    inside, _ = np.histogram(values, bins=int(n_bins), range=(lo, hi))
+    under = int(np.count_nonzero(values < lo))
+    over = len(values) - under - int(inside.sum())
+    return np.concatenate([[under], inside, [over]]).astype(np.uint64)
+
+
+def vdf_of_arrays(state, grid, n_bins, v_max, ids=None):
+    """NumPy restatement of the VDF words one amc_sample_now adds for `state` (mapping with 'x', 'y', 'z', 'vx', 'vy',
+    'vz'): acc [ncz][VDF_HISTS][n_bins + 2] uint64, the layout of Simulation.vdf_raw.  The particles are those of the
+    field sample (sample_cells_of: inside the grid), the region is the z layer of their cell.  ids: optional indices
+    into the arrays selecting the particles (default: all)."""
+    sel = (lambda a: np.asarray(a, dtype=np.float64)) if ids is None else (lambda a: np.asarray(a, dtype=np.float64)[np.asarray(ids)])
+    cell, inside = sample_cells_of(sel(state["x"]), sel(state["y"]), sel(state["z"]), grid)
+    nz = sample_grid_shape(grid)[2]
+    layer = cell[inside] % nz
+    vx, vy, vz = (sel(state[k])[inside] for k in ("vx", "vy", "vz"))
+    with np.errstate(over="ignore", invalid="ignore"):
+        speed = np.sqrt((vx * vx + vy * vy) + vz * vz)
+    v = float(v_max)
+    acc = np.zeros((nz, VDF_HISTS, int(n_bins) + 2), dtype=np.uint64)
+    order = np.argsort(layer, kind="stable")
+    bounds = np.searchsorted(layer[order], np.arange(nz + 1))
+    cols = [(a[order], lo) for a, lo in ((vx, -v), (vy, -v), (vz, -v), (speed, 0.0))]
+    for k in range(nz):
+        if bounds[k] < bounds[k + 1]:
+            for j, (vals, lo) in enumerate(cols):
+                acc[k, j] = vdf_words_of(vals[bounds[k]:bounds[k + 1]], n_bins, lo, v)
+    return acc
+
+
 def combine_digests(parts):
     """Sum of per-rank digests (mod 2^64 per component)."""
     m = (1 << 64) - 1
@@ -441,6 +485,7 @@ class Simulation:
         self.sampling = None    # (every, first_step) while field sampling is enabled
         self.host_steps = 0     # timesteps taken by step_host_rng (the index the sampling schedule of that path uses)
         self.surface_on = False  # surface recording enabled (amc_surface_enable)
+        self.vdf = None         # (n_bins, v_max) while the velocity distribution is enabled
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -624,6 +669,7 @@ class Simulation:
     def sample_disable(self):
         self._check(self.lib.amc_sample_disable(self.h), "amc_sample_disable")
         self.sampling = None
+        self.vdf = None         # amc_sample_disable frees the VDF too
 
     def sample_due(self, step):
         if self.sampling is None or self.sampling[0] <= 0:
@@ -658,6 +704,37 @@ class Simulation:
         v = C.c_double(0.0)
         self._check(self.lib.amc_last_sample_ms(self.h, C.byref(v)), "amc_last_sample_ms")
         return float(v.value)
+
+    # ------------------------------------------------------------------ velocity distribution
+    def vdf_enable(self, n_bins, v_max):
+        """Histogram vx, vy, vz over [-v_max, v_max] and the speed over [0, v_max] per z layer of the sampling grid,
+        on the samples of the field sample (amc_vdf_enable; field sampling must be on).  Zeroes the histograms."""
+        self._check(self.lib.amc_vdf_enable(self.h, C.c_int32(int(n_bins)), C.c_double(float(v_max))), "amc_vdf_enable")
+        self.vdf = (int(n_bins), float(v_max))
+
+    def vdf_disable(self):
+        self._check(self.lib.amc_vdf_disable(self.h), "amc_vdf_disable")
+        self.vdf = None
+
+    def vdf_layout(self):
+        """(layers, bins, v_max) of the enabled VDF."""
+        ncz, nb, vm = C.c_int32(0), C.c_int32(0), C.c_double(0.0)
+        self._check(self.lib.amc_vdf_layout(self.h, C.byref(ncz), C.byref(nb), C.byref(vm)), "amc_vdf_layout")
+        return int(ncz.value), int(nb.value), float(vm.value)
+
+    def vdf_raw(self):
+        """acc [layers][VDF_HISTS][n_bins + 2] uint64: [under, bins, over] of vx, vy, vz and the speed per layer."""
+        ncz, nb, _ = self.vdf_layout()
+        acc = np.zeros((ncz, VDF_HISTS, nb + 2), dtype=np.uint64)
+        self._check(self.lib.amc_vdf_get_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64))), "amc_vdf_get_raw")
+        return acc
+
+    def vdf_set_raw(self, acc):
+        ncz, nb, _ = self.vdf_layout()
+        acc = np.ascontiguousarray(acc, dtype=np.uint64)
+        if acc.size != ncz * VDF_HISTS * (nb + 2):
+            raise AmcError("VDF histograms of %d words for a layout of %d layers x %d bins" % (acc.size, ncz, nb))
+        self._check(self.lib.amc_vdf_set_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64))), "amc_vdf_set_raw")
 
     # ------------------------------------------------------------------ surface recording
     def surface_enable(self):
@@ -751,6 +828,8 @@ class Simulation:
             acc, ns, no = self.sample_raw()
             st.update(sample_acc=acc, sample_n=np.uint64(ns), sample_outside=np.uint64(no),
                       sample_schedule=np.array(self.sampling, dtype=np.int64), host_steps=np.int64(self.host_steps))
+        if self.vdf is not None:
+            st.update(vdf_acc=self.vdf_raw(), vdf_bins=np.int64(self.vdf[0]), vdf_vmax=np.float64(self.vdf[1]))
         if self.surface_on:
             acc, ns, out = self.surface_raw()
             st.update(surface_acc=acc, surface_n_steps=np.uint64(ns), surface_outside=out)
@@ -782,6 +861,9 @@ class Simulation:
             self.sample_enable(every, first)
             self.sample_set_raw(ck["sample_acc"], int(ck["sample_n"]), int(ck["sample_outside"]))
             self.host_steps = int(ck["host_steps"])
+        if "vdf_acc" in ck:             # checkpoints written without the VDF have none of these keys
+            self.vdf_enable(int(ck["vdf_bins"]), float(ck["vdf_vmax"]))
+            self.vdf_set_raw(ck["vdf_acc"])
         if "surface_acc" in ck:         # checkpoints written without surface recording have none of these keys
             self.surface_enable()
             self.surface_set_raw(ck["surface_acc"], int(ck["surface_n_steps"]), ck["surface_outside"])

@@ -75,6 +75,12 @@ struct amc_handle {
     std::vector<cudaEvent_t> sample_events; // two per sample of the last call: around k_sample
     int sample_slot = 0;                    // samples recorded into sample_events by the current call
     double last_sample_ms = 0;
+    // velocity distribution (amc_vdf_*): histograms [ncz][AMC_VDF_HISTS][n_bins + 2]; null: disabled
+    unsigned long long *d_vdf = nullptr;
+    double *d_vdf_edges = nullptr; // VdfArgs::edges
+    VdfArgs va = {};               // kernel parameter of k_sample<true> (va.acc = d_vdf)
+    int32_t vdf_ncz = 0;
+    double vdf_vmax = 0;
     // surface recording (amc_surface_*): accumulators [elements][AMC_SURF_WORDS] + outside[AMC_NUM_CASES]; null: off
     unsigned long long *d_surf = nullptr;
     double *d_surf_rsq = nullptr; // annulus bounds, SurfP::rsq
@@ -189,6 +195,8 @@ extern "C" int amc_destroy(amc_handle *h)
     for (cudaEvent_t e : h->sc_events) cudaEventDestroy(e);
     for (cudaEvent_t e : h->sample_events) cudaEventDestroy(e);
     if (h->d_sample) cudaFree(h->d_sample);
+    if (h->d_vdf) cudaFree(h->d_vdf);
+    if (h->d_vdf_edges) cudaFree(h->d_vdf_edges);
     if (h->d_surf) cudaFree(h->d_surf);
     if (h->d_surf_rsq) cudaFree(h->d_surf_rsq);
     if (h->h_stats) cudaFreeHost(h->h_stats);
@@ -615,7 +623,8 @@ static int launch_sample(amc_handle *h, int64_t grid_n, int64_t *launches)
     else { sa.zedge = p.edge[2]; sa.ncz = p.nc[2]; sa.ze0 = p.e0[2]; sa.zinv = p.inv_d[2]; }
     CK(cudaEventRecord(h->sample_events[2 * h->sample_slot], h->stream));
     if (grid_n > 0) {
-        k_sample<<<grid_for(grid_n, SAMPLE_THREADS), SAMPLE_THREADS, 0, h->stream>>>(p, sa);
+        if (h->d_vdf) k_sample<true><<<grid_for(grid_n, SAMPLE_THREADS), SAMPLE_THREADS, 0, h->stream>>>(p, sa, h->va);
+        else k_sample<false><<<grid_for(grid_n, SAMPLE_THREADS), SAMPLE_THREADS, 0, h->stream>>>(p, sa, VdfArgs{});
         if (launches) *launches += 1;
     }
     CK(cudaEventRecord(h->sample_events[2 * h->sample_slot + 1], h->stream));
@@ -667,7 +676,7 @@ extern "C" int amc_sample_disable(amc_handle *h)
     if (h->d_sample) CK(cudaFree(h->d_sample));
     h->d_sample = nullptr;
     h->sample_cells = 0; h->sample_every = 0; h->sample_first = 0; h->n_samples = 0;
-    return AMC_OK;
+    return amc_vdf_disable(h); // the VDF is part of the field sample
 }
 
 extern "C" int amc_sample_now(amc_handle *h)
@@ -710,6 +719,97 @@ extern "C" int amc_last_sample_ms(amc_handle *h, double *ms)
 {
     if (!h || !ms) return AMC_E_INVALID;
     *ms = h->last_sample_ms;
+    return AMC_OK;
+}
+
+// ---- velocity distribution -------------------------------------------------------------------------
+static size_t vdf_words(const amc_handle *h)
+{
+    return (size_t)h->vdf_ncz * AMC_VDF_HISTS * (h->va.n_bins + 2);
+}
+
+// np.linspace(lo, hi, n + 1): lo + k * ((hi - lo) / n), the last edge hi itself.  The volatile keeps the host compiler
+// from fusing the multiply and the add, which NumPy does not.
+static void linspace_edges(double lo, double hi, int n, double *e)
+{
+    const double step = (hi - lo) / n;
+    for (int k = 0; k < n; k++) {
+        volatile double t = (double)k * step;
+        e[k] = t + lo;
+    }
+    e[n] = hi;
+}
+
+extern "C" int amc_vdf_enable(amc_handle *h, int32_t n_bins, double v_max)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_sample) return h->fail(AMC_E_STATE, "the VDF extends the field sample: enable sampling first (amc_sample_enable)");
+    if (n_bins < 1 || n_bins > AMC_VDF_MAX_BINS) return h->fail(AMC_E_INVALID, "n_bins outside [1, AMC_VDF_MAX_BINS]");
+    if (!(std::isfinite(v_max) && v_max > 0)) return h->fail(AMC_E_INVALID, "v_max must be finite and > 0");
+    int rc = amc_vdf_disable(h);
+    if (rc != AMC_OK) return rc;
+    h->vdf_ncz = (int32_t)(h->sample_cells / ((int64_t)h->cfg.nc[0] * h->cfg.nc[1]));
+    h->vdf_vmax = v_max;
+    VdfArgs &va = h->va;
+    va.n_bins = n_bins;
+    va.lo[0] = -v_max; va.hi[0] = v_max;
+    va.lo[1] = 0.0; va.hi[1] = v_max;
+    std::vector<double> edges(2 * (size_t)(n_bins + 1));
+    linspace_edges(va.lo[0], va.hi[0], n_bins, edges.data());
+    linspace_edges(va.lo[1], va.hi[1], n_bins, edges.data() + n_bins + 1);
+    cudaError_t e = cudaMalloc(&h->d_vdf, vdf_words(h) * sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMalloc(&h->d_vdf_edges, edges.size() * sizeof(double));
+    if (e != cudaSuccess) {
+        amc_vdf_disable(h);
+        return h->fail(AMC_E_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    }
+    CK(cudaMemset(h->d_vdf, 0, vdf_words(h) * sizeof(unsigned long long)));
+    CK(cudaMemcpy(h->d_vdf_edges, edges.data(), edges.size() * sizeof(double), cudaMemcpyHostToDevice));
+    va.acc = h->d_vdf;
+    va.edges = h->d_vdf_edges;
+    return AMC_OK;
+}
+
+extern "C" int amc_vdf_disable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    if (h->d_vdf) CK(cudaFree(h->d_vdf));
+    if (h->d_vdf_edges) CK(cudaFree(h->d_vdf_edges));
+    h->d_vdf = nullptr; h->d_vdf_edges = nullptr;
+    h->va = VdfArgs{};
+    h->vdf_ncz = 0; h->vdf_vmax = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_vdf_layout(amc_handle *h, int32_t *ncz, int32_t *n_bins, double *v_max)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_vdf) return h->fail(AMC_E_STATE, "the VDF is not enabled (amc_vdf_enable)");
+    if (ncz) *ncz = h->vdf_ncz;
+    if (n_bins) *n_bins = h->va.n_bins;
+    if (v_max) *v_max = h->vdf_vmax;
+    return AMC_OK;
+}
+
+extern "C" int amc_vdf_get_raw(amc_handle *h, uint64_t *acc)
+{
+    if (!h || !acc) return AMC_E_INVALID;
+    if (!h->d_vdf) return h->fail(AMC_E_STATE, "the VDF is not enabled (amc_vdf_enable)");
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpy(acc, h->d_vdf, vdf_words(h) * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    return AMC_OK;
+}
+
+extern "C" int amc_vdf_set_raw(amc_handle *h, const uint64_t *acc)
+{
+    if (!h || !acc) return AMC_E_INVALID;
+    if (!h->d_vdf) return h->fail(AMC_E_STATE, "the VDF is not enabled (amc_vdf_enable)");
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpy(h->d_vdf, acc, vdf_words(h) * sizeof(uint64_t), cudaMemcpyHostToDevice));
     return AMC_OK;
 }
 

@@ -2509,7 +2509,49 @@ __device__ __forceinline__ void sample_limbs(const double v, const double s1, co
     const double rem = v - (double)i1 * s1inv;
     i2 = __double2ll_rn(rem * s2);
 }
-__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample(const __grid_constant__ P p, const SampleArgs sa)
+
+// velocity distribution (amc_vdf_*): per z layer of the sampling grid, histograms of vx, vy, vz over [-v_max, v_max]
+// and of the speed over [0, v_max], AMC_VDF_HISTS x (n_bins + 2) words [under, bins, over] (include/amc.h).  A kernel
+// parameter of its own, so that P and every other kernel stay as they are.
+struct VdfArgs {
+    unsigned long long *acc; /* [ncz][AMC_VDF_HISTS][n_bins + 2] */
+    const double *edges;     /* [2][n_bins + 1]: np.linspace of the component range, then of the speed range */
+    double lo[2], hi[2];     /* [0]: components (-v_max, v_max), [1]: speed (0, v_max) */
+    int32_t n_bins;
+};
+// word of x in a histogram of range h: 0 under (x < lo), 1 + the bin of np.histogram(x, n_bins, (lo, hi)) with the edge
+// corrections of hist_add, n_bins + 1 over (x > hi or NaN)
+__device__ __forceinline__ int vdf_word(const VdfArgs &va, const int h, const double x)
+{
+    const double lo = va.lo[h], hi = va.hi[h];
+    const int nb = va.n_bins;
+    if (x < lo) return 0;
+    if (!(x <= hi)) return nb + 1;
+    const double *e = va.edges + h * (nb + 1);
+    long long idx = (long long)(((x - lo) / (hi - lo)) * (double)nb);
+    if (idx == nb) idx--;
+    if (x < e[idx]) idx--;
+    else if (x >= e[idx + 1] && idx != nb - 1) idx++;
+    return (int)idx + 1;
+}
+// one count per histogram of a sampled particle (layer >= 0), straight to global memory.  A per-CTA copy of the
+// histograms in shared memory was slower (DESIGN section 14): at ~18 particles per cell a CTA sees few particles of a
+// layer, so the flush issues about as many atomics as it saves.
+__device__ __forceinline__ void vdf_add(const VdfArgs &va, const int layer, const double v[3])
+{
+    static_assert(AMC_VDF_HISTS == 4, "histograms of vdf_add");
+    const int hw = va.n_bins + 2;
+    unsigned long long *a = va.acc + (size_t)layer * AMC_VDF_HISTS * hw;
+    const double speed = sqrt((v[0] * v[0] + v[1] * v[1]) + v[2] * v[2]);
+    atomicAdd(a + vdf_word(va, 0, v[0]), 1ull);
+    atomicAdd(a + hw + vdf_word(va, 0, v[1]), 1ull);
+    atomicAdd(a + 2 * hw + vdf_word(va, 0, v[2]), 1ull);
+    atomicAdd(a + 3 * hw + vdf_word(va, 1, speed), 1ull);
+}
+
+// VDF: also bin the velocity distribution of the sampled particles (vdf_add), in the same pass over the state
+template <bool VDF>
+__global__ void __launch_bounds__(SAMPLE_THREADS) k_sample(const __grid_constant__ P p, const SampleArgs sa, const __grid_constant__ VdfArgs va)
 {
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned lane = threadIdx.x & 31u;
@@ -2532,6 +2574,7 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample(const __grid_constant
                     sample_limbs(v[a], 0x1p19, 0x1p-19, 0x1p49, w[2 * a], w[2 * a + 1]);
                     sample_limbs(v[a] * v[a], 0x1p6, 0x1p-6, 0x1p36, w[6 + 2 * a], w[6 + 2 * a + 1]);
                 }
+                if constexpr (VDF) vdf_add(va, oz, v);
             }
         }
     }

@@ -11,6 +11,16 @@ import numpy as np
 from . import outputs
 
 
+VDF_VMAX_SIGMAS = 6.0   # default VDF range: this many thermal speeds; P(|v_a - u_a| > 6 sigma) = 2e-9 per component
+
+
+def vdf_default_vmax(cfg):
+    """VDF_VMAX_SIGMAS * sqrt(k_B T / m) at the hottest wall temperature of the config (the ambient temperature where the
+    walls have none of their own)."""
+    t = max(float(getattr(cfg, k)) for k in ("temp_ambient", "t_cold", "t_hot") if hasattr(cfg, k))
+    return VDF_VMAX_SIGMAS * float(np.sqrt(float(cfg.boltzman) * t / float(cfg.argon_mass)))
+
+
 def parse_args(default_steps, description, temp=False, argv=None):
     ap = argparse.ArgumentParser(description=description)
     ap.add_argument("--steps", type=int, default=int(os.environ.get("AMC_STEPS", default_steps)),
@@ -30,9 +40,22 @@ def parse_args(default_steps, description, temp=False, argv=None):
     ap.add_argument("--surface-start", type=int, default=None, metavar="S",
                     help="record wall pressure, shear stress and heat flux per wall element from timestep S to the end "
                          "and write surface.csv (default: off)")
+    ap.add_argument("--vdf-bins", type=int, default=0, metavar="N",
+                    help="with --sample-every: also histogram vx, vy, vz and the speed per z layer on the sampled steps, "
+                         "N bins each, and write vdf_z.csv (default 0: off)")
+    ap.add_argument("--vdf-vmax", type=float, default=None, metavar="V",
+                    help="range of the VDF in m/s: [-V, V] for the components, [0, V] for the speed (default: "
+                         "%g times the thermal speed sqrt(k_B T / m) at the config's hottest wall temperature)" % VDF_VMAX_SIGMAS)
     args = ap.parse_args(argv)
     if args.sample_every < 0 or args.sample_start < 0:
         ap.error("--sample-every and --sample-start must be >= 0")
+    if args.vdf_bins:
+        if args.sample_every <= 0:
+            ap.error("--vdf-bins extends the field sample: it needs --sample-every")
+        if not 1 <= args.vdf_bins <= 4096:
+            ap.error("--vdf-bins must be in [1, 4096]")
+    if args.vdf_vmax is not None and (args.vdf_bins <= 0 or not (np.isfinite(args.vdf_vmax) and args.vdf_vmax > 0)):
+        ap.error("--vdf-vmax needs --vdf-bins and must be finite and > 0")
     if args.surface_start is not None and args.surface_start < 0:
         ap.error("--surface-start must be >= 0")
     return args
@@ -60,15 +83,21 @@ def surface_finish(sim, cfg, args):
 
 
 def sampling_begin(sim, args):
-    """Enable field sampling on `sim` if --sample-every asks for it."""
+    """Enable field sampling on `sim` if --sample-every asks for it, and the VDF if --vdf-bins does."""
     if args.sample_every > 0:
         sim.sample_enable(args.sample_every, args.sample_start)
+        if args.vdf_bins:
+            sim.vdf_enable(args.vdf_bins, args.vdf_vmax or vdf_default_vmax(sim.cfg))
 
 
 def sampling_finish(sim, cfg, args):
-    """Write profile_z.csv (one row per z layer) into --outdir if sampling was on."""
+    """Write profile_z.csv (one row per z layer) and, with --vdf-bins, vdf_z.csv into --outdir if sampling was on."""
     if args.sample_every > 0:
-        outputs.write_axial_profile(os.path.join(args.outdir, "profile_z.csv"), outputs.axial_profile(sim.sample_raw(), cfg))
+        raw = sim.sample_raw()
+        outputs.write_axial_profile(os.path.join(args.outdir, "profile_z.csv"), outputs.axial_profile(raw, cfg))
+        if args.vdf_bins:
+            fields = outputs.vdf_fields(sim.vdf_raw(), sim.vdf_layout(), raw, cfg)
+            outputs.write_vdf_csv(os.path.join(args.outdir, "vdf_z.csv"), fields)
 
 
 def final_report(sim, total_errs, total_cols, start, outdir, show=False, labels=("Simulation mean free path: ",

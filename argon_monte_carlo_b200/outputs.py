@@ -148,6 +148,93 @@ def write_axial_profile(path, profile):
                              for c in PROFILE_COLUMNS) + "\n")
 
 
+# ---------------------------------------------------------------- velocity distribution (amc_vdf_*)
+VDF_NAMES = ("vx", "vy", "vz", "speed")
+VDF_COLUMNS = ("z_lo", "z_hi", "histogram", "bin", "v_lo", "v_hi", "count", "pdf", "maxwellian", "under_fraction",
+               "over_fraction", "l1")
+
+
+def maxwell_component_cdf(v, u, sigma):
+    """CDF of one velocity component of a Maxwellian with drift u and sigma = sqrt(k_B T / m)."""
+    from scipy.special import erf
+    return 0.5 * (1.0 + erf((np.asarray(v, dtype=np.float64) - u) / (sigma * np.sqrt(2.0))))
+
+
+def maxwell_speed_cdf(c, u, sigma):
+    """CDF of the speed |v| of a Maxwellian with drift speed u = |<v>| and sigma = sqrt(k_B T / m):
+    (erf((c-u)/(s sqrt2)) + erf((c+u)/(s sqrt2))) / 2 - s / (u sqrt(2 pi)) (exp(-(c-u)^2/2s^2) - exp(-(c+u)^2/2s^2)),
+    at u = 0 the Maxwell-Boltzmann speed CDF erf(c/(s sqrt2)) - sqrt(2/pi) (c/s) exp(-c^2/2s^2)."""
+    from scipy.special import erf
+    c = np.asarray(c, dtype=np.float64)
+    r2 = sigma * np.sqrt(2.0)
+    if u <= 1e-6 * sigma:
+        return erf(c / r2) - np.sqrt(2.0 / np.pi) * (c / sigma) * np.exp(-c * c / (2 * sigma * sigma))
+    return (0.5 * (erf((c - u) / r2) + erf((c + u) / r2))
+            - sigma / (u * np.sqrt(2 * np.pi)) * (np.exp(-(c - u) ** 2 / (2 * sigma * sigma)) - np.exp(-(c + u) ** 2 / (2 * sigma * sigma))))
+
+
+def vdf_fields(raw, layout, sample_raw, cfg, grid=None):
+    """Per z layer and histogram (vx, vy, vz, speed) of the VDF words raw [ncz][4][n_bins + 2] (Simulation.vdf_raw)
+    with layout (ncz, n_bins, v_max) and the field sample sample_raw = (acc, n_samples, n_outside) taken with it:
+      pdf         the measured pdf over the in-range counts (np.histogram's density=True), [ncz, 4, n_bins]
+      under_fraction, over_fraction   the share of the layer's particles below / above the range, [ncz, 4]
+      maxwellian  the Maxwellian at the layer's sampled drift velocity and temperature (axial_profile), averaged over
+                  each bin: (CDF(v_hi) - CDF(v_lo)) / width; not renormalised to the range, [ncz, 4, n_bins]
+      l1          sum over bins of |pdf - maxwellian| * width, [ncz, 4]
+    with the config's own argon_mass and boltzman.  Layers without a particle give NaN."""
+    from .amc import vdf_edges
+    grid = grid or cfg.grid
+    ncz, nb, vmax = int(layout[0]), int(layout[1]), float(layout[2])
+    words = np.asarray(raw, dtype=np.uint64).reshape(ncz, 4, nb + 2)
+    acc = words.astype(np.float64)
+    prof = axial_profile(sample_raw, cfg, grid)
+    acc_s = np.asarray(sample_raw[0], dtype=np.uint64).reshape(-1, 13)
+    nx, ny = int(grid.nc[0]), int(grid.nc[1])
+    count, sv, _ = decode_sample_sums(acc_s)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        drift = sv.reshape(nx * ny, ncz, 3).sum(axis=0) / count.reshape(nx * ny, ncz).sum(axis=0)[:, None]
+        sigma = np.sqrt(float(cfg.boltzman) * prof["temperature"] / float(cfg.argon_mass))
+    ec, es = vdf_edges(nb, vmax)
+    edges = [ec, ec, ec, es]
+    width = np.stack([np.diff(e) for e in edges])                       # [4, n_bins]
+    bins, total = acc[:, :, 1:-1], acc.sum(axis=2)
+    inside = bins.sum(axis=2)
+    maxw = np.full((ncz, 4, nb), np.nan)
+    for k in range(ncz):
+        if not (np.isfinite(sigma[k]) and sigma[k] > 0):
+            continue
+        for j in range(3):
+            cdf = maxwell_component_cdf(ec, drift[k, j], sigma[k])
+            maxw[k, j] = np.diff(cdf) / width[j]
+        maxw[k, 3] = np.diff(maxwell_speed_cdf(es, float(np.sqrt(np.sum(drift[k] ** 2))), sigma[k])) / width[3]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        pdf = bins / (inside[:, :, None] * width[None])
+        under, over = acc[:, :, 0] / total, acc[:, :, -1] / total
+        l1 = np.sum(np.abs(pdf - maxw) * width[None], axis=2)
+    l1[inside == 0] = np.nan
+    z = np.asarray(grid.edge[2], dtype=np.float64)
+    return {"z_lo": z[:-1], "z_hi": z[1:], "n_bins": nb, "v_max": vmax, "edges": edges, "counts": words[:, :, 1:-1],
+            "particles": total, "temperature": prof["temperature"], "drift": drift, "pdf": pdf, "maxwellian": maxw,
+            "under_fraction": under, "over_fraction": over, "l1": l1}
+
+
+def write_vdf_csv(path, fields):
+    """vdf_z.csv: one row per z layer, histogram (vx, vy, vz, speed) and bin, the VDF_COLUMNS of vdf_fields (velocities in
+    m/s, pdfs in s/m; the per-histogram under / over fractions and l1 repeated on every bin row), floats with 17
+    significant digits."""
+    nb = fields["n_bins"]
+    with open(path, "w") as f:
+        f.write(",".join(VDF_COLUMNS) + "\n")
+        for k in range(len(fields["z_lo"])):
+            for j, name in enumerate(VDF_NAMES):
+                e = fields["edges"][j]
+                tail = "%.17g,%.17g,%.17g" % (fields["under_fraction"][k, j], fields["over_fraction"][k, j], fields["l1"][k, j])
+                for b in range(nb):
+                    f.write("%.17g,%.17g,%s,%d,%.17g,%.17g,%d,%.17g,%.17g,%s\n" % (
+                        fields["z_lo"][k], fields["z_hi"][k], name, b, e[b], e[b + 1], int(fields["counts"][k, j, b]),
+                        fields["pdf"][k, j, b], fields["maxwellian"][k, j, b], tail))
+
+
 # ---------------------------------------------------------------- wall surfaces (amc_surface_*)
 SURFACE_COLUMNS = ("element", "case", "lo1", "hi1", "lo2", "hi2", "area", "hits", "number_flux", "pressure", "shear_1",
                    "shear_2", "heat_flux")

@@ -562,6 +562,28 @@ class SlabSimulation:
     def last_sample_ms(self):
         return [r.sim.last_sample_ms() for r in self.ranks]
 
+    def vdf_enable(self, n_bins, v_max):
+        """Velocity distribution on every local rank (Simulation.vdf_enable; after sample_enable): each rank bins its
+        own particles by the global z layers, so the merged histograms equal those of the single-domain run."""
+        for r in self.ranks:
+            r.sim.vdf_enable(n_bins, v_max)
+
+    def vdf_disable(self):
+        for r in self.ranks:
+            r.sim.vdf_disable()
+
+    def vdf_raw(self, reduce=True):
+        """VDF words summed over the local ranks and, with a distributed transport and reduce=True, over all processes
+        (element-wise uint64 sums)."""
+        acc = None
+        with np.errstate(over="ignore"):
+            for r in self.ranks:
+                a = r.sim.vdf_raw()
+                acc = a if acc is None else acc + a
+        if reduce and not isinstance(self.transport, LocalTransport):
+            acc = self.transport.allreduce_u64(acc)
+        return acc
+
     # ------------------------------------------------------------------ surface recording
     def surface_enable(self):
         """Surface recording on every local rank (Simulation.surface_enable); a hit is recorded by the rank that owns

@@ -263,6 +263,36 @@ int amc_sample_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_samples, uint64
 int amc_sample_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_samples, uint64_t n_outside);
 int amc_last_sample_ms(amc_handle *h, double *ms);
 
+/* Velocity distribution (VDF): an extension of the field sample.  It covers the particles of the field sample (owned,
+ * inside the sampling grid) on the steps of the field sample (the schedule of amc_sample_enable, and amc_sample_now).
+ * One region per z layer k of the sampling grid (a slab handle: the global z edges), the rows of profile_z.csv.  Per
+ * layer AMC_VDF_HISTS histograms, in the order vx, vy, vz, speed: the components over [lo, hi] = [-v_max, v_max], the
+ * speed sqrt((vx*vx + vy*vy) + vz*vz) (fp64, separate roundings, correctly rounded sqrt) over [0, v_max].  Each
+ * histogram has n_bins + 2 uint64 words [under, bin 0 .. bin n_bins-1, over]: x < lo counts in under, x > hi or NaN in
+ * over, and lo <= x <= hi in the bin of np.histogram(x, bins=n_bins, range=(lo, hi)) -- the last bin closed on the
+ * right -- found as in np.histogram against edges = np.linspace(lo, hi, n_bins + 1) computed on the host at enable time:
+ *   i = (int64)(((x - lo) / (hi - lo)) * n_bins);  i == n_bins: i - 1;  then x < edges[i]: i - 1, else
+ *   x >= edges[i+1] and i != n_bins - 1: i + 1
+ * Every histogram of a layer, under and over included, therefore sums to the particle counts (word 0) of the field
+ * sample's cells of that layer.  Layout [ncz][AMC_VDF_HISTS][n_bins + 2]; all counts are integer adds, so the words do
+ * not depend on thread order or on the split over ranks, and merging ranks is an element-wise sum (mod 2^64).  The
+ * number of samples is the one amc_sample_get_raw reports; amc_last_sample_ms covers the VDF too.  The VDF changes no
+ * state, counter, histogram, digest or field-sampling word; while it is disabled (the default) nothing is added.
+ * Memory: ncz * AMC_VDF_HISTS * (n_bins + 2) * 8 bytes.
+ *   amc_vdf_enable   allocate and zero the histograms; AMC_E_STATE without field sampling, AMC_E_INVALID for n_bins
+ *                    outside [1, AMC_VDF_MAX_BINS] or v_max not finite and > 0; re-enabling starts from zero
+ *   amc_vdf_disable  free them (amc_sample_disable does too)
+ *   amc_vdf_layout   layers, bins and v_max of the enabled VDF
+ *   amc_vdf_get_raw  acc: [ncz][AMC_VDF_HISTS][n_bins + 2]
+ *   amc_vdf_set_raw  resume from amc_vdf_get_raw's words (the VDF must be enabled with the same layout) */
+#define AMC_VDF_HISTS 4
+#define AMC_VDF_MAX_BINS 4096
+int amc_vdf_enable(amc_handle *h, int32_t n_bins, double v_max);
+int amc_vdf_disable(amc_handle *h);
+int amc_vdf_layout(amc_handle *h, int32_t *ncz, int32_t *n_bins, double *v_max);
+int amc_vdf_get_raw(amc_handle *h, uint64_t *acc);
+int amc_vdf_set_raw(amc_handle *h, const uint64_t *acc);
+
 /* Surface recording: what the gas does to the walls, per wall element, accumulated on the device as every wall
  * interaction happens.  The walls are the AMC_CASE_* slots of the handle's kind (Pore 9, Temp 10, Cube 6; a case the
  * kind does not have has no element), each cut into bins on the handle's sampling grid (that of amc_sample_*; a slab
