@@ -93,7 +93,8 @@ EXPORTS = ("amc_create", "amc_destroy", "amc_last_error", "amc_abi_version", "am
            "amc_slab_p2p_setup", "amc_slab_p2p_connect", "amc_slab_step", "amc_wall_operator", "amc_seed_relax", "amc_last_scatter_ms",
            "amc_sample_enable", "amc_sample_disable", "amc_sample_now", "amc_sample_get_raw", "amc_sample_set_raw",
            "amc_last_sample_ms", "amc_surface_enable", "amc_surface_disable", "amc_surface_layout", "amc_surface_get_raw",
-           "amc_surface_set_raw", "amc_vdf_enable", "amc_vdf_disable", "amc_vdf_layout", "amc_vdf_get_raw", "amc_vdf_set_raw")
+           "amc_surface_set_raw", "amc_vdf_enable", "amc_vdf_disable", "amc_vdf_layout", "amc_vdf_get_raw", "amc_vdf_set_raw",
+           "amc_flux_enable", "amc_flux_disable", "amc_flux_now", "amc_flux_layout", "amc_flux_get_raw", "amc_flux_set_raw")
 
 # field sampling (include/amc.h): words per cell and the binary scales of the fixed-point limbs
 SAMPLE_WORDS = 13
@@ -103,6 +104,11 @@ SAMPLE_Q1, SAMPLE_Q2 = 6, 36      # sums of squares: high / low limb
 # velocity distribution (include/amc.h): histograms per z layer (vx, vy, vz, speed) and the largest bin count
 VDF_HISTS = 4
 VDF_MAX_BINS = 4096
+
+# plane flux recording (include/amc.h): words per plane and the binary scales of the fixed-point limbs
+FLUX_WORDS = 10
+FLUX_V1, FLUX_V2 = 16, 46         # velocity sums: high / low limb
+FLUX_Q1, FLUX_Q2 = 2, 32          # sums of v^2: high / low limb
 
 # surface recording (include/amc.h): words per wall element and the binary scales of the fixed-point limbs
 SURF_WORDS = 9
@@ -418,6 +424,41 @@ def vdf_of_arrays(state, grid, n_bins, v_max, ids=None):
     return acc
 
 
+def flux_counts_of(z, edge_z):
+    """Plane count of every position: the number of planes edge_z[k] <= z (NaN: len(edge_z)), as amc_flux_* counts."""
+    return np.searchsorted(np.asarray(edge_z, dtype=np.float64), np.asarray(z, dtype=np.float64), side="right")
+
+
+def flux_of_states(state_prev, state_cur, edge_z):
+    """NumPy restatement of the flux words one record point adds (include/amc.h): acc [planes][FLUX_WORDS] uint64 for
+    the move from state_prev to state_cur (mappings with 'z' and, for state_cur, 'vx', 'vy', 'vz', indexed by particle
+    id), planes edge_z.  Integer sums: the words of consecutive record points add up (mod 2^64) to those of the run."""
+    c0, c1 = flux_counts_of(state_prev["z"], edge_z), flux_counts_of(state_cur["z"], edge_z)
+    acc = np.zeros((len(edge_z), FLUX_WORDS), dtype=np.uint64)
+    moved = np.flatnonzero(c0 != c1)
+    if len(moved) == 0:
+        return acc
+    a, b = c0[moved], c1[moved]
+    lo, n_planes = np.minimum(a, b), np.abs(b - a)
+    sign = np.where(b > a, 1.0, -1.0)
+    vx, vy, vz = (np.asarray(state_cur[k], dtype=np.float64)[moved] for k in ("vx", "vy", "vz"))
+    with np.errstate(over="ignore", invalid="ignore"):
+        q = (vx * vx + vy * vy) + vz * vz
+    words = []
+    for v, s1, s2 in ((vx, FLUX_V1, FLUX_V2), (vy, FLUX_V1, FLUX_V2), (vz, FLUX_V1, FLUX_V2), (q, FLUX_Q1, FLUX_Q2)):
+        words += list(sample_limbs(sign * v, s1, s2))
+    # one row per crossed plane: particle j crosses planes lo[j] .. lo[j] + n_planes[j] - 1
+    j = np.repeat(np.arange(len(moved)), n_planes)
+    plane = lo[j] + (np.arange(len(j)) - np.repeat(np.cumsum(n_planes) - n_planes, n_planes))
+    up = b[j] > a[j]
+    acc[:, 0] = np.bincount(plane[up], minlength=len(edge_z)).astype(np.uint64)
+    acc[:, 1] = np.bincount(plane[~up], minlength=len(edge_z)).astype(np.uint64)
+    with np.errstate(over="ignore"):
+        for k, w in enumerate(words):
+            np.add.at(acc[:, 2 + k], plane, w.view(np.uint64)[j])
+    return acc
+
+
 def combine_digests(parts):
     """Sum of per-rank digests (mod 2^64 per component)."""
     m = (1 << 64) - 1
@@ -486,6 +527,7 @@ class Simulation:
         self.host_steps = 0     # timesteps taken by step_host_rng (the index the sampling schedule of that path uses)
         self.surface_on = False  # surface recording enabled (amc_surface_enable)
         self.vdf = None         # (n_bins, v_max) while the velocity distribution is enabled
+        self.flux_on = False    # plane flux recording enabled (amc_flux_enable)
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc, what):
@@ -657,6 +699,8 @@ class Simulation:
         self.host_steps += 1
         if self.sample_due(self.host_steps - 1):
             self.sample_now()
+        if self.flux_on:
+            self.flux_now()
         return st
 
     # ------------------------------------------------------------------ field sampling
@@ -771,6 +815,42 @@ class Simulation:
         self._check(self.lib.amc_surface_set_raw(self.h, acc.ctypes.data_as(u64), C.c_uint64(int(n_steps)), outside.ctypes.data_as(u64)),
                     "amc_surface_set_raw")
 
+    # ------------------------------------------------------------------ plane flux recording
+    def flux_enable(self):
+        """Count the particles crossing the z planes of the sampling grid, and what they carry, at every timestep of
+        step() and at every flux_now() (amc_flux_enable); zeroes the words and takes the snapshot of the current state."""
+        self._check(self.lib.amc_flux_enable(self.h), "amc_flux_enable")
+        self.flux_on = True
+
+    def flux_disable(self):
+        self._check(self.lib.amc_flux_disable(self.h), "amc_flux_disable")
+        self.flux_on = False
+
+    def flux_now(self):
+        """One record point: the crossings since the previous one (step_host_rng calls it after its timestep)."""
+        self._check(self.lib.amc_flux_now(self.h), "amc_flux_now")
+
+    def flux_layout(self):
+        """Number of planes (z edges of the sampling grid)."""
+        n = C.c_int32(0)
+        self._check(self.lib.amc_flux_layout(self.h, C.byref(n)), "amc_flux_layout")
+        return int(n.value)
+
+    def flux_raw(self):
+        """(acc [planes][FLUX_WORDS] uint64, record points taken)."""
+        acc = np.zeros((self.flux_layout(), FLUX_WORDS), dtype=np.uint64)
+        ns = C.c_uint64(0)
+        self._check(self.lib.amc_flux_get_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(ns)), "amc_flux_get_raw")
+        return acc, int(ns.value)
+
+    def flux_set_raw(self, acc, n_steps):
+        acc = np.ascontiguousarray(acc, dtype=np.uint64)
+        n = self.flux_layout()
+        if acc.size != n * FLUX_WORDS:
+            raise AmcError("flux words of %d words for a layout of %d planes" % (acc.size, n))
+        self._check(self.lib.amc_flux_set_raw(self.h, acc.ctypes.data_as(C.POINTER(C.c_uint64)), C.c_uint64(int(n_steps))),
+                    "amc_flux_set_raw")
+
     # ------------------------------------------------------------------ outputs
     def histograms(self):
         """(counts[4, 200] uint64 in the order total/x/y/z, number of completed paths, sums[4])."""
@@ -833,6 +913,9 @@ class Simulation:
         if self.surface_on:
             acc, ns, out = self.surface_raw()
             st.update(surface_acc=acc, surface_n_steps=np.uint64(ns), surface_outside=out)
+        if self.flux_on:
+            acc, ns = self.flux_raw()
+            st.update(flux_acc=acc, flux_n_steps=np.uint64(ns))
         if path is not None:
             np.savez(path, **st)
         return st
@@ -867,6 +950,9 @@ class Simulation:
         if "surface_acc" in ck:         # checkpoints written without surface recording have none of these keys
             self.surface_enable()
             self.surface_set_raw(ck["surface_acc"], int(ck["surface_n_steps"]), ck["surface_outside"])
+        if "flux_acc" in ck:            # checkpoints written without flux recording have none of these keys
+            self.flux_enable()          # the snapshot of the restored state: the one the checkpointed handle held
+            self.flux_set_raw(ck["flux_acc"], int(ck["flux_n_steps"]))
 
     def state_digest(self):
         """(sum0, sum1, count): order-independent checksum of the owned particle state, computed on the device

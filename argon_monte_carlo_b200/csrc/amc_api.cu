@@ -87,6 +87,11 @@ struct amc_handle {
     SurfP sp = {};                // kernel parameter of the recording kernels (sp.acc = d_surf)
     uint64_t surf_steps = 0;      // wall phases recorded
     double surf_dr = 0;           // x cell width of the grid: (edge[0][nc] - edge[0][0]) / nc
+    // plane flux recording (amc_flux_*): accumulators [ncz + 1][AMC_FLUX_WORDS] + FluxArgs::bad, the snapshot [cap];
+    // null: off
+    unsigned long long *d_flux = nullptr;
+    int32_t *d_flux_snap = nullptr;
+    uint64_t flux_steps = 0;      // record points taken
     std::string error;
 
     int fail(int code, const std::string &msg)
@@ -199,6 +204,8 @@ extern "C" int amc_destroy(amc_handle *h)
     if (h->d_vdf_edges) cudaFree(h->d_vdf_edges);
     if (h->d_surf) cudaFree(h->d_surf);
     if (h->d_surf_rsq) cudaFree(h->d_surf_rsq);
+    if (h->d_flux) cudaFree(h->d_flux);
+    if (h->d_flux_snap) cudaFree(h->d_flux_snap);
     if (h->h_stats) cudaFreeHost(h->h_stats);
     if (h->aux) { cudaStreamSynchronize(h->aux); cudaStreamDestroy(h->aux); }
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -405,6 +412,8 @@ extern "C" int amc_create(const amc_config *cfg, int device, amc_handle **out)
     return AMC_OK;
 }
 
+static int flux_retake(amc_handle *h);
+
 static int ensure_prior(amc_handle *h)
 {
     if (h->have_prior) return AMC_OK;
@@ -437,7 +446,7 @@ extern "C" int amc_set_state(amc_handle *h, int64_t n, const double *x, const do
     if (n) k_pack_pos<<<grid_for(n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(h->p, 0); // slot == particle index
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(h->stream));
-    return AMC_OK;
+    return flux_retake(h);
 }
 
 extern "C" int amc_init_synthetic(amc_handle *h, const amc_init_spec *spec, int64_t *n_kept)
@@ -465,7 +474,7 @@ extern "C" int amc_init_synthetic(amc_handle *h, const amc_init_spec *spec, int6
     h->init_spec = *spec;
     h->have_init_spec = keep_all;
     if (n_kept) *n_kept = n;
-    return AMC_OK;
+    return flux_retake(h);
 }
 
 // bring the state back to original index order (slot == id); b arrays are scratch between phases
@@ -921,6 +930,132 @@ extern "C" int amc_surface_set_raw(amc_handle *h, const uint64_t *acc, uint64_t 
     return AMC_OK;
 }
 
+// ---- plane flux recording ------------------------------------------------------------------------
+static size_t flux_words(const amc_handle *h)
+{
+    return (size_t)(h->cfg.nc[2] + 1) * AMC_FLUX_WORDS;
+}
+
+static FluxArgs flux_args(const amc_handle *h)
+{
+    return FluxArgs{h->d_flux, h->d_flux_snap, h->d_flux + flux_words(h)};
+}
+
+// one record point on h->stream; launches (nullable) counts the kernel launch
+static int launch_flux(amc_handle *h, int64_t *launches)
+{
+    if (h->n) {
+        k_flux<<<grid_for(h->n, FLUX_THREADS), FLUX_THREADS, 0, h->stream>>>(h->p, flux_args(h));
+        if (launches) *launches += 1;
+    }
+    CK(cudaGetLastError());
+    h->flux_steps++;
+    return AMC_OK;
+}
+
+// the snapshot of the current state; AMC_E_INVALID unless the ids are 0 .. n-1 (the snapshot is indexed by id)
+static int flux_snapshot(amc_handle *h)
+{
+    const FluxArgs fa = flux_args(h);
+    CK(cudaMemsetAsync(fa.bad, 0, sizeof(unsigned long long), h->stream));
+    CK(cudaMemsetAsync(fa.snap, 0xff, h->n * sizeof(int32_t), h->stream));
+    if (h->n) k_flux_snap<<<grid_for(h->n, FLUX_THREADS), FLUX_THREADS, 0, h->stream>>>(h->p, fa);
+    CK(cudaGetLastError());
+    unsigned long long bad = 0;
+    CK(cudaMemcpyAsync(&bad, fa.bad, sizeof(bad), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (bad) return h->fail(AMC_E_INVALID, "flux recording indexes its snapshot by particle id: the ids must be 0 .. n-1");
+    return AMC_OK;
+}
+
+// after a call that replaced the state: a new snapshot while recording is on.  A state the snapshot cannot index
+// ends the recording, so that no later record point reads outside it.
+static int flux_retake(amc_handle *h)
+{
+    if (!h->d_flux) return AMC_OK;
+    const int rc = flux_snapshot(h);
+    if (rc != AMC_OK) {
+        const std::string msg = h->error;
+        amc_flux_disable(h);
+        h->error = msg + " (flux recording disabled)";
+    }
+    return rc;
+}
+
+extern "C" int amc_flux_enable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    if (h->slab) return h->fail(AMC_E_STATE, "flux recording needs a single-domain handle (a migrant between slab ranks would have to carry its plane count)");
+    int rc = amc_flux_disable(h);
+    if (rc != AMC_OK) return rc;
+    cudaError_t e = cudaMalloc(&h->d_flux, (flux_words(h) + 1) * sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMalloc(&h->d_flux_snap, (size_t)h->cap * sizeof(int32_t));
+    if (e != cudaSuccess) {
+        amc_flux_disable(h);
+        return h->fail(AMC_E_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    }
+    CK(cudaMemsetAsync(h->d_flux, 0, flux_words(h) * sizeof(unsigned long long), h->stream));
+    if ((rc = flux_snapshot(h)) != AMC_OK) {
+        const std::string msg = h->error;
+        amc_flux_disable(h);
+        h->error = msg;
+    }
+    return rc;
+}
+
+extern "C" int amc_flux_disable(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->stream));
+    if (h->d_flux) CK(cudaFree(h->d_flux));
+    if (h->d_flux_snap) CK(cudaFree(h->d_flux_snap));
+    h->d_flux = nullptr; h->d_flux_snap = nullptr;
+    h->flux_steps = 0;
+    return AMC_OK;
+}
+
+extern "C" int amc_flux_now(amc_handle *h)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_flux) return h->fail(AMC_E_STATE, "flux recording is not enabled (amc_flux_enable)");
+    CK(cudaSetDevice(h->device));
+    int rc = launch_flux(h, nullptr);
+    if (rc != AMC_OK) return rc;
+    CK(cudaStreamSynchronize(h->stream));
+    return AMC_OK;
+}
+
+extern "C" int amc_flux_layout(amc_handle *h, int32_t *n_planes)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_flux) return h->fail(AMC_E_STATE, "flux recording is not enabled (amc_flux_enable)");
+    if (n_planes) *n_planes = h->cfg.nc[2] + 1;
+    return AMC_OK;
+}
+
+extern "C" int amc_flux_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_steps)
+{
+    if (!h) return AMC_E_INVALID;
+    if (!h->d_flux) return h->fail(AMC_E_STATE, "flux recording is not enabled (amc_flux_enable)");
+    CK(cudaSetDevice(h->device));
+    if (acc) CK(cudaMemcpyAsync(acc, h->d_flux, flux_words(h) * sizeof(uint64_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    if (n_steps) *n_steps = h->flux_steps;
+    return AMC_OK;
+}
+
+extern "C" int amc_flux_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_steps)
+{
+    if (!h || !acc) return AMC_E_INVALID;
+    if (!h->d_flux) return h->fail(AMC_E_STATE, "flux recording is not enabled (amc_flux_enable)");
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(h->d_flux, acc, flux_words(h) * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->flux_steps = n_steps;
+    return AMC_OK;
+}
+
 extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
 {
     if (!h) return AMC_E_INVALID;
@@ -937,6 +1072,7 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
     h->last_scatter_ms = 0;
     h->last_launches = 0;
     sample_reset_timing(h);
+    const bool flux = h->d_flux != nullptr; // every step is a record point
     int done = 0;
     if (sweep && h->n) { // the sweep kernel addresses particles by id: keep slot == id
         int rc = unsort(h);
@@ -955,7 +1091,8 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
             p.stats = h->d_stats + s;
             p.step = h->step_index++;
             if (h->sp.acc) h->surf_steps++;
-            // a sampled step is closed like the last step of a chunk, so the sample sees the state at its end
+            // a sampled or recorded step is closed like the last step of a chunk, so the sample and the flux
+            // recording see the state at its end
             const bool sample = sample_due(h, p.step);
             if (h->n > 0) {
                 // the recapture that closes step s-1's pair pass rides along in step s's advect kernel
@@ -996,15 +1133,19 @@ extern "C" int amc_step(amc_handle *h, int32_t n_steps, amc_step_stats *stats)
                 h->det_slot = -1;
                 if (rc != AMC_OK) return rc;
                 CK(cudaEventRecord(h->events[4 * s + 3], h->stream));
-                closed_prev = s == chunk - 1 || sample;
-                if (has_recap && closed_prev) { // last step of the call (or a sampled step): close it now
+                closed_prev = s == chunk - 1 || sample || flux;
+                if (has_recap && closed_prev) { // last step of the call (or a sampled / recorded step): close it now
                     if (sweep) k_recapture_post<<<grid_for(h->n, ADVECT_THREADS), ADVECT_THREADS, 0, h->stream>>>(p);
                     else k_recapture_list<<<148, ADVECT_THREADS, 0, h->stream>>>(p);
                     h->last_launches += 1;
                 }
                 if (sample && (rc = launch_sample(h, h->n, &h->last_launches)) != AMC_OK) return rc;
+                if (flux && (rc = launch_flux(h, &h->last_launches)) != AMC_OK) return rc;
                 CK(cudaEventRecord(h->events[4 * s + 4], h->stream));
-            } else if (sample && (rc = launch_sample(h, 0, nullptr)) != AMC_OK) return rc;
+            } else {
+                if (sample && (rc = launch_sample(h, 0, nullptr)) != AMC_OK) return rc;
+                if (flux && (rc = launch_flux(h, nullptr)) != AMC_OK) return rc;
+            }
         }
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(h->h_stats, h->d_stats, chunk * sizeof(StatsDev), cudaMemcpyDeviceToHost, h->stream));
@@ -1152,7 +1293,7 @@ extern "C" int amc_seed_relax(amc_handle *h, int32_t max_rounds, int64_t *n_redr
     // worklists built by the seed-mode passes are reset by the next pair pass (prepare_pairs)
     if (n_redrawn) *n_redrawn = total;
     if (n_left) *n_left = left;
-    return AMC_OK;
+    return flux_retake(h);
 }
 
 extern "C" int amc_wall_operator(amc_handle *h, int32_t op, const uint8_t *mask, double param, int64_t *n_hits, int64_t *errors)
@@ -1409,6 +1550,7 @@ extern "C" int amc_set_stream(amc_handle *h, void *cuda_stream)
 extern "C" int amc_set_ids(amc_handle *h, const int64_t *ids)
 {
     if (!h || !ids) return AMC_E_INVALID;
+    if (h->d_flux) return h->fail(AMC_E_STATE, "flux recording indexes its snapshot by particle id: disable it before amc_set_ids");
     CK(cudaSetDevice(h->device));
     std::vector<int32_t> v((size_t)h->n);
     for (int64_t i = 0; i < h->n; i++) {
@@ -1432,6 +1574,7 @@ extern "C" int amc_slab_enable(amc_handle *h, const amc_slab_config *c)
     if (h->p.wall_bits) return h->fail(AMC_E_INVALID, "AMC_TAP_WALL_BITS is indexed by particle id (global on a slab handle): not available with slabs");
     if (h->d_sample) return h->fail(AMC_E_STATE, "enable sampling after amc_slab_enable (a slab handle samples the global grid)");
     if (h->d_surf) return h->fail(AMC_E_STATE, "enable surface recording after amc_slab_enable (a slab handle bins on the global grid)");
+    if (h->d_flux) return h->fail(AMC_E_STATE, "flux recording needs a single-domain handle: disable it first (amc_flux_disable)");
     CK(cudaSetDevice(h->device));
     P &p = h->p;
     p.slab = 1; p.srank = c->rank; p.nranks = c->nranks; p.zoff = c->cuts[c->rank]; p.gncz = c->gncz;

@@ -14,6 +14,7 @@
 //   k_case_*          per-case wall kernels for the host-RNG parity mode
 //   k_init_synthetic  synthetic Maxwellian initial state
 //   k_xfer_*, k_bnd_* slab decomposition: migration / ghost copies, per-group hand-over
+//   k_flux            plane flux recording: net crossings of the z planes since the last record point
 #pragma once
 #include "amc_device.cuh"
 
@@ -2615,5 +2616,65 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) k_sample(const __grid_constant
             }
         }
         __syncwarp();
+    }
+}
+
+// ---------------------------------------------------------------- plane flux recording (amc_flux_*)
+// Net crossings of the z planes of the sampling grid between consecutive record points (include/amc.h).  One thread
+// per slot: the 32-byte record gives z and the id, and the plane count of z is compared with the snapshot snap[id].
+// Only a particle that crossed a plane -- a fraction of a percent per step at the pore's timestep -- loads its
+// velocity and adds its words with 64-bit atomics: a few hundred thousand atomics per step at 12.5 M particles,
+// spread over the planes, so a warp-level reduction of them would not pay for itself.  A kernel parameter of its own,
+// so that P and every other kernel stay as they are.
+#define FLUX_THREADS 256
+struct FluxArgs {
+    unsigned long long *acc; /* [ncz + 1][AMC_FLUX_WORDS] */
+    int32_t *snap;           /* [max_particles] plane count of every particle id at the last record point */
+    unsigned long long *bad; /* [1] k_flux_snap: ids outside 0 .. n-1 or met twice */
+};
+// cnt(z): the number of planes edge[k] <= z, k = 0 .. nc (np.searchsorted(edge, z, side='right'); NaN: nc + 1).  The
+// guess from the uniform spacing is corrected against the uploaded edges, so the answer is NumPy's for every z.
+__device__ __forceinline__ int flux_count(const double *edge, const int nc, const double e0, const double inv_d, const double z)
+{
+    if (z != z) return nc + 1;
+    const double t = (z - e0) * inv_d;
+    int c = !(t >= 0.0) ? 0 : (t >= (double)nc ? nc + 1 : (int)t + 1);
+    while (c > 0 && z < edge[c - 1]) c--;
+    while (c <= nc && edge[c] <= z) c++;
+    return c;
+}
+// the snapshot of the current state (snap[0 .. n-1] preset to -1): every id must be met once, in 0 .. n-1
+__global__ void __launch_bounds__(FLUX_THREADS) k_flux_snap(const __grid_constant__ P p, const FluxArgs fa)
+{
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= p.n) return;
+    const PosRec r = p.a.pos[s];
+    if ((uint32_t)r.id >= (uint32_t)p.n) { atomicAdd(fa.bad, 1ull); return; }
+    const int c = flux_count(p.edge[2], p.nc[2], p.e0[2], p.inv_d[2], r.z);
+    if (atomicExch(fa.snap + r.id, c) != -1) atomicAdd(fa.bad, 1ull);
+}
+// one record point: 32 bytes of record + a 4-byte snapshot read per particle; a crossing adds one full contribution
+// to every plane it passed and writes the snapshot back
+__global__ void __launch_bounds__(FLUX_THREADS) k_flux(const __grid_constant__ P p, const FluxArgs fa)
+{
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= p.n) return;
+    const PosRec r = p.a.pos[s];
+    const int c1 = flux_count(p.edge[2], p.nc[2], p.e0[2], p.inv_d[2], r.z);
+    const int c0 = fa.snap[r.id];
+    if (c1 == c0) return;
+    fa.snap[r.id] = c1;
+    const double v[3] = {p.a.vx[s], p.a.vy[s], p.a.vz[s]};
+    const double sg = c1 > c0 ? 1.0 : -1.0;
+    static_assert(AMC_FLUX_WORDS == 10 && AMC_FLUX_V1 == 16 && AMC_FLUX_V2 == 46 && AMC_FLUX_Q1 == 2 && AMC_FLUX_Q2 == 32, "words of k_flux");
+    long long w[8];
+#pragma unroll
+    for (int a = 0; a < 3; a++) sample_limbs(sg * v[a], 0x1p16, 0x1p-16, 0x1p46, w[2 * a], w[2 * a + 1]);
+    sample_limbs(sg * ((v[0] * v[0] + v[1] * v[1]) + v[2] * v[2]), 0x1p2, 0x1p-2, 0x1p32, w[6], w[7]);
+    for (int k = min(c0, c1); k < max(c0, c1); k++) {
+        unsigned long long *a = fa.acc + (size_t)k * AMC_FLUX_WORDS;
+        atomicAdd(a + (c1 > c0 ? 0 : 1), 1ull);
+#pragma unroll
+        for (int j = 0; j < 8; j++) if (w[j]) atomicAdd(a + 2 + j, (unsigned long long)w[j]);
     }
 }

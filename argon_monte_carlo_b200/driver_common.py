@@ -40,6 +40,9 @@ def parse_args(default_steps, description, temp=False, argv=None):
     ap.add_argument("--surface-start", type=int, default=None, metavar="S",
                     help="record wall pressure, shear stress and heat flux per wall element from timestep S to the end "
                          "and write surface.csv (default: off)")
+    ap.add_argument("--flux-start", type=int, default=None, metavar="S",
+                    help="count the particles crossing every z plane of the sampling grid, with their momentum and "
+                         "energy, from timestep S to the end and write flux_z.csv (default: off)")
     ap.add_argument("--vdf-bins", type=int, default=0, metavar="N",
                     help="with --sample-every: also histogram vx, vy, vz and the speed per z layer on the sampled steps, "
                          "N bins each, and write vdf_z.csv (default 0: off)")
@@ -58,6 +61,8 @@ def parse_args(default_steps, description, temp=False, argv=None):
         ap.error("--vdf-vmax needs --vdf-bins and must be finite and > 0")
     if args.surface_start is not None and args.surface_start < 0:
         ap.error("--surface-start must be >= 0")
+    if args.flux_start is not None and args.flux_start < 0:
+        ap.error("--flux-start must be >= 0")
     return args
 
 
@@ -80,6 +85,27 @@ def surface_finish(sim, cfg, args):
         sim.surface_enable()
     grid = getattr(sim, "sample_grid", cfg.grid)
     outputs.write_surface_csv(os.path.join(args.outdir, "surface.csv"), outputs.surface_fields(sim.surface_raw(), cfg, grid, sim.kind))
+
+
+def flux_chunk(sim, args, done, chunk):
+    """The number of timesteps to take from timestep `done` on, at most `chunk`: a batch never straddles
+    --flux-start, and recording starts when the run reaches it."""
+    s = args.flux_start
+    if s is None:
+        return chunk
+    if done >= s and not sim.flux_on:
+        sim.flux_enable()
+    return s - done if done < s < done + chunk else chunk
+
+
+def flux_finish(sim, cfg, args):
+    """Write flux_z.csv (one row per z plane) into --outdir if --flux-start was given."""
+    if args.flux_start is None:
+        return
+    if not sim.flux_on:         # the run ended before timestep S: nothing recorded
+        sim.flux_enable()
+    grid = getattr(sim, "sample_grid", cfg.grid)
+    outputs.write_flux_csv(os.path.join(args.outdir, "flux_z.csv"), outputs.flux_fields(sim.flux_raw(), cfg, grid, sim.kind))
 
 
 def sampling_begin(sim, args):

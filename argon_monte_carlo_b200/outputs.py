@@ -333,3 +333,74 @@ def write_surface_csv(path, fields):
         f.write(",".join(SURFACE_COLUMNS) + "\n")
         for k in range(len(fields["element"])):
             f.write(",".join(str(int(fields[c][k])) if c in ints else "%.17g" % float(fields[c][k]) for c in SURFACE_COLUMNS) + "\n")
+
+
+# ---------------------------------------------------------------- plane fluxes (amc_flux_*)
+FLUX_COLUMNS = ("plane", "z", "area", "up", "down", "up_rate", "down_rate", "particle_flux", "mass_flux", "p_xz", "p_yz",
+                "p_zz", "energy_flux")
+
+
+def decode_flux_sums(acc):
+    """acc [planes][10] uint64 (Simulation.flux_raw) -> (up [planes], down [planes], sums [planes, 4]: sum s*vx, s*vy,
+    s*vz in m/s and sum s*v^2 in m^2/s^2) as float64, each sum high * 2^-S1 + low * 2^-S2 of its signed limbs
+    (include/amc.h)."""
+    from .amc import FLUX_Q1, FLUX_Q2, FLUX_V1, FLUX_V2, FLUX_WORDS
+    w = np.ascontiguousarray(acc, dtype=np.uint64).reshape(-1, FLUX_WORDS).view(np.int64)
+    dec = lambda j, s1, s2: np.ldexp(w[:, j].astype(np.float64), -s1) + np.ldexp(w[:, j + 1].astype(np.float64), -s2)
+    sums = np.stack([dec(2, FLUX_V1, FLUX_V2), dec(4, FLUX_V1, FLUX_V2), dec(6, FLUX_V1, FLUX_V2), dec(8, FLUX_Q1, FLUX_Q2)], axis=1)
+    u = w.view(np.uint64)
+    return u[:, 0].astype(np.float64), u[:, 1].astype(np.float64), sums
+
+
+def plane_areas(cfg, kind, z):
+    """Cross-section pi R^2 of the pore at each plane z, R the wall radius of the section the plane lies in: R_oa in the
+    open air, R_p in the coated sections, R_g in the gap (the z bounds of the wall masks: the gap ends at z_gt_pore in
+    Pore, at z_gt in Temp); a plane on a section boundary takes the smaller radius, a plane outside [0, H] the open-air
+    one.  Cube (kind 0): cube_x * cube_y."""
+    from .amc import KIND_CUBE, KIND_PORE
+    z = np.asarray(z, dtype=np.float64)
+    if kind == KIND_CUBE:
+        return np.full(z.shape, float(cfg.cube_x) * float(cfg.cube_y))
+    g = cfg.geom
+    z_top = g.z_gt_pore if kind == KIND_PORE else g.z_gt
+    sections = ((0.0, g.oah, g.R_oa), (g.oah, g.z_gb, g.R_p), (g.z_gb, z_top, g.R_g), (z_top, g.z_cold, g.R_p),
+                (g.z_cold, g.H, g.R_oa))
+    r = np.full(z.shape, float(g.R_oa))
+    inside = np.zeros(z.shape, dtype=bool)
+    for lo, hi, R in sections:
+        m = (z >= float(lo)) & (z <= float(hi))
+        r = np.where(m, np.where(inside, np.minimum(r, float(R)), float(R)), r)
+        inside |= m
+    return np.pi * r * r
+
+
+def flux_fields(raw, cfg, grid, kind):
+    """Per plane of raw = (acc, n_steps) (Simulation.flux_raw) on the z edges of `grid` for a handle of `kind`: the
+    FLUX_COLUMNS -- plane index, z, cross-section A (plane_areas), crossings up / down and their rates per second,
+    the net particle flux (up - down) / (A n_steps dt) (1 / (m^2 s)) and mass flux m times it (kg / (m^2 s)), the
+    momentum fluxes m sum(s v_a) / (A n_steps dt) for a = x, y, z (P_xz, P_yz, P_zz in Pa) and the energy flux
+    m/2 sum(s v^2) / (A n_steps dt) (W / m^2), with the config's own argon_mass and dt.  No record point: NaN rates."""
+    acc, n_steps = raw
+    z = np.asarray(grid.edge[2], dtype=np.float64)
+    area = plane_areas(cfg, kind, z)
+    up, down, sums = decode_flux_sums(acc)
+    m, t = float(cfg.argon_mass), float(n_steps) * float(cfg.dt)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        tt = t if t > 0 else np.nan
+        net = (up - down) / (area * tt)
+        words = np.asarray(acc, dtype=np.uint64).reshape(len(z), -1)
+        return {"plane": np.arange(len(z)), "z": z, "area": area, "up": words[:, 0], "down": words[:, 1],
+                "up_rate": up / tt, "down_rate": down / tt, "particle_flux": net, "mass_flux": m * net,
+                "p_xz": m * sums[:, 0] / (area * tt), "p_yz": m * sums[:, 1] / (area * tt), "p_zz": m * sums[:, 2] / (area * tt),
+                "energy_flux": 0.5 * m * sums[:, 3] / (area * tt), "n_steps": int(n_steps)}
+
+
+def write_flux_csv(path, fields):
+    """flux_z.csv: one row per z plane, the FLUX_COLUMNS (z in m, area in m^2, rates in 1 / s, particle flux in
+    1 / (m^2 s), mass flux in kg / (m^2 s), momentum fluxes in Pa, energy flux in W / m^2), floats with 17 significant
+    digits."""
+    ints = ("plane", "up", "down")
+    with open(path, "w") as f:
+        f.write(",".join(FLUX_COLUMNS) + "\n")
+        for k in range(len(fields["plane"])):
+            f.write(",".join(str(int(fields[c][k])) if c in ints else "%.17g" % float(fields[c][k]) for c in FLUX_COLUMNS) + "\n")

@@ -23,7 +23,7 @@ if __name__ == "__main__":
     driver_common.sampling_begin(sim, args)
     done = 0
     while done < args.steps:
-        chunk = driver_common.surface_chunk(sim, args, done, min(args.chunk, args.steps - done))
+        chunk = driver_common.flux_chunk(sim, args, done, driver_common.surface_chunk(sim, args, done, min(args.chunk, args.steps - done)))
         for k, s in enumerate(sim.step(chunk)):
             print('  timestep', done + k, 'of', cfg.num_timesteps, '  (sim', 1, '/', 1, ')')
             print('    ', s["pp_collisions"], ' collisions')
@@ -36,5 +36,6 @@ if __name__ == "__main__":
     outputs.write_histograms(counts, args.outdir)
     driver_common.sampling_finish(sim, cfg, args)
     driver_common.surface_finish(sim, cfg, args)
+    driver_common.flux_finish(sim, cfg, args)
     sim.close()
     driver_common.maybe_show(args.show)

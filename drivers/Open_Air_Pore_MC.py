@@ -30,7 +30,7 @@ if __name__ == "__main__":
     total_cols = total_errs = 0
     done = 0
     while done < args.steps:
-        chunk = driver_common.surface_chunk(sim, args, done, min(args.chunk, args.steps - done))
+        chunk = driver_common.flux_chunk(sim, args, done, driver_common.surface_chunk(sim, args, done, min(args.chunk, args.steps - done)))
         stats = sim.step(chunk)
         ms, _ = sim.last_timing()
         for k, s in enumerate(stats):
@@ -47,6 +47,7 @@ if __name__ == "__main__":
     driver_common.final_report(sim, total_errs, total_cols, start, args.outdir)
     driver_common.sampling_finish(sim, cfg, args)
     driver_common.surface_finish(sim, cfg, args)
+    driver_common.flux_finish(sim, cfg, args)
     print('Runtime: ' + str((time() - start) / 60.0) + ' minutes')
     sim.close()
     driver_common.maybe_show(args.show)

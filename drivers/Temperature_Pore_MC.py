@@ -46,7 +46,7 @@ if __name__ == "__main__":
     total_cols = total_errs = 0
     done = 0
     while done < args.steps:
-        chunk = driver_common.surface_chunk(sim, args, done, 1 if host else min(args.chunk, args.steps - done))
+        chunk = driver_common.flux_chunk(sim, args, done, driver_common.surface_chunk(sim, args, done, 1 if host else min(args.chunk, args.steps - done)))
         t0 = time()
         stats = [sim.step_host_rng()] if host else sim.step(chunk)
         wall_dt = (time() - t0) / chunk
@@ -69,6 +69,7 @@ if __name__ == "__main__":
     driver_common.final_report(sim, total_errs, total_cols, start, args.outdir)
     driver_common.sampling_finish(sim, cfg, args)
     driver_common.surface_finish(sim, cfg, args)
+    driver_common.flux_finish(sim, cfg, args)
     outputs.write_momentum_energy_csv(momentum, e_cold, e_hot, os.path.join(args.outdir, "momentum_energy.csv"))
     import mpmath
     for series in (momentum, e_cold, e_hot):

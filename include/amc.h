@@ -348,6 +348,51 @@ int amc_surface_layout(amc_handle *h, int64_t offsets[AMC_NUM_CASES + 1]);
 int amc_surface_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_steps, uint64_t outside[AMC_NUM_CASES]);
 int amc_surface_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_steps, const uint64_t outside[AMC_NUM_CASES]);
 
+/* Plane flux recording: particles and what they carry through the z planes of the sampling grid, counted on the
+ * device.  Planes: the ncz + 1 z edges edge_z[0..ncz] of the handle's sampling grid (that of amc_sample_*), the
+ * boundaries of the rows of profile_z.csv.  The plane count of a position is cnt(z) = the number of planes with
+ * edge_z[k] <= z (np.searchsorted(edge_z, z, side='right'); NaN counts ncz + 1, as in NumPy).  At every record point
+ * each particle's cnt(z) (c1) is compared with the one stored at the previous record point (c0, a per-particle int32
+ * snapshot indexed by particle id): c1 > c0 crossed planes c0 .. c1-1 upward (s = +1), c1 < c0 crossed planes
+ * c1 .. c0-1 downward (s = -1); every crossed plane gets one full contribution, then the snapshot becomes c1.  The
+ * carried quantities use the particle's velocity in the current state (the end of the step).  Per plane
+ * AMC_FLUX_WORDS uint64 words:
+ *   [0] upward crossings;  [1] downward crossings;  [2..3] sum s*vx;  [4..5] sum s*vy;  [6..7] sum s*vz;
+ *   [8..9] sum s*((vx*vx + vy*vy) + vz*vz) (fp64, separate roundings)
+ * every sum as two signed 64-bit fixed-point limbs, the scheme of amc_sample_*: S1 / S2 = AMC_FLUX_V1 / _V2 for the
+ * velocities, AMC_FLUX_Q1 / _Q2 for the squares.  Headroom: 10^10 crossings per plane at speeds <= 10^4 m/s keep every
+ * limb inside the signed 64-bit range (worst case: 6.6e18 in a velocity high limb, 4.0e18 in a square high limb,
+ * 5.4e18 in a low limb).  Rates are sums / (n_steps * dt), n_steps = record points.
+ * The words count net crossings between consecutive record points: a particle that crosses and comes back in between
+ * counts nothing, and everything that moves a particle counts -- drift, wall reflections, collision moves, and the
+ * recapture's z teleports (at most 10*a in Pore, to 50 nm from an end in Temp: only planes that close to z = 0 or
+ * z = H see those).  The words are a function of the sequence of states at the record points alone.
+ * Record points: the end of every timestep of amc_step, and every amc_flux_now.  amc_set_state, amc_init_synthetic
+ * and amc_seed_relax re-take the snapshot from the state they leave; the other phase-level calls do not (their moves
+ * are recorded at the next record point).  Single-domain handles only: a migrant between slab ranks would have to
+ * carry its plane count.  Recording changes no state, counter, histogram, digest or sample / VDF / surface word;
+ * while it is disabled (the default) no launch and no memory is added.  Memory: 8 * AMC_FLUX_WORDS bytes per plane and
+ * 4 bytes per particle slot (max_particles).
+ *   amc_flux_enable   allocate and zero the accumulators, take the snapshot of the current state; re-enabling starts
+ *                     from zero.  AMC_E_STATE on a slab handle (and amc_slab_enable / amc_set_ids return AMC_E_STATE
+ *                     while recording is on), AMC_E_INVALID unless the particle ids are 0 .. n-1
+ *   amc_flux_disable  free everything
+ *   amc_flux_now      one record point (the host-RNG / phase-level paths call it after a timestep)
+ *   amc_flux_layout   number of planes (ncz + 1)
+ *   amc_flux_get_raw  acc: [planes][AMC_FLUX_WORDS] (nullable), record points taken
+ *   amc_flux_set_raw  resume from amc_flux_get_raw's values (recording must be enabled) */
+#define AMC_FLUX_WORDS 10
+#define AMC_FLUX_V1 16
+#define AMC_FLUX_V2 46
+#define AMC_FLUX_Q1 2
+#define AMC_FLUX_Q2 32
+int amc_flux_enable(amc_handle *h);
+int amc_flux_disable(amc_handle *h);
+int amc_flux_now(amc_handle *h);
+int amc_flux_layout(amc_handle *h, int32_t *n_planes);
+int amc_flux_get_raw(amc_handle *h, uint64_t *acc, uint64_t *n_steps);
+int amc_flux_set_raw(amc_handle *h, const uint64_t *acc, uint64_t n_steps);
+
 /* set the step counter that keys the device RNG (default: counts amc_step / amc_walls calls from 0) */
 int amc_set_step_index(amc_handle *h, int64_t step);
 
