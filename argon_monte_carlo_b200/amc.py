@@ -622,9 +622,10 @@ class Simulation:
 
     # ------------------------------------------------------------------ host-RNG parity mode
     def wall_case(self, case):
-        n = C.c_int64(0)
-        self._check(self.lib.amc_wall_case(self.h, int(case), C.byref(n)), "amc_wall_case")
-        return int(n.value)
+        """One specular case (1, 2a, 2b): (hits, hits that took the floating-point error path)."""
+        n, errs = C.c_int64(0), C.c_int64(0)
+        self._check(self.lib.amc_wall_case(self.h, int(case), C.byref(n), C.byref(errs)), "amc_wall_case")
+        return int(n.value), int(errs.value)
 
     def wall_hits_pending(self, case, cap=None):
         cap = int(cap or max(self.n, 1))
@@ -663,7 +664,8 @@ class Simulation:
         errors = 0
         for case in range(NUM_CASES):
             if case <= 2:
-                counts[case] = self.wall_case(case)
+                counts[case], er = self.wall_case(case)
+                errors += er
                 continue
             idx, nrm, colz = self.wall_hits_pending(case)
             counts[case] = len(idx)

@@ -1317,7 +1317,7 @@ extern "C" int amc_wall_operator(amc_handle *h, int32_t op, const uint8_t *mask,
 }
 
 // ---- host-RNG parity hooks ----------------------------------------------------------------------
-extern "C" int amc_wall_case(amc_handle *h, int32_t c, int64_t *n_hits)
+extern "C" int amc_wall_case(amc_handle *h, int32_t c, int64_t *n_hits, int64_t *errors)
 {
     if (!h) return AMC_E_INVALID;
     if (h->cfg.kind != AMC_KIND_TEMP) return h->fail(AMC_E_STATE, "amc_wall_case: AMC_KIND_TEMP only");
@@ -1330,6 +1330,7 @@ extern "C" int amc_wall_case(amc_handle *h, int32_t c, int64_t *n_hits)
     amc_step_stats st;
     rc = phase_end(h, &st);
     if (n_hits) *n_hits = st.wall_hits[c];
+    if (errors) *errors = st.errors; /* case 1 hits whose contact cannot be found (Temp:317-347) */
     return rc;
 }
 

@@ -159,7 +159,8 @@ enum { AMC_OP_PLANE_MFP = 0, AMC_OP_SIDE_MFP = 1, AMC_OP_PLANE_SPECULAR = 2, AMC
 int amc_wall_operator(amc_handle *h, int32_t op, const uint8_t *mask, double param, int64_t *n_hits, int64_t *errors);
 
 /* parity hooks for the energized walls (AMC_KIND_TEMP): one wall case at a time, in AMC_CASE_*
- * order, after amc_drift.  Specular cases (AMC_CASE_1, _2A, _2B): call amc_wall_case.
+ * order, after amc_drift.  Specular cases (AMC_CASE_1, _2A, _2B): call amc_wall_case (*errors: AMC_CASE_1 hits that
+ * took the reference's floating-point error path).
  * Energized cases: amc_wall_hits_pending reports the hits in ascending particle index with the
  * vector the reference hands to random_inbounds_direction (Temp:375,444,514; NaN = the hit raised a
  * floating-point error in the reference and draws nothing) and the contact height (argument of
@@ -167,7 +168,7 @@ int amc_wall_operator(amc_handle *h, int32_t op, const uint8_t *mask, double par
  * its Mersenne-Twister streams (Temp:132-141) and calls amc_wall_apply_directions, which returns
  * per-hit momentum / energy contributions (dpz[k], de[k]) so the host can sum them in the
  * reference's sequential order (Temp:385,389).  surf_e: per-hit surface energy, AMC_CASE_4 only. */
-int amc_wall_case(amc_handle *h, int32_t case_id, int64_t *n_hits);
+int amc_wall_case(amc_handle *h, int32_t case_id, int64_t *n_hits, int64_t *errors);
 int amc_wall_hits_pending(amc_handle *h, int32_t case_id, int64_t cap, int64_t *n_hits, int64_t *idx, double *normal3,
                           double *col_z);
 int amc_wall_apply_directions(amc_handle *h, int32_t case_id, int64_t n_hits, const int64_t *idx, const double *dir3,

@@ -166,19 +166,10 @@ def test_calm_regions_never_hide_a_wall_event(oracle, temp_cfg):
     thrown at every wall from both sides with displacements of up to several nanometres per step: for every particle
     the predicate calls calm, the reference's step is the drift and nothing else."""
     import math
+    from wall_edges import calm_bounds
     g, dt = temp_cfg.geom, temp_cfg.dt
-
-    def sq_threshold_gt(R):           # amc_api.cu: largest double t with sqrt(t) <= R
-        t = R * R
-        while math.sqrt(t) <= R:
-            t = np.nextafter(t, np.inf)
-        while math.sqrt(t) > R:
-            t = np.nextafter(t, 0.0)
-        return float(t)
     zs = [g.oah, g.zh3, g.z_gb, g.zgb_p, g.z_gt, g.zgt_m, g.z_cold, g.zc3]
-    zA, zB = min(zs + [g.H]), max(zs + [0.0])
-    rA = min(sq_threshold_gt(g.R_oa), g.R_oa_sq)
-    rC = min(rA, g.R_p_sq, g.R_g_c_sq, g.R_p_c_sq, g.R_g_sq)
+    zA, zB, rA, rC = calm_bounds(g)
     assert 0 < zA < zB < g.H and 0 < rC < rA
 
     rng = np.random.default_rng(42)
